@@ -35,6 +35,11 @@ are computed once on the GPU during set-up, exactly as the reference computes th
 
 --impl reference times only the CPU arm, on all host cores, and prints the same JSON line shape.
 Timed outputs are 196 MB per step (> the 126 MB L2), so every step streams to HBM; no explicit flush.
+
+--dump-outputs DIR writes what the timed steps computed, so that two builds can be compared output for output on
+identical inputs: DIR/rsurf.npy, the result rows of the last device-resident step, and DIR/rsurf_e2e.npy, those of
+the last host-pointer step, each for the same fixed, seeded sample of 1536 of the 11 664 lines (all 2101 bands,
+float64, 26 MB), and DIR/rsurf_lines.npy, the indices of those lines.  Rank 0's forest only.
 """
 import argparse
 import json
@@ -48,6 +53,8 @@ from pathlib import Path
 
 import numpy as np
 
+# the tree may be read-only and stays as the build left it: no __pycache__ from the project imports below
+sys.dont_write_bytecode = True
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
 sys.path.insert(0, str(ROOT / "tests"))
@@ -57,6 +64,8 @@ UNIT = "evals/s"
 F_LAMBDA = 92.0          # algorithmic FP64 ops per evaluation (SURVEY.md App. D)
 F_GEOM = 350.0           # per (line, set)
 F_LUT = 2.5e6            # per parameter set, outputs-only algorithm (SURVEY.md 8d)
+DUMP_LINES = 1536        # lines of the sweep in --dump-outputs: 2 x 1536 x 2101 doubles = 52 MB, under 64 MB
+DUMP_SEED = 2101
 
 
 def load_peaks():
@@ -206,6 +215,22 @@ def probe_host_placement(gort_b200, torch, dev, ts, barrier, rank):
                           "how": "all ranks copying 64 MB device-to-host at once into buffers pinned from each group"}
 
 
+def dump_lines(G):
+    """the fixed, seeded sample of sweep lines that --dump-outputs writes (sorted line indices)"""
+    rng = np.random.Generator(np.random.PCG64(DUMP_SEED))
+    return np.sort(rng.choice(G, size=min(G, DUMP_LINES), replace=False))
+
+
+def dump_outputs(out_dir, arrays):
+    """arrays {name: array} -> out_dir/<name>.npy, float64"""
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float64) for k, v in arrays.items()}
+    assert sum(a.nbytes for a in arrays.values()) <= 64 << 20
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(out_dir / (name + ".npy"), a)
+
+
 def sweep_inputs(rank):
     from gort_b200 import workloads as wk
     w = wk.c2_hemisphere(sets=1, lai0=4.0 + 0.25 * rank)
@@ -288,7 +313,10 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the C3 / C4 / C5 kernel measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a fixed sample of the last timed step's rsurf to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -364,6 +392,9 @@ def main():
     barrier()
     ms_total = e0.elapsed_time(e1)
     launches = g.launch_count() - l0
+    # the rows the last timed step stored, read before anything else writes d_out (the barrier above synchronised)
+    lines = dump_lines(G)
+    rsurf_dev = d_out[0].index_select(0, torch.from_numpy(lines).to(dev))[:, :W].cpu().numpy() if args.dump_outputs and rank == 0 else None
     # per-kernel durations: the same K steps again, this time with CUDA events recorded on the launching
     # stream around each kernel (gort_profile_begin/end).  Kept out of the timed region above because an
     # event between the two launches of a step would defeat their programmatic-dependent-launch overlap.
@@ -402,6 +433,8 @@ def main():
     clocks = sampler.stop() if rank == 0 else None       # sampled over both timed regions (device-resident and e2e)
     checksum = float(h_out.array[0, ::997, ::211].sum())
     rsurf_e2e = h_out.array[0].copy()                    # the result of the e2e leg (the copy test below reuses the buffer)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"rsurf": rsurf_dev, "rsurf_e2e": rsurf_e2e[lines], "rsurf_lines": lines})
 
     # ---- the ceiling of the e2e leg: a plain pinned D2H copy of the same 196 MB, all ranks at once ----
     d2h_ms = _plain_d2h_ms(torch, dev, ts, d_out, h_out.array, barrier)

@@ -6,6 +6,7 @@ tables parsed from PROSPECT-D/dataSpec_PDB.f90 itself when the reference tree is
 each other's code; they must agree to rounding, and the table generator's output must equal the Fortran literals
 rounded to REAL(4).
 """
+import os
 import re
 from pathlib import Path
 
@@ -16,6 +17,8 @@ from gort_b200 import workloads as wk
 
 ROOT = Path(__file__).resolve().parent.parent
 REF = Path("/root/reference/PROSPECT-D/dataSpec_PDB.f90")
+# os.path.isfile, not Path.exists: a tree this user may not enter counts as absent instead of raising PermissionError
+HAVE_REF = os.path.isfile(REF)
 NW = 2101
 NAMES = ["refractive", "k_Cab", "k_Car", "k_Anth", "k_Brown", "k_Cw", "k_Cm"]
 
@@ -147,7 +150,7 @@ def prospect_db(T, N, Cab, Car, Anth, Cbrown, Cw, Cm):
 
 
 def test_table_generator_matches_fortran_literals():
-    if not REF.exists():
+    if not HAVE_REF:
         pytest.skip("reference tree not present")
     tf, th = tables_from_fortran(), tables_from_header()
     for name in NAMES:
@@ -155,7 +158,7 @@ def test_table_generator_matches_fortran_literals():
 
 
 def test_second_restatement_agrees_with_the_oracle(oracle):
-    T = tables_from_fortran() if REF.exists() else tables_from_header()
+    T = tables_from_fortran() if HAVE_REF else tables_from_header()
     rng = np.random.Generator(np.random.PCG64(77))
     leaves = np.concatenate([wk.DEFAULT_LEAF.reshape(7, 1), wk.random_leaves(rng, 12)], axis=1)
     leaves[4, 3] = 0.0          # Cbrown = 0

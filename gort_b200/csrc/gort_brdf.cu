@@ -472,6 +472,9 @@ int launch_brdf(gort_ctx *ctx, cudaStream_t s, const gort_shape &sh, const doubl
     const long L = (long) sh.n_sets * sh.n_geom;
     const long pitch = sh.out_pitch > 0 ? sh.out_pitch : sh.n_wl;
     if (pitch < sh.n_wl) return set_error(ctx, GORT_ERR_INVALID, "gort_brdf: out_pitch smaller than n_wl");
+    // every path stores a { C, G, T, Z } quadruple as one vector: double4 in rsurf_flat_kernel, double2 pairs or bulk
+    // copies in the wide kernel
+    if (((size_t) scomp & 31) != 0) return set_error(ctx, GORT_ERR_INVALID, "gort_brdf: scomp must be 32-byte aligned");
     const bool use_pdl = !ctx->dbg_no_pdl;
     // calls on different streams are ordered one after the other (record buffers and the flags are shared)
     if (ctx->last_stream && ctx->last_stream != s) {

@@ -191,7 +191,8 @@ int gort_soil_from_table_dev(gort_ctx *ctx, void *stream, const double *table, i
  *      angle normalisation, gortt_prime_theta, fd, gortt_set_zenith_dependant_probabilities,
  *      gortt_rsurf (include/gortt.h:216-219).
  *      rsurf [M][G][pitch] (pitch = shape.out_pitch, default W); scomp (optional, may be NULL)
- *      [M][G][pitch][4] = C,G,T,Z (gortt.c:562-565);
+ *      [M][G][pitch][4] = C,G,T,Z (gortt.c:562-565), 32-byte aligned (each quadruple is stored as one vector;
+ *      any other address is GORT_ERR_INVALID and nothing is enqueued);
  *      kprop (optional) [M][G][4] = Kc,Kg,Kt,Kz (gortt.c:570-573). -------------------------- */
 int gort_brdf_batch(gort_ctx *ctx, const gort_shape *shape, const double *structure,
                     const double *lut, const double *angles,

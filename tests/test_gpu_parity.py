@@ -7,50 +7,9 @@ import pytest
 
 from gort_b200 import workloads as wk
 import gort_b200
-from checkers import sensitivity
+from checkers import assert_close, assert_close_cond, sensitivity
 
 pytestmark = pytest.mark.gpu
-
-RTOL = 1e-9
-FLOOR = 1e-12
-
-
-def rel_err(x, ref):
-    x = np.asarray(x); ref = np.asarray(ref)
-    assert x.shape == ref.shape, (x.shape, ref.shape)
-    nx, nr = np.isnan(x), np.isnan(ref)
-    assert np.array_equal(nx, nr), "NaN positions differ: %d vs %d" % (nx.sum(), nr.sum())
-    ok = ~nr
-    if not ok.any():
-        return 0.0
-    return float(np.max(np.abs(x[ok] - ref[ok]) / np.maximum(np.abs(ref[ok]), FLOOR)))
-
-
-def assert_close(x, ref, what, rtol=RTOL):
-    e = rel_err(x, ref)
-    assert e <= rtol, "%s: max rel err %.3e > %.1e" % (what, e, rtol)
-    return e
-
-
-COND_FACTOR = 32.0
-
-
-def assert_close_cond(x, ref, sens, what, rtol=RTOL):
-    """Strict bound first.  An entry that misses it must be explained by the reference algorithm's own
-    conditioning: |x - ref| <= COND_FACTOR * (how far the oracle itself moves under a 1-ULP libm,
-    tests/checkers.py:sensitivity).  Returns (strict worst rel err, number of entries excused)."""
-    x = np.asarray(x); ref = np.asarray(ref)
-    nx, nr = np.isnan(x), np.isnan(ref)
-    assert np.array_equal(nx, nr), "%s: NaN positions differ" % what
-    ok = ~nr
-    err = np.abs(x[ok] - ref[ok])
-    strict = err <= rtol * np.maximum(np.abs(ref[ok]), FLOOR)
-    excused = ~strict & (err <= COND_FACTOR * sens[ok])
-    bad = ~strict & ~excused
-    rel = err / np.maximum(np.abs(ref[ok]), FLOOR)
-    assert not bad.any(), "%s: %d entries miss 1e-9 and are not explained by conditioning; worst rel %.3e (sens %.3e, err %.3e)" % (
-        what, bad.sum(), rel[bad].max(), sens[ok][bad][rel[bad].argmax()], err[bad][rel[bad].argmax()])
-    return (float(rel.max()) if rel.size else 0.0), int(excused.sum())
 
 
 # ---------------------------------------------------------------------------------------------

@@ -429,6 +429,29 @@ int gort_oracle_lut(const double *st6, int method, double *lut)
     return 0;
 }
 
+/* The histogram bins the crown-count loop of gap_probabilities_full reaches (gortt_pn_kopen.c:457-527, h = 0):
+ * umax[t] = the largest s / ds + 0.5 over entry heights sp_i < NLAY - 1 and crown counts n, the value that
+ * s_to_index truncates; umax[NTH - 1] = 0 (no epgap there).  s depends on E[S] and s' only, so the tube
+ * volumes are not evaluated; the s of each (sp_i, n) is formed exactly as above. */
+int gort_oracle_lut_bins(const double *st6, double *umax)
+{
+    canopy_t c;
+    canopy_init(&c, st6);
+    for (int t = 0; t < NTH; t++) umax[t] = 0.0;
+    for (int t = 0; t < NTH - 1; t++) {
+        double es = expected_single_crown_path(&c, 0, t);
+        for (int sp_i = NLAY - 2; sp_i > 0; sp_i--) {
+            double s_p = (double) (c.height_p[sp_i] - c.height_p[0]) / cos(c.theta_p[t]);
+            for (int n = 1; n <= MAXCROWNS; n++) {
+                double s = s_p * (1.0 - exp(-1.0 * (double) n * es / s_p));
+                double u = s / c.ds + 0.5;
+                if (u > umax[t]) umax[t] = u;
+            }
+        }
+    }
+    return 0;
+}
+
 int gort_oracle_lut_intermediates(const double *st6, double *v_g, double *p_n0, double *derived,
                                   double *theta_p, double *height_p)
 {

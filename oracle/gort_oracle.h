@@ -14,6 +14,9 @@
 int gort_oracle_lut(const double *st6, int method, double *lut);
 int gort_oracle_lut_intermediates(const double *st6, double *v_g, double *p_n0, double *derived,
                                   double *theta_p, double *height_p);
+/* umax[t] = largest s/ds + 0.5 the crown-count loop of the full method reaches at zenith t (the value truncated to a
+ * histogram bin); umax[NTH - 1] = 0 */
+int gort_oracle_lut_bins(const double *st6, double *umax);
 int gort_oracle_brdf(const double *st6, const double *lut, const double *opt,
                      int ngeom, const double *ang, int nw,
                      const double *rleaf, const double *tleaf, const double *rsoil,

@@ -102,13 +102,30 @@ class Checker:
 
     def lut_dead(self, st6):
         """vb[15], fb[15][91], t_open[15][15], dt_open[15][15], dk_open[15], k_open[15] (gortt_pn_kopen.c:925-1078)."""
+        rc, out = self.lut_dead_rc(st6)
+        assert rc == 0, "negative sphere volume: the reference exits on this structure"
+        return out
+
+    def lut_dead_rc(self, st6):
+        """(rc, outputs of lut_dead): rc = 1 where the reference exits on a negative sphere volume (gortt_calc_vb);
+        the outputs are then undefined."""
         fn = getattr(self.lib, self.prefix + "lut_dead")
         fn.argtypes = [_dp] * 7
         fn.restype = C.c_int
         out = dict(vb=np.empty(15), fb=np.empty((15, NTH)), t_open=np.empty((15, 15)), dt_open=np.empty((15, 15)),
                    dk_open=np.empty(15), k_open=np.empty(15))
         rc = fn(_p(self._st(st6)), *[_p(out[k]) for k in ("vb", "fb", "t_open", "dt_open", "dk_open", "k_open")])
-        assert rc == 0, "negative sphere volume: the reference exits on this structure"
+        return rc, out
+
+    def lut_bins(self, st6):
+        """(restatement only) umax[91]: per zenith, the largest s/ds + 0.5 the full method's crown-count loop reaches,
+        i.e. the largest histogram bin is int(umax[t]) (gortt_pn_kopen.c:457-527, :134-139)."""
+        fn = getattr(self.lib, self.prefix + "lut_bins")
+        fn.argtypes = [_dp, _dp]
+        fn.restype = C.c_int
+        out = np.empty(NTH)
+        rc = fn(_p(self._st(st6)), _p(out))
+        assert rc == 0
         return out
 
     def soil_table(self, path):
@@ -239,6 +256,39 @@ def assert_close_cond(x, ref, sens, what, rtol=RTOL):
     assert not bad.any(), "%s: %d entries miss 1e-9 and are not explained by conditioning; worst rel %.3e (sens %.3e, err %.3e)" % (
         what, bad.sum(), rel[bad].max(), sens[ok][bad][rel[bad].argmax()], err[bad][rel[bad].argmax()])
     return (float(rel.max()) if rel.size else 0.0), int(excused.sum())
+
+
+DEAD_KEYS = ("vb", "fb", "t_open", "dt_open", "dk_open", "k_open")
+
+
+def check_set(got, st6, oracle, what):
+    """One set's gort_lut_intermediates outputs against the oracle's lut_dead.  fb = (1 - exp(-lv' vb)) / (1 - p_n0) is
+    rounding noise wherever p_n0 rounds to 1 (the reference divides by DBL_MIN * 2 there, gortt_pn_kopen.c:990) and
+    wherever vb is itself a cancelled ~1e-16 (a sphere centred on the lowest layer touches the h1 plane): those entries
+    are compared for finiteness only.  Everything else: 1e-9, conditioning-aware like the LUT tests."""
+    import parity_audit as pa                      # imports this module: deferred
+    KEYS = DEAD_KEYS
+    want = oracle.lut_dead(st6)
+    lut = oracle.lut_intermediates(st6)
+    sens = None
+    worst = {}
+    for k in KEYS:
+        x, r = got[k], want[k]
+        mask = np.ones(r.shape, dtype=bool)
+        if k == "fb":
+            mask = (1.0 - lut["p_n0"] >= 1e-12) & (want["vb"][:, None] > 1e-9)      # see the docstring
+            assert np.isfinite(x).all()
+        if k == "vb":
+            mask = r > 1e-9
+            assert np.all(np.abs(x[~mask] - r[~mask]) < 1e-12)
+        s = pa.compare(x[mask], r[mask])
+        if s["n_beyond_tol"]:
+            if sens is None:
+                sens = dict(zip(KEYS, sensitivity(lambda c: tuple(c.lut_dead(st6)[q] for q in KEYS), tuple(want[q] for q in KEYS))))
+            s = pa.compare(x[mask], r[mask], sens[k][mask])
+        assert pa.passed(s), "%s %s: %r" % (what, k, s)
+        worst[k] = s["max_rel_err"]
+    return worst
 
 
 def ref():

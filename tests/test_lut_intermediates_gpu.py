@@ -4,42 +4,14 @@ pin to the compiled reference bit for bit.
 
 fb = (1 - exp(-lv' vb)) / (1 - p_n0) is rounding noise wherever p_n0 rounds to 1 (the reference divides by DBL_MIN * 2 there,
 :990) and wherever vb is itself a cancelled ~1e-16 (a sphere centred on the lowest layer touches the h1 plane): those entries
-are compared for finiteness only.  Everything else: 1e-9, conditioning-aware like the LUT tests."""
+are compared for finiteness only (checkers.check_set).  Everything else: 1e-9, conditioning-aware like the LUT tests."""
 import numpy as np
 import pytest
 
-import gort_b200
-import parity_audit as pa
-from checkers import sensitivity
+from checkers import DEAD_KEYS as KEYS, check_set
 from gort_b200 import workloads as wk
 
 pytestmark = pytest.mark.gpu
-KEYS = ("vb", "fb", "t_open", "dt_open", "dk_open", "k_open")
-
-
-def check_set(got, st6, oracle, what):
-    want = oracle.lut_dead(st6)
-    lut = oracle.lut_intermediates(st6)
-    sens = None
-    worst = {}
-    for k in KEYS:
-        x, r = got[k], want[k]
-        mask = np.ones(r.shape, dtype=bool)
-        if k == "fb":
-            mask = (1.0 - lut["p_n0"] >= 1e-12) & (want["vb"][:, None] > 1e-9)      # see the module docstring
-            assert np.isfinite(x).all()
-        if k == "vb":
-            mask = r > 1e-9
-            assert np.all(np.abs(x[~mask] - r[~mask]) < 1e-12)
-        s = pa.compare(x[mask], r[mask])
-        if s["n_beyond_tol"]:
-            if sens is None:
-                sens = dict(zip(KEYS, sensitivity(lambda c: tuple(c.lut_dead(st6)[q] for q in KEYS), tuple(want[q] for q in KEYS))))
-            s = pa.compare(x[mask], r[mask], sens[k][mask])
-        assert pa.passed(s), "%s %s: %r" % (what, k, s)
-        worst[k] = s["max_rel_err"]
-    return worst
-
 
 def test_dead_intermediates_random_structures(gort, oracle):
     rng = np.random.Generator(np.random.PCG64(41))

@@ -10,8 +10,8 @@
 //   tav_kernel       once per context: tav_abs(90 deg) and tav_abs(40 deg) for the 2101-entry
 //                    refractive-index table -- they depend on no leaf parameter.
 //   spectra_kernel   one thread per (parameter set, requested wavelength): evaluates PROSPECT-D only
-//                    at the table rows the reference's linear interpolation touches (2 rows, or 1
-//                    when the float fraction is 0) and the Price EOF sum.  Coalesced [M][W] stores.
+//                    at the two table rows the reference's linear interpolation touches (1 at 2500 nm)
+//                    and the Price EOF sum.  Coalesced [M][W] stores.
 //   prospect_full_kernel  the whole 2101-band RT array of prospect_DB_, [M][2101].
 #include <string.h>
 #include "gort_internal.h"
@@ -200,9 +200,10 @@ spectra_kernel(int n_sets, int n_wl, const double* __restrict__ leaf, const doub
         float omf = 1 - fraction;
         double rl, tl, ru = 0.0, tu = 0.0;
         prospect_row(tab, p, lower, rl, tl);
-        // the upper row only matters when the fraction is non-zero (x*(1-0) + y*0 == x for finite y);
-        // at 2500 nm the reference's upper row is one past the array and its fraction is 0
-        if (fraction != 0.0f && upper < NWP) prospect_row(tab, p, upper, ru, tu);
+        // the upper row is evaluated even when the fraction is 0: y*0 is NaN for a NaN row (N > 1 and k > 85:
+        // tau = 0, b = inf, Rsub = inf/inf), and the reference's interpolation propagates it.  At 2500 nm the
+        // reference's upper row is one past the array and its fraction is 0: it contributes 0
+        if (upper < NWP) prospect_row(tab, p, upper, ru, tu);
         rleaf[e] = rl * omf + ru * fraction;
         tleaf[e] = tl * omf + tu * fraction;
     }

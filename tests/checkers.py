@@ -100,6 +100,18 @@ class Checker:
         self._spectra(_p(leaf7), _p(soil4), user_leaf, user_soil, nw, _p(wl), _p(rl), _p(tl), _p(rs))
         return rl, tl, rs
 
+    def prospect_full(self, leaf7):
+        """(restatement only) the whole 2101-row PROSPECT-D table of one leaf, uninterpolated
+        (prospect_DB.f90:72-191): refl[2101], tran[2101]."""
+        fn = getattr(self.lib, self.prefix + "prospect_full")
+        fn.argtypes = [_dp, _dp, _dp]
+        fn.restype = None
+        leaf7 = np.ascontiguousarray(leaf7, dtype=np.float64)
+        assert leaf7.shape == (7,)
+        refl = np.empty(2101); tran = np.empty(2101)
+        fn(_p(leaf7), _p(refl), _p(tran))
+        return refl, tran
+
     def lut_dead(self, st6):
         """vb[15], fb[15][91], t_open[15][15], dt_open[15][15], dk_open[15], k_open[15] (gortt_pn_kopen.c:925-1078)."""
         rc, out = self.lut_dead_rc(st6)

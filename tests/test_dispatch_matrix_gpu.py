@@ -122,6 +122,9 @@ CASES = {
     "signatures_thread":    (1500, 7, 97, 0, True, True, False, 0, "geom_kernel", "rsurf_wide_kernel<2,1,2,0,0>"),
     "bands_geom_lines":     (4000, 16, 7, 0, True, True, True, 0, "geom_lines_kernel", "rsurf_flat_kernel"),
     "unaligned_rsurf":      (2, 1200, 2101, 2112, False, False, False, 1, "geom_kernel", "rsurf_wide_kernel<4,0,2,0,0>"),
+    # rows that cannot take TMA with 65..96 (or 96 written) columns: LPT = 3 wastes the fewest columns
+    "lpt3_dense":           (300, 16, 95, 0, False, True, True, 0, "geom_kernel", "rsurf_wide_kernel<3,0,2,0,0>"),
+    "lpt3_padded_unaligned": (2, 1500, 90, 96, False, False, False, 1, "geom_kernel", "rsurf_wide_kernel<3,0,2,0,0>"),
 }
 
 

@@ -55,6 +55,18 @@ void *workspace(gort_ctx *ctx, size_t bytes) { return grow(ctx, &ctx->work, &ctx
 void *rec_buffer(gort_ctx *ctx, int which, size_t bytes) { return grow(ctx, &ctx->rec_buf[which], &ctx->rec_cap[which], bytes); }
 void *tab_buffer(gort_ctx *ctx, int which, size_t bytes) { return grow(ctx, &ctx->tab_buf[which], &ctx->tab_cap[which], bytes); }
 
+int order_after_previous(gort_ctx *ctx, cudaStream_t s)
+{
+    if (ctx->last_stream && ctx->last_stream != s) {
+        cudaError_t e = cudaEventRecord(ctx->xstream_ev, ctx->last_stream);
+        if (e == cudaSuccess) e = cudaStreamWaitEvent(s, ctx->xstream_ev, 0);
+        if (e != cudaSuccess) return check_cuda(ctx, e, "ordering calls across streams");
+        ctx->last_was_wide = 0;
+    }
+    ctx->last_stream = s;
+    return GORT_OK;
+}
+
 }  // namespace gort
 
 using namespace gort;
@@ -169,7 +181,8 @@ int gort_synchronize(gort_ctx *ctx)
 {
     if (!ctx) return GORT_ERR_INVALID;
     TRYCUDA(ctx, cudaSetDevice(ctx->device), "cudaSetDevice");
-    // everything this context enqueued, on its own stream and on the last caller-supplied one
+    // everything this context enqueued: each call waited for the one before it (order_after_previous), so the last
+    // call's stream completes after all of them
     TRYCUDA(ctx, cudaStreamSynchronize(ctx->stream), "synchronize");
     if (ctx->last_stream && ctx->last_stream != ctx->stream) TRYCUDA(ctx, cudaStreamSynchronize(ctx->last_stream), "synchronize");
     ctx->last_stream = NULL;           // everything is complete: the caller may destroy its stream now
@@ -207,6 +220,7 @@ static void probe_host_placement(gort_ctx *ctx)
     for (int c = 0; c < CPU_SETSIZE && n < 1024; c++) if (CPU_ISSET(c, &all)) cpus[n++] = c;
     if (n < 4) { snprintf(ctx->near_desc, sizeof ctx->near_desc, "%d cpus: nothing to choose", n); return; }
     const size_t probe_bytes = (size_t) 32 << 20;
+    if (order_after_previous(ctx, ctx->stream) != GORT_OK) { snprintf(ctx->near_desc, sizeof ctx->near_desc, "probe failed"); return; }
     void *d = workspace(ctx, probe_bytes);
     if (!d) return;
     const int n_groups = n >= 16 ? 8 : 4;
@@ -316,7 +330,9 @@ int gort_lut_batch_dev(gort_ctx *ctx, void *stream, int n_sets, const double *st
     if (!structure || !lut || n_sets <= 0) return set_error(ctx, GORT_ERR_INVALID, "gort_lut_batch: bad arguments");
     if (method != GORT_LUT_FULL && method != GORT_LUT_Q08) return set_error(ctx, GORT_ERR_INVALID, "gort_lut_batch: unknown method %d", method);
     TRYCUDA(ctx, cudaSetDevice(ctx->device), "cudaSetDevice");
-    return launch_lut(ctx, pick(ctx, stream), n_sets, structure, method, lut);
+    const cudaStream_t s = pick(ctx, stream);
+    TRY(order_after_previous(ctx, s));
+    return launch_lut(ctx, s, n_sets, structure, method, lut);
 }
 
 int gort_lut_batch_scatter_dev(gort_ctx *ctx, void *stream, int n_sets, const double *structure, int method,
@@ -329,7 +345,9 @@ int gort_lut_batch_scatter_dev(gort_ctx *ctx, void *stream, int n_sets, const do
         if (!dst[q] || ((uintptr_t) dst[q] & 7)) return set_error(ctx, GORT_ERR_INVALID, "gort_lut_batch_scatter: destination %d is null or misaligned", q);
     if (method != GORT_LUT_FULL && method != GORT_LUT_Q08) return set_error(ctx, GORT_ERR_INVALID, "gort_lut_batch: unknown method %d", method);
     TRYCUDA(ctx, cudaSetDevice(ctx->device), "cudaSetDevice");
-    return launch_lut_out(ctx, pick(ctx, stream), n_sets, structure, method, lut, n_dst, dst, multicast != 0);
+    const cudaStream_t s = pick(ctx, stream);
+    TRY(order_after_previous(ctx, s));
+    return launch_lut_out(ctx, s, n_sets, structure, method, lut, n_dst, dst, multicast != 0);
 }
 
 int gort_lut_batch(gort_ctx *ctx, int n_sets, const double *structure, int method, double *lut)
@@ -337,6 +355,7 @@ int gort_lut_batch(gort_ctx *ctx, int n_sets, const double *structure, int metho
     if (!ctx) return GORT_ERR_INVALID;
     if (!structure || !lut || n_sets <= 0) return set_error(ctx, GORT_ERR_INVALID, "gort_lut_batch: bad arguments");
     TRYCUDA(ctx, cudaSetDevice(ctx->device), "cudaSetDevice");
+    TRY(order_after_previous(ctx, ctx->stream));
     double *d_st, *d_lut;
     TRY(h2d(ctx, 0, structure, (size_t) 6 * n_sets, &d_st));
     TRY(dout(ctx, 1, lut, (size_t) n_sets * GORT_LUT_STRIDE, &d_lut));
@@ -351,7 +370,9 @@ int gort_lut_intermediates_batch_dev(gort_ctx *ctx, void *stream, int n_sets, co
     if (!ctx) return GORT_ERR_INVALID;
     if (!structure || n_sets <= 0) return set_error(ctx, GORT_ERR_INVALID, "gort_lut_intermediates_batch: bad arguments");
     TRYCUDA(ctx, cudaSetDevice(ctx->device), "cudaSetDevice");
-    return launch_lut_dead(ctx, pick(ctx, stream), n_sets, structure, vb, fb, t_open, dt_open, dk_open, k_open);
+    const cudaStream_t s = pick(ctx, stream);
+    TRY(order_after_previous(ctx, s));
+    return launch_lut_dead(ctx, s, n_sets, structure, vb, fb, t_open, dt_open, dk_open, k_open);
 }
 
 int gort_lut_intermediates_batch(gort_ctx *ctx, int n_sets, const double *structure, double *vb, double *fb,
@@ -360,6 +381,7 @@ int gort_lut_intermediates_batch(gort_ctx *ctx, int n_sets, const double *struct
     if (!ctx) return GORT_ERR_INVALID;
     if (!structure || n_sets <= 0) return set_error(ctx, GORT_ERR_INVALID, "gort_lut_intermediates_batch: bad arguments");
     TRYCUDA(ctx, cudaSetDevice(ctx->device), "cudaSetDevice");
+    TRY(order_after_previous(ctx, ctx->stream));
     const size_t M = n_sets;
     double *d_st, *d[6];
     double *h[6] = {vb, fb, t_open, dt_open, dk_open, k_open};
@@ -379,7 +401,9 @@ int gort_spectra_batch_dev(gort_ctx *ctx, void *stream, int n_sets, const double
     if (!ctx) return GORT_ERR_INVALID;
     if (!wavelength || !rleaf || !tleaf || !rsoil) return set_error(ctx, GORT_ERR_INVALID, "gort_spectra_batch: NULL argument");
     TRYCUDA(ctx, cudaSetDevice(ctx->device), "cudaSetDevice");
-    return launch_spectra(ctx, pick(ctx, stream), n_sets, leaf, soil, user_leaf, user_soil, n_wl, wavelength, rleaf, tleaf, rsoil);
+    const cudaStream_t s = pick(ctx, stream);
+    TRY(order_after_previous(ctx, s));
+    return launch_spectra(ctx, s, n_sets, leaf, soil, user_leaf, user_soil, n_wl, wavelength, rleaf, tleaf, rsoil);
 }
 
 int gort_spectra_batch(gort_ctx *ctx, int n_sets, const double *leaf, const double *soil,
@@ -393,6 +417,7 @@ int gort_spectra_batch(gort_ctx *ctx, int n_sets, const double *leaf, const doub
         if (wavelength[i] < GORT_WL_MIN || wavelength[i] > GORT_WL_MAX)
             return set_error(ctx, GORT_ERR_RANGE, "wavlength out of range (400-2500)");   /* sic, gortt.c:1300 */
     TRYCUDA(ctx, cudaSetDevice(ctx->device), "cudaSetDevice");
+    TRY(order_after_previous(ctx, ctx->stream));
     double *d_leaf, *d_soil, *d_wl, *d_rl, *d_tl, *d_rs;
     size_t n = (size_t) n_sets * n_wl;
     TRY(h2d(ctx, 0, user_leaf < 0.0 ? leaf : NULL, (size_t) 7 * n_sets, &d_leaf));
@@ -413,6 +438,7 @@ int gort_prospect_batch(gort_ctx *ctx, int n_sets, const double *leaf, double *r
     if (!ctx) return GORT_ERR_INVALID;
     if (!leaf || !refl || !tran || n_sets <= 0) return set_error(ctx, GORT_ERR_INVALID, "gort_prospect_batch: bad arguments");
     TRYCUDA(ctx, cudaSetDevice(ctx->device), "cudaSetDevice");
+    TRY(order_after_previous(ctx, ctx->stream));
     double *d_leaf, *d_r, *d_t;
     size_t n = (size_t) n_sets * GORT_PROSPECT_NW;
     TRY(h2d(ctx, 0, leaf, (size_t) 7 * n_sets, &d_leaf));
@@ -467,7 +493,9 @@ int gort_soil_from_table_dev(gort_ctx *ctx, void *stream, const double *table, i
     if (!table || !wavelength || !rsoil || n_sets <= 0 || n_wl <= 0)
         return set_error(ctx, GORT_ERR_INVALID, "gort_soil_from_table: bad arguments");
     TRYCUDA(ctx, cudaSetDevice(ctx->device), "cudaSetDevice");
-    return launch_soil_table(ctx, pick(ctx, stream), table, n_sets, n_wl, wavelength, rsoil);
+    const cudaStream_t s = pick(ctx, stream);
+    TRY(order_after_previous(ctx, s));
+    return launch_soil_table(ctx, s, table, n_sets, n_wl, wavelength, rsoil);
 }
 
 int gort_soil_from_table(gort_ctx *ctx, const double *table, int n_sets, int n_wl, const double *wavelength, double *rsoil)
@@ -479,6 +507,7 @@ int gort_soil_from_table(gort_ctx *ctx, const double *table, int n_sets, int n_w
         if (wavelength[i] < GORT_WL_MIN || wavelength[i] > GORT_WL_MAX)
             return set_error(ctx, GORT_ERR_RANGE, "wavlength out of range (400-2500)");
     TRYCUDA(ctx, cudaSetDevice(ctx->device), "cudaSetDevice");
+    TRY(order_after_previous(ctx, ctx->stream));
     double *d_tab, *d_wl, *d_rs;
     TRY(h2d(ctx, 0, table, GORT_SOIL_TABLE_NW, &d_tab));
     TRY(h2d(ctx, 1, wavelength, n_wl, &d_wl));
@@ -508,7 +537,9 @@ int gort_brdf_batch_dev(gort_ctx *ctx, void *stream, const gort_shape *shape, co
     if (!structure || !lut || !angles || !rleaf || !tleaf || !rsoil || !rsurf)
         return set_error(ctx, GORT_ERR_INVALID, "gort_brdf_batch: NULL argument");
     TRYCUDA(ctx, cudaSetDevice(ctx->device), "cudaSetDevice");
-    return launch_brdf(ctx, pick(ctx, stream), *shape, structure, lut, angles, rleaf, tleaf, rsoil, rsurf, scomp, kprop);
+    const cudaStream_t s = pick(ctx, stream);
+    TRY(order_after_previous(ctx, s));
+    return launch_brdf(ctx, s, *shape, structure, lut, angles, rleaf, tleaf, rsoil, rsurf, scomp, kprop);
 }
 
 static int copy_rows(gort_ctx *ctx, cudaStream_t s, double *dst, size_t dst_pitch, const double *src, size_t src_pitch,
@@ -540,6 +571,7 @@ int gort_brdf_batch(gort_ctx *ctx, const gort_shape *shape, const double *struct
     if (!structure || !lut || !angles || !rleaf || !tleaf || !rsoil || !rsurf)
         return set_error(ctx, GORT_ERR_INVALID, "gort_brdf_batch: NULL argument");
     TRYCUDA(ctx, cudaSetDevice(ctx->device), "cudaSetDevice");
+    TRY(order_after_previous(ctx, ctx->stream));
     Staged d;
     TRY(stage_inputs(ctx, shape, structure, lut, angles, rleaf, tleaf, rsoil, &d));
     size_t nl = (size_t) shape->n_sets * shape->n_geom;
@@ -620,6 +652,9 @@ int gort_forward_batch(gort_ctx *ctx, const gort_shape *shape, int lut_method, c
     gort_shape sh = *shape;
     sh.spectra_per_set = 1;
     sh.out_pitch = 0;
+    // the kernels wait for the previous call; the input copies on B need not: they only fill this call's scratch slots,
+    // which no other call reads while this one runs (every host-pointer call returns synchronised)
+    TRY(order_after_previous(ctx, A));
     int chunk_no = 0;
     for (size_t m0 = 0; m0 < M; m0 += C, chunk_no++) {
         const size_t c = M - m0 < C ? M - m0 : C;
@@ -674,6 +709,7 @@ int gort_jacobian_batch(gort_ctx *ctx, const gort_shape *shape, int lut_method, 
     const double h = rel_step > 0.0 ? rel_step : 1e-4;
     const int row = param == GORT_JAC_LAI ? 5 : param;
     cudaStream_t A = ctx->stream;
+    TRY(order_after_previous(ctx, A));
     // members in chunks that keep the three result buffers below ~768 MB
     size_t C = ((size_t) 256 << 20) / (G * W * sizeof(double));
     if (C < 1) C = 1;
@@ -729,7 +765,9 @@ int gort_energy_batch_dev(gort_ctx *ctx, void *stream, const gort_shape *shape, 
     if (!structure || !lut || !angles || !rleaf || !tleaf || !rsoil || !albedo || !favegt || !fasoil)
         return set_error(ctx, GORT_ERR_INVALID, "gort_energy_batch: NULL argument");
     TRYCUDA(ctx, cudaSetDevice(ctx->device), "cudaSetDevice");
-    return launch_energy(ctx, pick(ctx, stream), *shape, structure, lut, angles, rleaf, tleaf, rsoil, albedo, favegt, fasoil);
+    const cudaStream_t s = pick(ctx, stream);
+    TRY(order_after_previous(ctx, s));
+    return launch_energy(ctx, s, *shape, structure, lut, angles, rleaf, tleaf, rsoil, albedo, favegt, fasoil);
 }
 
 int gort_energy_batch(gort_ctx *ctx, const gort_shape *shape, const double *structure, const double *lut,
@@ -741,6 +779,7 @@ int gort_energy_batch(gort_ctx *ctx, const gort_shape *shape, const double *stru
     if (!structure || !lut || !angles || !rleaf || !tleaf || !rsoil || !albedo || !favegt || !fasoil)
         return set_error(ctx, GORT_ERR_INVALID, "gort_energy_batch: NULL argument");
     TRYCUDA(ctx, cudaSetDevice(ctx->device), "cudaSetDevice");
+    TRY(order_after_previous(ctx, ctx->stream));
     Staged d;
     TRY(stage_inputs(ctx, shape, structure, lut, angles, rleaf, tleaf, rsoil, &d));
     size_t n = (size_t) shape->n_sets * shape->n_geom * shape->n_wl;
@@ -759,6 +798,7 @@ int gort_gauleg(gort_ctx *ctx, double *abscissa, double *weights)
 {
     if (!ctx || !abscissa || !weights) return GORT_ERR_INVALID;
     TRYCUDA(ctx, cudaSetDevice(ctx->device), "cudaSetDevice");
+    TRY(order_after_previous(ctx, ctx->stream));
     TRYCUDA(ctx, cudaMemcpyAsync(abscissa, ctx->d_gauleg, sizeof(double) * GORT_NQUAD, cudaMemcpyDeviceToHost, ctx->stream), "gauleg copy");
     TRYCUDA(ctx, cudaMemcpyAsync(weights, ctx->d_gauleg + GORT_NQUAD, sizeof(double) * GORT_NQUAD, cudaMemcpyDeviceToHost, ctx->stream), "gauleg copy");
     return check_cuda(ctx, cudaStreamSynchronize(ctx->stream), "gort_gauleg");
@@ -768,6 +808,7 @@ int gort_dfma_peak(gort_ctx *ctx, double *tflops)
 {
     if (!ctx || !tflops) return GORT_ERR_INVALID;
     TRYCUDA(ctx, cudaSetDevice(ctx->device), "cudaSetDevice");
+    TRY(order_after_previous(ctx, ctx->stream));
     return launch_dfma_peak(ctx, ctx->stream, tflops);
 }
 

@@ -476,13 +476,8 @@ int launch_brdf(gort_ctx *ctx, cudaStream_t s, const gort_shape &sh, const doubl
     // copies in the wide kernel
     if (((size_t) scomp & 31) != 0) return set_error(ctx, GORT_ERR_INVALID, "gort_brdf: scomp must be 32-byte aligned");
     const bool use_pdl = !ctx->dbg_no_pdl;
-    // calls on different streams are ordered one after the other (record buffers and the flags are shared)
-    if (ctx->last_stream && ctx->last_stream != s) {
-        cudaError_t e = cudaEventRecord(ctx->xstream_ev, ctx->last_stream);
-        if (e == cudaSuccess) e = cudaStreamWaitEvent(s, ctx->xstream_ev, 0);
-        if (e != cudaSuccess) return check_cuda(ctx, e, "ordering BRDF calls across streams");
-        ctx->last_was_wide = 0;
-    }
+    // a call on another stream than the previous one has been ordered after it by the entry point (order_after_previous),
+    // which also ended the previous call's claim to overlap
     ctx->call_no++;
     // line records, the (set, lambda) table and the ready flags are double-buffered by call parity: this call's
     // geometry kernel may run while the previous call's per-wavelength kernel still reads its own
@@ -630,7 +625,6 @@ int launch_brdf(gort_ctx *ctx, cudaStream_t s, const gort_shape &sh, const doubl
     }
     ctx->launches++;
     if (ev) { cudaError_t e = cudaEventRecord(ev[2], s); if (e != cudaSuccess) return check_cuda(ctx, e, "cudaEventRecord"); ctx->prof_n++; }
-    ctx->last_stream = s;
     ctx->last_was_wide = (sh.n_wl >= 64) && !ev;
     ctx->last_out_lo[0] = (const char *) rsurf; ctx->last_out_hi[0] = (const char *) (rsurf + (size_t) L * pitch);
     ctx->last_out_lo[1] = (const char *) scomp; ctx->last_out_hi[1] = scomp ? (const char *) (scomp + 4 * (size_t) L * pitch) : NULL;

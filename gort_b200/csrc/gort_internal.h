@@ -41,11 +41,11 @@ struct gort_ctx {
     unsigned long long epoch;          // per-wavelength launches so far
     unsigned long long call_no;        // BRDF calls so far
     unsigned long long last_sig[8];    // kernel kind, grid shape and output identity of the previous per-wavelength launch
-    cudaStream_t last_stream;          // stream of the previous BRDF call (must stay alive until the next call or gort_synchronize)
+    cudaStream_t last_stream;          // stream of the previous call (must stay alive until the next call or gort_synchronize)
     int last_was_wide;                 // the previous operation this context enqueued was a per-wavelength kernel
     int overlap;                       // gort_set_overlap: consecutive same-shape BRDF calls may overlap on the GPU
     const char *last_out_lo[3], *last_out_hi[3];   // byte ranges of the previous call's rsurf / scomp / kprop
-    cudaEvent_t xstream_ev;            // orders BRDF calls issued on different streams
+    cudaEvent_t xstream_ev;            // orders calls issued on different streams (order_after_previous)
     struct { int key_lpt, key_scomp, key_minb, key_wl, key_threads; int occ; } wide_plan[8];
     int n_wide_plan;
     int geom_carveout_set, rows_attr_set, lut_attr_set;
@@ -76,6 +76,9 @@ void *rec_buffer(gort_ctx *ctx, int which, size_t bytes);
 void *tab_buffer(gort_ctx *ctx, int which, size_t bytes);
 // any non-BRDF work this context enqueues ends the "previous operation was a per-wavelength kernel" state
 inline void note_other_work(gort_ctx *ctx) { ctx->last_was_wide = 0; }
+// every entry point calls this before it enqueues anything on `s`: consecutive calls on one context run one after the
+// other whatever streams they use (they share the workspace, the record buffers and the pipeline flags)
+int order_after_previous(gort_ctx *ctx, cudaStream_t s);
 
 // kernels (device pointers, async on `s`)
 int launch_brdf(gort_ctx *ctx, cudaStream_t s, const gort_shape &sh, const double *structure,

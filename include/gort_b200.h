@@ -23,8 +23,11 @@
  *     The reference convention (print to stderr, exit(EXIT_FAILURE)) is kept by the gortt CLI,
  *     not by the library.
  *   - There is no CPU fallback: without a CUDA device gort_create() fails.
- *   - One CUDA stream per context at a time.  By default every call is ordered on its stream like any other CUDA
- *     work.  A caller-supplied stream must stay alive until the next call on another stream or gort_synchronize().
+ *   - Consecutive calls on one context run one after the other, whatever streams they use: a call on another stream
+ *     than the previous call's waits for the work enqueued on that stream (the calls share the context's device
+ *     scratch), and gort_synchronize() waits for every call.  So the previous call's stream must stay alive until the
+ *     next call or gort_synchronize(); the Python binding's callers pass streams of a pool that never destroys them,
+ *     so they meet this.  To run work concurrently, use two contexts.
  *   - gort_set_overlap(ctx, 1) (off by default) lets CONSECUTIVE gort_brdf_batch_dev calls of the same shape into the
  *     same output buffers overlap on the GPU: the geometry kernel of call i+1 runs under the store phase of call i;
  *     the stores of call i+1 to a region start only after call i's stores to that region are complete, so the

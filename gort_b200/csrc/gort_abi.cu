@@ -53,7 +53,6 @@ static void *grow(gort_ctx *ctx, void **p, size_t *cap, size_t bytes)
 void *scratch(gort_ctx *ctx, int slot, size_t bytes) { return grow(ctx, &ctx->scratch[slot], &ctx->scratch_cap[slot], bytes); }
 void *workspace(gort_ctx *ctx, size_t bytes) { return grow(ctx, &ctx->work, &ctx->work_cap, bytes); }
 void *rec_buffer(gort_ctx *ctx, int which, size_t bytes) { return grow(ctx, &ctx->rec_buf[which], &ctx->rec_cap[which], bytes); }
-void *tab_buffer(gort_ctx *ctx, int which, size_t bytes) { return grow(ctx, &ctx->tab_buf[which], &ctx->tab_cap[which], bytes); }
 
 int order_after_previous(gort_ctx *ctx, cudaStream_t s)
 {
@@ -114,11 +113,6 @@ int gort_create(int device, gort_ctx **out)
         rc = set_error(ctx, GORT_ERR_NOMEM, "cudaMalloc of the pipeline flags failed");
     if (rc == GORT_OK) rc = check_cuda(ctx, cudaMemsetAsync(ctx->d_done, 0, sizeof(unsigned long long) * (GORT_MAX_WIDE_CTAS + 1), ctx->stream), "pipeline flags");
     if (rc == GORT_OK) rc = check_cuda(ctx, cudaEventCreateWithFlags(&ctx->xstream_ev, cudaEventDisableTiming), "cudaEventCreate");
-    ctx->dbg_no_pdl = getenv("GORT_NO_PDL") ? 1 : 0;
-    ctx->dbg_no_tma = getenv("GORT_NO_TMA") ? 1 : 0;
-    ctx->dbg_rows_on = getenv("GORT_ROWS") ? 1 : 0;
-    ctx->dbg_table_on = getenv("GORT_WIDE_TABLE") ? 1 : 0;
-    ctx->dbg_rows = getenv("GORT_ROWS_DBG") ? atoi(getenv("GORT_ROWS_DBG")) : 0;
     ctx->dbg_timeline = getenv("GORT_TIMELINE") ? atoi(getenv("GORT_TIMELINE")) : 0;
     if (rc == GORT_OK) rc = launch_gauleg(ctx, ctx->stream, ctx->d_gauleg);
     if (rc == GORT_OK) rc = launch_tav_tables(ctx, ctx->stream, ctx->d_prospect);
@@ -142,7 +136,6 @@ void gort_destroy(gort_ctx *ctx)
     if (ctx->work) cudaFree(ctx->work);
     for (int i = 0; i < 2; i++) {
         if (ctx->rec_buf[i]) cudaFree(ctx->rec_buf[i]);
-        if (ctx->tab_buf[i]) cudaFree(ctx->tab_buf[i]);
         if (ctx->d_flags[i]) cudaFree(ctx->d_flags[i]);
     }
     if (ctx->d_done) cudaFree(ctx->d_done);

@@ -17,9 +17,29 @@
 #include "gort_device.cuh"
 #include "gort_internal.h"
 #include "gort_rsurf_wide.cuh"
-#include "gort_rsurf_rows.cuh"
 
 namespace gort {
+
+// The packed record of `line` (angles index `a` of `na` per angle) and its kprop row.  Flags bit0: the sun of this line
+// differs from the previous line's (every sun-dependent term is a function of |sza| and the set only); bit1: first line
+// of a parameter set.
+__device__ __forceinline__ void store_record(const GeomRec& r, long line, int n_geom, const double* __restrict__ angles,
+                                             long na, long a, double* __restrict__ rec, double* __restrict__ kprop)
+{
+    int flags = 0;
+    if (line % n_geom == 0) flags = 3;
+    else if (fabs(angles[2 * na + a]) != fabs(angles[2 * na + a - 1])) flags = 1;
+    double2* o = reinterpret_cast<double2*>(rec + (size_t) line * GORT_REC_STRIDE);
+    o[0] = make_double2(r.cA, r.Kc);   o[1] = make_double2(r.cG, r.cZ);
+    o[2] = make_double2(r.Kt, __longlong_as_double((long long) flags));
+    o[3] = make_double2(r.q, r.fd);
+    o[4] = make_double2(r.mus, r.t0);  o[5] = make_double2(r.tp0, r.pe_s);
+    o[6] = make_double2(r.Kpg, r.Kpz); o[7] = make_double2(r.Kg, r.Kz);
+    if (kprop) {
+        kprop[4 * line + 0] = r.Kc; kprop[4 * line + 1] = r.Kg;
+        kprop[4 * line + 2] = r.Kt; kprop[4 * line + 3] = r.Kz;
+    }
+}
 
 // ------------------------------------------------------------------------------------------------
 // geom_kernel: one CTA = 32 lines x 5 role warps.  A line's record is ~4200 dependent SASS instructions
@@ -32,34 +52,19 @@ namespace gort {
 //   warp 3  exp terms of Kz / K'g / t0 and the mutual-shadowing beta     gortt.c:439-449, gortt_brdf.c:223-232
 //   warp 4  zenith interpolation of the LUT and the Kuusk hotspot        gortt.c:872-915, gortt_brdf.c:638-702
 #define GEOM_ROLES 5
-// The first `n_tiles` CTAs of a geometry kernel do not compute line records: they fill the (set, lambda) table the
-// full-spectrum per-wavelength kernel loads (gort_rsurf_rows.cuh) and publish one flag per tile.  n_tiles = 0: none.
-struct TableJob {
-    int n_tiles, n_wl, spectra_per_set, ncolt;
-    const double *rleaf, *tleaf, *rsoil;
-    double *table;
-    unsigned long long *flags;          // one per tile
-};
-
 __global__ void __launch_bounds__(32 * GEOM_ROLES)
 geom_kernel(int n_sets, int n_geom, int geom_per_set, gort_options opt,
             const double* __restrict__ structure, const double* __restrict__ lut,
             const double* __restrict__ angles, double* __restrict__ rec, double* __restrict__ kprop,
-            unsigned long long* __restrict__ tile_flags, unsigned long long call_no, const TableJob tj)
+            unsigned long long* __restrict__ tile_flags, unsigned long long call_no)
 {
     // let the dependent per-wavelength kernel start its prologue while this grid runs: it never waits for this
     // grid's completion, it acquires the per-tile flags published below
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-    if ((int) blockIdx.x < tj.n_tiles) {
-        leaf_table_tile(blockIdx.x, n_sets, tj.n_wl, tj.spectra_per_set, tj.ncolt, structure, lut, tj.rleaf, tj.tleaf,
-                        tj.rsoil, tj.table, tj.flags, call_no);
-        return;
-    }
-    const unsigned gblock = blockIdx.x - tj.n_tiles;
     __shared__ double ex[12][32];
     const long L = (long) n_sets * n_geom;
     const int lane = threadIdx.x & 31, role = threadIdx.x >> 5;
-    const long line_raw = (long) gblock * 32 + lane;
+    const long line_raw = (long) blockIdx.x * 32 + lane;
     const long line = min(line_raw, L - 1);
     const int m = (int) (line / n_geom);
     const long a = geom_per_set ? line : (line - (long) m * n_geom);
@@ -105,28 +110,14 @@ geom_kernel(int n_sets, int n_geom, int geom_per_set, gort_options opt,
     h.kuusk = ex[6][lane]; h.pn0_s = ex[7][lane]; h.pe_s = ex[8][lane];
     const double fd = opt.use_fd ? opt.fd : cos(g.sza) / (cos(g.sza) + 0.09);       // gortt.c:290-291
     const GeomRec r = geom_combine(c, P, pa, ex[0][lane], ex[1][lane], tl, h, g.raa, fd);
-    // flags bit0: the sun of this line differs from the previous line's (every sun-dependent term is a
-    // function of |sza| and the set only); bit1: first line of a parameter set
-    int flags = 0;
-    if (line % n_geom == 0) flags = 3;
-    else if (fabs(angles[2 * na + a]) != fabs(angles[2 * na + a - 1])) flags = 1;
-    double2* o = reinterpret_cast<double2*>(rec + (size_t) line * GORT_REC_STRIDE);
-    o[0] = make_double2(r.cA, r.Kc);   o[1] = make_double2(r.cG, r.cZ);
-    o[2] = make_double2(r.Kt, __longlong_as_double((long long) flags));
-    o[3] = make_double2(r.q, r.fd);
-    o[4] = make_double2(r.mus, r.t0);  o[5] = make_double2(r.tp0, r.pe_s);
-    o[6] = make_double2(r.Kpg, r.Kpz); o[7] = make_double2(r.Kg, r.Kz);
-    if (kprop) {
-        kprop[4 * line + 0] = r.Kc; kprop[4 * line + 1] = r.Kg;
-        kprop[4 * line + 2] = r.Kt; kprop[4 * line + 3] = r.Kz;
-    }
+    store_record(r, line, n_geom, angles, na, a, rec, kprop);
     }
     // publish this tile: the per-wavelength kernel waits on these flags, not on the completion of this grid (a
     // grid launched as a programmatic dependent is not complete before its predecessors in the stream are)
     __syncwarp();
     if (lane == 0) {
         __threadfence();
-        asm volatile("st.release.gpu.global.u64 [%0], %1;" :: "l"(tile_flags + gblock), "l"(call_no) : "memory");
+        asm volatile("st.release.gpu.global.u64 [%0], %1;" :: "l"(tile_flags + blockIdx.x), "l"(call_no) : "memory");
     }
 }
 
@@ -139,16 +130,11 @@ __global__ void __launch_bounds__(128, 6)
 geom_lines_kernel(int n_sets, int n_geom, int geom_per_set, gort_options opt,
                   const double* __restrict__ structure, const double* __restrict__ lut,
                   const double* __restrict__ angles, double* __restrict__ rec, double* __restrict__ kprop,
-                  unsigned long long* __restrict__ tile_flags, unsigned long long call_no, const TableJob tj)
+                  unsigned long long* __restrict__ tile_flags, unsigned long long call_no)
 {
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-    if ((int) blockIdx.x < tj.n_tiles) {
-        leaf_table_tile(blockIdx.x, n_sets, tj.n_wl, tj.spectra_per_set, tj.ncolt, structure, lut, tj.rleaf, tj.tleaf,
-                        tj.rsoil, tj.table, tj.flags, call_no);
-        return;
-    }
     const long L = (long) n_sets * n_geom;
-    const long line = (long) (blockIdx.x - tj.n_tiles) * blockDim.x + threadIdx.x;
+    const long line = (long) blockIdx.x * blockDim.x + threadIdx.x;
     if (line < L) {
         const int m = (int) (line / n_geom);
         const long a = geom_per_set ? line : (line - (long) m * n_geom);
@@ -157,19 +143,7 @@ geom_lines_kernel(int n_sets, int n_geom, int geom_per_set, gort_options opt,
         const Line g = line_from_degrees(angles[0 * na + a], angles[1 * na + a], angles[2 * na + a], angles[3 * na + a]);
         const double fd = opt.use_fd ? opt.fd : cos(g.sza) / (cos(g.sza) + 0.09);       // gortt.c:290-291
         const GeomRec r = geom_record(c, lut + (size_t) m * GORT_LUT_STRIDE, opt, g.vza, g.sza, g.raa, fd);
-        int flags = 0;
-        if (line % n_geom == 0) flags = 3;
-        else if (fabs(angles[2 * na + a]) != fabs(angles[2 * na + a - 1])) flags = 1;
-        double2* o = reinterpret_cast<double2*>(rec + (size_t) line * GORT_REC_STRIDE);
-        o[0] = make_double2(r.cA, r.Kc);   o[1] = make_double2(r.cG, r.cZ);
-        o[2] = make_double2(r.Kt, __longlong_as_double((long long) flags));
-        o[3] = make_double2(r.q, r.fd);
-        o[4] = make_double2(r.mus, r.t0);  o[5] = make_double2(r.tp0, r.pe_s);
-        o[6] = make_double2(r.Kpg, r.Kpz); o[7] = make_double2(r.Kg, r.Kz);
-        if (kprop) {
-            kprop[4 * line + 0] = r.Kc; kprop[4 * line + 1] = r.Kg;
-            kprop[4 * line + 2] = r.Kt; kprop[4 * line + 3] = r.Kz;
-        }
+        store_record(r, line, n_geom, angles, na, a, rec, kprop);
     }
     // a warp is one 32-line tile
     __syncwarp();
@@ -275,17 +249,22 @@ int read_kernel_stamps(gort_ctx *ctx, double *span_us, double *startup_us, doubl
     return GORT_OK;
 }
 
-// what launch_brdf hands to the per-wavelength launchers
+// what launch_brdf hands to the per-wavelength launcher
 struct BrdfPlan {
     long L;
     const double *rec;
-    unsigned long long *flags;      // this call's flag array: geometry tiles, then table tiles
+    unsigned long long *flags;      // this call's flag array, one per 32-line geometry tile
     bool pdl;                       // launch as a programmatic dependent of the geometry kernel
     bool gate;                      // overlap mode: wait per CTA for the previous launch's CTA of the same index
-    const double *table;            // per-call (set, lambda) table for the wide kernel's TMA variants, or NULL
-    int tab_ncol;
-    long tab_flag_base;
 };
+
+// columns written per row: the spectrum, plus -- when the caller's pitch leaves room -- the padding up to the end of the
+// row's last 128-byte line (16 doubles), so that no row ends in a partially written line
+static int written_columns(int n_wl, long pitch)
+{
+    const long padded = (long) (n_wl + 15) / 16 * 16;
+    return (int) (pitch % 16 == 0 ? (padded < pitch ? padded : pitch) : n_wl);
+}
 
 // chunking of the wide kernel for a given variant: as few wavelength chunks as possible with <= pick threads per CTA
 static void wide_chunking(int n_col, int lpt, int pick, int *n_chunks, int *threads)
@@ -295,23 +274,20 @@ static void wide_chunking(int n_col, int lpt, int pick, int *n_chunks, int *thre
     *threads = ((t + 31) / 32) * 32;
 }
 
-template <int LPT, bool SCOMP, int MINB, int TMAB, bool TAB = false>
+template <int LPT, bool SCOMP, int TMAB>
 static int launch_wide(gort_ctx *ctx, cudaStream_t s, const gort_shape &sh, const BrdfPlan &pl, const double *structure,
                        const double *lut, const double *rleaf, const double *tleaf,
                        const double *rsoil, double *rsurf, double *scomp)
 {
     const long L = pl.L;
-    // columns written per row: the spectrum, plus -- when the caller's pitch leaves room -- the padding up to
-    // the end of the row's last 128-byte line (16 doubles), so that no row ends in a partially written line
     const long pitch_ = sh.out_pitch > 0 ? sh.out_pitch : sh.n_wl;
-    const int n_col = (int) (pitch_ % 16 == 0 ? ((long) (sh.n_wl + 15) / 16 * 16 < pitch_ ? (long) (sh.n_wl + 15) / 16 * 16 : pitch_) : sh.n_wl);
+    const int n_col = written_columns(sh.n_wl, pitch_);
     // wavelength chunks: as few as possible with <= WIDE_PICK_THREADS threads per CTA, lanes spread evenly
     // block size cap: with the TMA row ring two CTAs must still fit an SM's shared memory
     const int pick = TMAB > 0 ? WIDE_PICK_THREADS_TMA : WIDE_PICK_THREADS;
     int n_chunks, threads;
     wide_chunking(n_col, LPT, pick, &n_chunks, &threads);
     WideArgs a;
-    a.table = TAB ? pl.table : NULL; a.tab_ncol = pl.tab_ncol; a.tab_flag_base = pl.tab_flag_base;
     a.n_sets = sh.n_sets; a.n_geom = sh.n_geom; a.n_wl = sh.n_wl; a.spectra_per_set = sh.spectra_per_set;
     a.chunk = LPT * threads;
     a.n_col = n_col;
@@ -325,12 +301,12 @@ static int launch_wide(gort_ctx *ctx, cudaStream_t s, const gort_shape &sh, cons
     constexpr int RINGW = SCOMP ? 5 : 1;                  // doubles per evaluation in the output ring
     const size_t smem = sizeof(double2) * 8 * STAGE + sizeof(unsigned) * 4
                       + sizeof(double) * (WIDE_NLEAF + 2 * TMAB * RINGW) * (size_t) a.chunk;
-    auto kern = rsurf_wide_kernel<LPT, SCOMP, MINB, TMAB, TAB>;
+    auto kern = rsurf_wide_kernel<LPT, SCOMP, TMAB>;
     // occupancy of this (variant, block size) is looked up once per context
     int occ = 0;
     for (int i = 0; i < ctx->n_wide_plan; i++) {
         auto &wp = ctx->wide_plan[i];
-        if (wp.key_lpt == LPT && wp.key_scomp == (int) SCOMP + 2 * TMAB + 16 * (int) TAB && wp.key_minb == MINB && wp.key_threads == threads) occ = wp.occ;
+        if (wp.key_lpt == LPT && wp.key_scomp == (int) SCOMP && wp.key_tmab == TMAB && wp.key_threads == threads) occ = wp.occ;
     }
     if (occ == 0) {
         // allow the largest chunk any block size can ask for, so that the attribute never shrinks
@@ -342,7 +318,7 @@ static int launch_wide(gort_ctx *ctx, cudaStream_t s, const gort_shape &sh, cons
         if (e != cudaSuccess || occ < 1) occ = 1;
         if (ctx->n_wide_plan < 8) {
             auto &wp = ctx->wide_plan[ctx->n_wide_plan++];
-            wp.key_lpt = LPT; wp.key_scomp = (int) SCOMP + 2 * TMAB + 16 * (int) TAB; wp.key_minb = MINB; wp.key_threads = threads; wp.key_wl = sh.n_wl; wp.occ = occ;
+            wp.key_lpt = LPT; wp.key_scomp = (int) SCOMP; wp.key_tmab = TMAB; wp.key_threads = threads; wp.occ = occ;
         }
     }
     // one resident wave: grid.y contiguous line ranges so that n_chunks * grid.y ~ SMs * occupancy
@@ -373,71 +349,6 @@ static int launch_wide(gort_ctx *ctx, cudaStream_t s, const gort_shape &sh, cons
     if (a.tl) { ctx->stamps_ncta = n_chunks * (int) nby; ctx->stamps_half = (int) (a.epoch & 1); ctx->stamps_stream = s; }
     if (a.tl) timeline_report(ctx, s, n_chunks * (int) nby, (int) (a.epoch & 1), "rsurf_wide_kernel");
     return check_cuda(ctx, e, "rsurf_wide_kernel launch");
-}
-
-// ---- full-spectrum kernel (gort_rsurf_rows.cuh) -------------------------------------------------------------------
-struct RowsShape { bool ok; int n_col, ncolt, threads, tiles_per_set; size_t smem, tab_doubles; long lines_per_cta, grid; };
-
-static RowsShape rows_shape(const gort_ctx *ctx, const gort_shape &sh, long L, const double *rsurf, const double *scomp)
-{
-    RowsShape r = {};
-    const long pitch = sh.out_pitch > 0 ? sh.out_pitch : sh.n_wl;
-    // EXPERIMENTAL, off unless GORT_ROWS=1: measured on C2 the kernel is correct (same bits as the chunked kernel) but
-    // slower -- 50 us isolated against 43.6 us: with its 153 KB table a single CTA fits an SM, so nothing overlaps its
-    // start-up (table load 3.6 us) and the (sun, lambda) terms of every new run (2 us each); see DESIGN.md 4.1
-    if (scomp || !ctx->dbg_rows_on || ctx->dbg_no_tma || pitch % 16 != 0 || ((size_t) rsurf & 15) != 0) return r;
-    const long padded = (long) (sh.n_wl + 15) / 16 * 16;
-    r.n_col = (int) (padded < pitch ? padded : pitch);
-    r.threads = ((r.n_col + 3) / 4 + 31) / 32 * 32;
-    r.ncolt = 4 * r.threads;
-    if (r.threads > ROWS_MAX_THREADS || r.threads < 256) return r;      // 1024 .. 2176 columns
-    if (L < 2L * ctx->sm_count) return r;                               // few lines: the chunked kernel spreads them better
-    r.tab_doubles = (size_t) sh.n_sets * ROWS_NLEAF * r.ncolt;
-    if (r.tab_doubles * sizeof(double) > ((size_t) 1 << 30)) return r;
-    r.tiles_per_set = r.ncolt / ROWS_TAB_TILE;
-    r.smem = sizeof(double) * (size_t) (ROWS_NLEAF + ROWS_NBUF) * r.ncolt + 128 * (size_t) ROWS_STAGE_LINES + 8 * (1 + 2 * ROWS_NBUF);
-    long nct = ctx->sm_count < L ? ctx->sm_count : L;
-    r.lines_per_cta = (L + nct - 1) / nct;
-    r.grid = (L + r.lines_per_cta - 1) / r.lines_per_cta;
-    r.ok = true;
-    return r;
-}
-
-static int launch_rows(gort_ctx *ctx, cudaStream_t s, const gort_shape &sh, const BrdfPlan &pl, const RowsShape &rs,
-                       const double *lut, const double *table, long tab_flag_base, double *rsurf)
-{
-    if (!ctx->rows_attr_set) {
-        const size_t smem_max = sizeof(double) * (size_t) (ROWS_NLEAF + ROWS_NBUF) * 4 * ROWS_MAX_THREADS + 128 * (size_t) ROWS_STAGE_LINES + 8 * (1 + 2 * ROWS_NBUF);
-        cudaError_t e = cudaFuncSetAttribute(rsurf_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem_max);
-        if (e != cudaSuccess) return check_cuda(ctx, e, "rsurf_rows_kernel shared memory");
-        ctx->rows_attr_set = 1;
-    }
-    RowsArgs a;
-    a.n_sets = sh.n_sets; a.n_geom = sh.n_geom; a.n_wl = sh.n_wl; a.spectra_per_set = sh.spectra_per_set;
-    a.n_col = rs.n_col; a.ncolt = rs.ncolt;
-    a.pdl = pl.pdl ? 1 : 0;
-    a.dbg = ctx->dbg_rows;
-    a.flags = pl.flags; a.tab_flag_base = tab_flag_base; a.call_no = ctx->call_no;
-    a.fault = ctx->d_done + GORT_MAX_WIDE_CTAS; a.done = ctx->d_done;
-    a.pitch = sh.out_pitch > 0 ? sh.out_pitch : sh.n_wl;
-    a.lines_per_cta = rs.lines_per_cta;
-    a.lut = lut; a.rec = pl.rec; a.table = table; a.rsurf = rsurf;
-    a.epoch = ++ctx->epoch;
-    a.tl = timeline_half(ctx, a.epoch);
-    a.wait_target = pl.gate ? a.epoch - 1 : 0;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned) rs.grid);
-    cfg.blockDim = dim3((unsigned) rs.threads + 32);      // compute warps + the store warp
-    cfg.dynamicSmemBytes = rs.smem;
-    cfg.stream = s;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = pl.pdl ? 1 : 0;
-    cudaError_t e = cudaLaunchKernelEx(&cfg, rsurf_rows_kernel, a);
-    if (a.tl) timeline_report(ctx, s, (int) rs.grid, (int) (a.epoch & 1), "rsurf_rows_kernel");
-    return check_cuda(ctx, e, "rsurf_rows_kernel launch");
 }
 
 static bool ranges_overlap(const void *p, const char *lo, const char *hi)
@@ -475,48 +386,26 @@ int launch_brdf(gort_ctx *ctx, cudaStream_t s, const gort_shape &sh, const doubl
     // every path stores a { C, G, T, Z } quadruple as one vector: double4 in rsurf_flat_kernel, double2 pairs or bulk
     // copies in the wide kernel
     if (((size_t) scomp & 31) != 0) return set_error(ctx, GORT_ERR_INVALID, "gort_brdf: scomp must be 32-byte aligned");
-    const bool use_pdl = !ctx->dbg_no_pdl;
     // a call on another stream than the previous one has been ordered after it by the entry point (order_after_previous),
     // which also ended the previous call's claim to overlap
     ctx->call_no++;
-    // line records, the (set, lambda) table and the ready flags are double-buffered by call parity: this call's
-    // geometry kernel may run while the previous call's per-wavelength kernel still reads its own
+    // line records and their ready flags are double-buffered by call parity: this call's geometry kernel may run while
+    // the previous call's per-wavelength kernel still reads its own
     ctx->rec_idx ^= 1;
     const int bi = ctx->rec_idx;
-    const RowsShape rs = sh.n_wl >= 64 ? rows_shape(ctx, sh, L, rsurf, scomp) : RowsShape{};
     const size_t geom_tiles = (size_t) ((L + 31) / 32);
-    // EXPERIMENTAL, off unless GORT_WIDE_TABLE=1: the wide kernel's TMA variants can take their (set, lambda) table from the
-    // geometry kernel's spare CTAs instead of computing it per CTA.  Measured on C2: 45.1 us per launch against 43.8 us,
-    // 41.1 us per overlapped step against 36.6 us -- the per-CTA computation runs under the previous CTA's stores for free,
-    // the table copy competes with them for L2 (DESIGN.md 4.1)
-    int wt_ncol = 0;
-    if (ctx->dbg_table_on && !rs.ok && sh.n_wl >= 64 && !ctx->dbg_no_tma && pitch % 16 == 0 && ((size_t) rsurf & 15) == 0 && ((size_t) scomp & 15) == 0) {
-        const long padded = (long) (sh.n_wl + 15) / 16 * 16;
-        const int n_col = (int) (padded < pitch ? padded : pitch);
-        int nc, thr;
-        wide_chunking(n_col, scomp ? 2 : 4, WIDE_PICK_THREADS_TMA, &nc, &thr);
-        const int chunk = (scomp ? 2 : 4) * thr;
-        if (chunk % 128 == 0 && (size_t) sh.n_sets * WIDE_NLEAF * nc * chunk * sizeof(double) <= ((size_t) 256 << 20)) wt_ncol = nc * chunk;
-    }
-    const int tab_ncol = rs.ok ? rs.ncolt : wt_ncol;
-    const size_t tab_tiles = tab_ncol ? (size_t) sh.n_sets * (tab_ncol / ROWS_TAB_TILE) : 0;
     {
-        int rc = ensure_flags(ctx, s, bi, geom_tiles + tab_tiles);
+        int rc = ensure_flags(ctx, s, bi, geom_tiles);
         if (rc != GORT_OK) return rc;
     }
     double *rec = (double *) rec_buffer(ctx, bi, sizeof(double) * GORT_REC_STRIDE * (size_t) L);
     if (!rec) return GORT_ERR_NOMEM;
-    double *table = NULL;
-    if (tab_ncol) {
-        table = (double *) tab_buffer(ctx, bi, sizeof(double) * (size_t) sh.n_sets * ROWS_NLEAF * tab_ncol);
-        if (!table) return GORT_ERR_NOMEM;
-    }
     cudaEvent_t *ev = (ctx->prof_ev && ctx->prof_n < ctx->prof_cap) ? ctx->prof_ev + 3 * ctx->prof_n : NULL;
     if (ev) { cudaError_t e = cudaEventRecord(ev[0], s); if (e != cudaSuccess) return check_cuda(ctx, e, "cudaEventRecord"); }
     // Cross-call overlap (gort_set_overlap, off by default): if the previous operation this context put on the stream
     // was a per-wavelength kernel of the same kind, shape and outputs (it releases its dependents once it is past its
     // start-up), this call's geometry kernel is launched as a programmatic dependent that never waits: it reads only
-    // this call's inputs and writes only the other record / table / flag buffers and kprop.  Not done if an input of
+    // this call's inputs and writes only the other record / flag buffers and kprop.  Not done if an input of
     // this call aliases an output of the previous call, or kprop aliases anything the previous call still reads or
     // writes.  The caller's side of the contract (nothing else enqueued on the stream in between that writes an
     // input of this call) is stated in include/gort_b200.h.
@@ -525,13 +414,13 @@ int launch_brdf(gort_ctx *ctx, cudaStream_t s, const gort_shape &sh, const doubl
         const void *in[7] = {structure, lut, angles, rleaf, tleaf, rsoil, kprop};
         for (int k = 0; k < 7; k++) for (int r = 0; r < 3; r++) alias |= ranges_overlap(in[k], ctx->last_out_lo[r], ctx->last_out_hi[r]);
     }
-    const unsigned long long sig[8] = {(unsigned long long) sh.n_sets, (unsigned long long) sh.n_geom, (unsigned long long) sh.n_wl,
+    const unsigned long long sig[7] = {(unsigned long long) sh.n_sets, (unsigned long long) sh.n_geom, (unsigned long long) sh.n_wl,
                                        (unsigned long long) pitch, (unsigned long long) (size_t) rsurf, (unsigned long long) (size_t) scomp,
-                                       (unsigned long long) (rs.ok ? 1 : 0), (unsigned long long) (size_t) kprop};
+                                       (unsigned long long) (size_t) kprop};
     bool same = ctx->last_was_wide != 0;
-    for (int k = 0; k < 8; k++) same &= sig[k] == ctx->last_sig[k];
-    for (int k = 0; k < 8; k++) ctx->last_sig[k] = sig[k];
-    const bool early_geom = ctx->overlap && use_pdl && !ev && !ctx->stamps_on && same && !alias && sh.n_wl >= 64;
+    for (int k = 0; k < 7; k++) same &= sig[k] == ctx->last_sig[k];
+    for (int k = 0; k < 7; k++) ctx->last_sig[k] = sig[k];
+    const bool early_geom = ctx->overlap && !ev && !ctx->stamps_on && same && !alias && sh.n_wl >= 64;
     {
         // the per-wavelength kernel that follows needs a large shared-memory carve-out; an SM only changes its
         // carve-out when idle, so ask for the same one here or the dependent kernel's CTAs could not join this
@@ -541,12 +430,6 @@ int launch_brdf(gort_ctx *ctx, cudaStream_t s, const gort_shape &sh, const doubl
             if (e == cudaSuccess) e = cudaFuncSetAttribute(geom_lines_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
             if (e != cudaSuccess) return check_cuda(ctx, e, "geometry kernel carve-out");
             ctx->geom_carveout_set = 1;
-        }
-        TableJob tj = {};
-        if (tab_ncol) {
-            tj.n_tiles = (int) tab_tiles; tj.n_wl = sh.n_wl; tj.spectra_per_set = sh.spectra_per_set; tj.ncolt = tab_ncol;
-            tj.rleaf = rleaf; tj.tleaf = tleaf; tj.rsoil = rsoil; tj.table = table;
-            tj.flags = ctx->d_flags[bi] + geom_tiles;
         }
         cudaLaunchConfig_t cfg = {};
         cfg.stream = s;
@@ -559,15 +442,15 @@ int launch_brdf(gort_ctx *ctx, cudaStream_t s, const gort_shape &sh, const doubl
         const bool by_line = L >= 64L * 4 * ctx->sm_count;
         cudaError_t e;
         if (by_line) {
-            cfg.gridDim = dim3((unsigned) ((L + 127) / 128 + tab_tiles));
+            cfg.gridDim = dim3((unsigned) ((L + 127) / 128));
             cfg.blockDim = dim3(128);
             e = cudaLaunchKernelEx(&cfg, geom_lines_kernel, sh.n_sets, sh.n_geom, sh.geom_per_set, sh.opt,
-                                   structure, lut, angles, rec, kprop, ctx->d_flags[bi], ctx->call_no, tj);
+                                   structure, lut, angles, rec, kprop, ctx->d_flags[bi], ctx->call_no);
         } else {
-            cfg.gridDim = dim3((unsigned) ((L + 31) / 32 + tab_tiles));
+            cfg.gridDim = dim3((unsigned) geom_tiles);
             cfg.blockDim = dim3(32 * GEOM_ROLES);
             e = cudaLaunchKernelEx(&cfg, geom_kernel, sh.n_sets, sh.n_geom, sh.geom_per_set, sh.opt,
-                                   structure, lut, angles, rec, kprop, ctx->d_flags[bi], ctx->call_no, tj);
+                                   structure, lut, angles, rec, kprop, ctx->d_flags[bi], ctx->call_no);
         }
         if (e != cudaSuccess) return check_cuda(ctx, e, "geom_kernel launch");
         ctx->launches++;
@@ -578,43 +461,33 @@ int launch_brdf(gort_ctx *ctx, cudaStream_t s, const gort_shape &sh, const doubl
         // are being recorded (an event between the two launches would time the overlap)
         BrdfPlan pl;
         pl.L = L; pl.rec = rec; pl.flags = ctx->d_flags[bi];
-        pl.pdl = use_pdl && !ev && !ctx->stamps_on;      // events or stamps: plain stream order, so that a launch is separable
+        pl.pdl = !ev && !ctx->stamps_on;      // events or stamps: plain stream order, so that a launch is separable
         pl.gate = early_geom;
-        pl.table = rs.ok ? NULL : table; pl.tab_ncol = tab_ncol; pl.tab_flag_base = (long) geom_tiles;
-        int rc;
-        if (rs.ok) {
-            // full spectrum, aligned rows: one persistent CTA per SM writes whole rows (gort_rsurf_rows.cuh)
-            rc = launch_rows(ctx, s, sh, pl, rs, lut, table, (long) geom_tiles, rsurf);
-        } else {
-            // wavelengths per thread: the value in {4, 3, 2} whose chunking wastes the fewest columns (ties: fewer
-            // chunks, then larger LPT)
-            int lpt = 4;
-            {
-                const long n_col = pitch % 16 == 0 ? ((long) (sh.n_wl + 15) / 16 * 16 < pitch ? (long) (sh.n_wl + 15) / 16 * 16 : pitch) : sh.n_wl;
-                long best_waste = -1; int best_chunks = 0;
-                for (int cand = 4; cand >= 2; cand--) {
-                    const long nc = (n_col + cand * WIDE_PICK_THREADS - 1) / (cand * WIDE_PICK_THREADS);
-                    long thr = (n_col + nc * cand - 1) / (nc * cand);
-                    thr = (thr + 31) / 32 * 32;
-                    const long waste = nc * cand * thr - n_col;
-                    if (best_waste < 0 || waste < best_waste || (waste == best_waste && nc < best_chunks)) { best_waste = waste; best_chunks = (int) nc; lpt = cand; }
-                }
+        // wavelengths per thread: the value in {4, 3, 2} whose chunking wastes the fewest columns (ties: fewer chunks,
+        // then larger LPT)
+        int lpt = 4;
+        {
+            const int n_col = written_columns(sh.n_wl, pitch);
+            long best_waste = -1; int best_chunks = 0;
+            for (int cand = 4; cand >= 2; cand--) {
+                int nc, thr;
+                wide_chunking(n_col, cand, WIDE_PICK_THREADS, &nc, &thr);
+                const long waste = (long) nc * cand * thr - n_col;
+                if (best_waste < 0 || waste < best_waste || (waste == best_waste && nc < best_chunks)) { best_waste = waste; best_chunks = nc; lpt = cand; }
             }
-#define WIDE_ARGS ctx, s, sh, pl, structure, lut, rleaf, tleaf, rsoil, rsurf, scomp
-            // Output path: rows through shared memory and TMA bulk stores (3 rows per CTA barrier, LPT = 4) when the
-            // rows are 128-byte aligned, else per-thread stores
-            const bool tma = !ctx->dbg_no_tma && pitch % 16 == 0 && ((size_t) rsurf & 15) == 0 && ((size_t) scomp & 15) == 0;
-            const bool tab = pl.table != NULL;
-            if (scomp && tma && tab) rc = launch_wide<2, true, 2, WIDE_TMA_ROWS_SCOMP, true>(WIDE_ARGS);
-            else if (scomp && tma) rc = launch_wide<2, true, 2, WIDE_TMA_ROWS_SCOMP>(WIDE_ARGS);
-            else if (scomp) rc = launch_wide<2, true, 2, 0>(WIDE_ARGS);
-            else if (tma && tab) rc = launch_wide<4, false, 2, WIDE_TMA_ROWS, true>(WIDE_ARGS);
-            else if (tma) rc = launch_wide<4, false, 2, WIDE_TMA_ROWS>(WIDE_ARGS);
-            else if (lpt == 4) rc = launch_wide<4, false, 2, 0>(WIDE_ARGS);
-            else if (lpt == 3) rc = launch_wide<3, false, 2, 0>(WIDE_ARGS);
-            else rc = launch_wide<2, false, 2, 0>(WIDE_ARGS);
-#undef WIDE_ARGS
         }
+#define WIDE_ARGS ctx, s, sh, pl, structure, lut, rleaf, tleaf, rsoil, rsurf, scomp
+        // Output path: rows through shared memory and TMA bulk stores (3 rows per CTA barrier, LPT = 4) when the
+        // rows are 128-byte aligned, else per-thread stores
+        const bool tma = pitch % 16 == 0 && ((size_t) rsurf & 15) == 0 && ((size_t) scomp & 15) == 0;
+        int rc;
+        if (scomp && tma) rc = launch_wide<2, true, WIDE_TMA_ROWS_SCOMP>(WIDE_ARGS);
+        else if (scomp) rc = launch_wide<2, true, 0>(WIDE_ARGS);
+        else if (tma) rc = launch_wide<4, false, WIDE_TMA_ROWS>(WIDE_ARGS);
+        else if (lpt == 4) rc = launch_wide<4, false, 0>(WIDE_ARGS);
+        else if (lpt == 3) rc = launch_wide<3, false, 0>(WIDE_ARGS);
+        else rc = launch_wide<2, false, 0>(WIDE_ARGS);
+#undef WIDE_ARGS
         if (rc != GORT_OK) return rc;
     } else {
         const int threads = 128;

@@ -27,31 +27,27 @@ struct gort_ctx {
     double *d_gauleg;      // [2][32] abscissa, weights          (gauleg, gortt_albedo.c:142-198)
     double *d_prospect;    // [9][2101] refractive,k_Cab,k_Car,k_Anth,k_Brown,k_Cw,k_Cm, tav90, tav40
     double *d_soil;        // [4][421] Price EOF vectors
-    // BRDF pipeline state (gort_brdf.cu).  Line records, the (set, lambda) table of the full-spectrum kernel and the
-    // ready flags of both are double-buffered by call parity, so that -- in overlap mode (gort_set_overlap) -- the
-    // geometry kernel of call i+1 can run under the store phase of call i
+    // BRDF pipeline state (gort_brdf.cu).  Line records and their ready flags are double-buffered by call parity, so
+    // that -- in overlap mode (gort_set_overlap) -- the geometry kernel of call i+1 can run under the store phase of call i
     void *rec_buf[2];                  // line records
     size_t rec_cap[2];
-    void *tab_buf[2];                  // (set, lambda) tables [n_sets][9][ncolt]
-    size_t tab_cap[2];
-    unsigned long long *d_flags[2];    // [flag_cap] per buffer: geometry tiles, then table tiles; value = BRDF call number published
+    unsigned long long *d_flags[2];    // [flag_cap] per buffer, one per 32-line tile; value = BRDF call number published
     size_t flag_cap[2];
     int rec_idx;
     unsigned long long *d_done;        // [GORT_MAX_WIDE_CTAS] per-CTA epoch of the last per-wavelength launch it finished; [+1] fault word
     unsigned long long epoch;          // per-wavelength launches so far
     unsigned long long call_no;        // BRDF calls so far
-    unsigned long long last_sig[8];    // kernel kind, grid shape and output identity of the previous per-wavelength launch
+    unsigned long long last_sig[7];    // grid shape and output identity of the previous per-wavelength launch
     cudaStream_t last_stream;          // stream of the previous call (must stay alive until the next call or gort_synchronize)
     int last_was_wide;                 // the previous operation this context enqueued was a per-wavelength kernel
     int overlap;                       // gort_set_overlap: consecutive same-shape BRDF calls may overlap on the GPU
     const char *last_out_lo[3], *last_out_hi[3];   // byte ranges of the previous call's rsurf / scomp / kprop
     cudaEvent_t xstream_ev;            // orders calls issued on different streams (order_after_previous)
-    struct { int key_lpt, key_scomp, key_minb, key_wl, key_threads; int occ; } wide_plan[8];
+    struct { int key_lpt, key_scomp, key_tmab, key_threads; int occ; } wide_plan[8];
     int n_wide_plan;
-    int geom_carveout_set, rows_attr_set, lut_attr_set;
-    // development switches, read once from the environment by gort_create (A/B measurements in DESIGN.md):
-    // GORT_NO_PDL, GORT_NO_TMA, GORT_WIDE_TABLE (experimental per-call table in the chunked kernel), GORT_ROWS (experimental full-spectrum kernel), GORT_ROWS_DBG, GORT_TIMELINE=<call number>
-    int dbg_no_pdl, dbg_no_tma, dbg_rows_on, dbg_timeline, dbg_rows, dbg_table_on;
+    int geom_carveout_set, lut_attr_set;
+    // development switch, read once from the environment by gort_create: GORT_TIMELINE=<call number>
+    int dbg_timeline;
     unsigned long long *d_timeline;
     int timeline_calls;
     int stamps_on, stamps_ncta, stamps_half;       // gort_kernel_stamps
@@ -73,7 +69,6 @@ int check_cuda(gort_ctx *ctx, cudaError_t e, const char *what);
 void *scratch(gort_ctx *ctx, int slot, size_t bytes);
 void *workspace(gort_ctx *ctx, size_t bytes);
 void *rec_buffer(gort_ctx *ctx, int which, size_t bytes);
-void *tab_buffer(gort_ctx *ctx, int which, size_t bytes);
 // any non-BRDF work this context enqueues ends the "previous operation was a per-wavelength kernel" state
 inline void note_other_work(gort_ctx *ctx) { ctx->last_was_wide = 0; }
 // every entry point calls this before it enqueues anything on `s`: consecutive calls on one context run one after the

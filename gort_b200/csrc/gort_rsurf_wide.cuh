@@ -69,21 +69,16 @@ struct WideArgs {
     long lines_per_cta;
     const double *structure, *lut, *rec, *rleaf, *tleaf, *rsoil;
     double *rsurf, *scomp;
-    // optional: the (set, lambda) table built once per call by spare CTAs of the geometry kernel
-    // (leaf_table_tile, gort_rsurf_rows.cuh), [n_sets][9][tab_ncol]; NULL: every CTA computes its own chunk
-    const double *table;
-    int tab_ncol;
-    long tab_flag_base;           // index of the first table-tile flag in tile_flags
 };
 
-template <int LPT, bool SCOMP, int MINB, int TMAB, bool TAB>
-__global__ void __launch_bounds__(WIDE_MAX_THREADS, MINB)
+template <int LPT, bool SCOMP, int TMAB>
+__global__ void __launch_bounds__(WIDE_MAX_THREADS, 2)
 rsurf_wide_kernel(const WideArgs a)
 {
     constexpr int STAGE = WIDE_STAGE_LINES;
 #define WIDE_TL(k) do { if (a.tl && threadIdx.x == 0) { unsigned long long t_; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_)); a.tl[(size_t) (blockIdx.y * gridDim.x + blockIdx.x) * 8 + (k)] = t_; } } while (0)
     WIDE_TL(0);                                                               // CTA entry
-    extern __shared__ double2 smem2[];
+    extern __shared__ __align__(128) double2 smem2[];                        // records of a stage are whole 128-byte lines
     double2* srec = smem2;                                                    // [STAGE][8] packed records
     unsigned* runmask = reinterpret_cast<unsigned*>(srec + 8 * STAGE);   // [STAGE / 32] run-start bits (16 bytes reserved)
     double* leaf = reinterpret_cast<double*>(runmask + 4);                 // [WIDE_NLEAF][chunk], 16-byte aligned
@@ -110,54 +105,9 @@ rsurf_wide_kernel(const WideArgs a)
     double k_open = 0.0, ke = 0.0;
     bool leaf_ready = false;
 
-    // (set, lambda) terms of this chunk into shared memory: copied from the per-call table when there is one (nine
-    // TMA bulk copies on one mbarrier: ~1 us instead of ~2.7 us of FP64 pipe per CTA), else computed here
-    __shared__ unsigned long long s_tab_mbar;
-    unsigned tab_parity = 0;
-    if (TAB && threadIdx.x == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" :: "r"((unsigned) __cvta_generic_to_shared(&s_tab_mbar)) : "memory");
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (TAB) __syncthreads();
+    // (set, lambda) terms of this chunk into shared memory, computed by every CTA: in the steady state this runs under
+    // the co-resident CTA's stores (DESIGN.md 4.1)
     auto fill_leaf = [&](int mm) {
-        if (TAB) {
-            const Canopy c0 = canopy_load(a.structure, a.n_sets, mm, a.lut);
-            k_open = c0.k_open; ke = c0.k_openep;
-            const unsigned mb = (unsigned) __cvta_generic_to_shared(&s_tab_mbar);
-            if (threadIdx.x == 0) {
-                // the table tiles that cover this chunk (128 columns each) must have been published
-                const int tiles_per_set = a.tab_ncol / 128;
-                const long t0 = a.tab_flag_base + (long) mm * tiles_per_set + wbase / 128;
-                for (int t = 0; t < chunk / 128; t++) {
-                    unsigned long long v, c0t = 0, c1t;
-                    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(c0t));
-                    for (;;) {
-                        asm volatile("ld.acquire.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(a.tile_flags + t0 + t) : "memory");
-                        if (v >= a.call_no) break;
-                        __nanosleep(100);
-                        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(c1t));
-                        if (c1t - c0t > 2000000000ull) { *a.fault = a.call_no; s_fault = 1; break; }
-                    }
-                }
-                const unsigned bytes = 8u * (unsigned) chunk;
-                asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" :: "r"(mb), "r"(bytes * WIDE_NLEAF) : "memory");
-                const double* src = a.table + (size_t) mm * WIDE_NLEAF * a.tab_ncol + wbase;
-#pragma unroll
-                for (int q = 0; q < WIDE_NLEAF; q++)
-                    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                                 :: "r"((unsigned) __cvta_generic_to_shared(leaf + (size_t) q * chunk)), "l"(src + (size_t) q * a.tab_ncol),
-                                    "r"(bytes), "r"(mb) : "memory");
-            }
-            if ((threadIdx.x & 31) == 0) {
-                unsigned okw = 0;
-                while (!okw)
-                    asm volatile("{\n .reg .pred p;\n mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n selp.u32 %0, 1, 0, p;\n}"
-                                 : "=r"(okw) : "r"(mb), "r"(tab_parity) : "memory");
-            }
-            __syncwarp();
-            tab_parity ^= 1u;
-            return;
-        }
         const Canopy c = canopy_load(a.structure, a.n_sets, mm, a.lut);
         k_open = c.k_open; ke = c.k_openep;
         const size_t sb = a.spectra_per_set ? (size_t) mm * a.n_wl : 0;

@@ -2,7 +2,7 @@
 
 launch_brdf (gort_b200/csrc/gort_brdf.cu) picks its kernels from the shape of each call: geom_kernel, or geom_lines_kernel
 once there are at least 256 lines per SM; then rsurf_flat_kernel (W < 64) or one of the
-rsurf_wide_kernel<LPT, SCOMP, MINB, TMAB, TAB> instantiations, chosen by the row pitch, the alignment of rsurf and scomp
+rsurf_wide_kernel<LPT, SCOMP, TMAB> instantiations, chosen by the row pitch, the alignment of rsurf and scomp
 and the wavelengths per thread that waste the fewest columns.  Every BRDF case below first asserts, from a torch.profiler
 trace of the call, which kernels ran, so that a later change of the heuristic cannot quietly move a case off the path it
 was written for.  Then it compares with the oracle on sampled lines and checks that the same sets computed alone, or as a
@@ -30,8 +30,8 @@ OPTIONS = [{}, {"beta": 0.3, "fd": 0.8}]      # -beta / -diffuse
 
 # ---- which kernels ran ----------------------------------------------------------------------------------------------
 def kernel_key(name):
-    """A kernel name as the profiler reports it -> 'geom_kernel', 'rsurf_wide_kernel<2,0,2,0,0>', ...  Accepts the
-    demangled spellings '<2, false, 2, 0, false>' and '<(int)2, (bool)0, ...>' and the mangled one."""
+    """A kernel name as the profiler reports it -> 'geom_kernel', 'rsurf_wide_kernel<2,0,0>', ...  Accepts the
+    demangled spellings '<2, false, 0>' and '<(int)2, (bool)0, ...>' and the mangled one."""
     m = re.search(r"([a-z_]+_kernel)I((?:L[ib]\d+E)+)E", name) if name.startswith("_Z") else None
     if m:
         return "%s<%s>" % (m.group(1), ",".join(re.findall(r"L[ib](\d+)E", m.group(2))))
@@ -45,10 +45,10 @@ def kernel_key(name):
 
 
 def test_kernel_key_spellings():
-    want = "rsurf_wide_kernel<2,0,2,0,0>"
-    assert kernel_key("void gort::rsurf_wide_kernel<2, false, 2, 0, false>(gort::WideArgs)") == want
-    assert kernel_key("void gort::rsurf_wide_kernel<(int)2, (bool)0, (int)2, (int)0, (bool)0>(gort::WideArgs)") == want
-    assert kernel_key("_ZN4gort17rsurf_wide_kernelILi2ELb0ELi2ELi0ELb0EEEvNS_8WideArgsE") == want
+    want = "rsurf_wide_kernel<2,0,0>"
+    assert kernel_key("void gort::rsurf_wide_kernel<2, false, 0>(gort::WideArgs)") == want
+    assert kernel_key("void gort::rsurf_wide_kernel<(int)2, (bool)0, (int)0>(gort::WideArgs)") == want
+    assert kernel_key("_ZN4gort17rsurf_wide_kernelILi2ELb0ELi0EEEvNS_8WideArgsE") == want
     assert kernel_key("gort::geom_lines_kernel(int, int, int, gort_options, const double *)") == "geom_lines_kernel"
 
 
@@ -114,17 +114,17 @@ def make_angles(rng, M, G, per_set):
 
 CASES = {
     # name: M, G, W, row pitch (0: dense), scomp, per-set geometry, per-set spectra, rsurf offset in doubles, kernels
-    "lpt2_few_lines":       (4, 3000, 300, 0, False, False, True, 0, "geom_kernel", "rsurf_wide_kernel<2,0,2,0,0>"),
-    "lpt2_many_lines":      (3, 20000, 301, 0, False, False, True, 0, "geom_lines_kernel", "rsurf_wide_kernel<2,0,2,0,0>"),
-    "hyperspectral_tma":    (2000, 16, 211, 224, False, True, True, 0, "geom_kernel", "rsurf_wide_kernel<4,0,2,3,0>"),
-    "hyperspectral_thread": (5000, 16, 211, 0, False, True, True, 0, "geom_lines_kernel", "rsurf_wide_kernel<4,0,2,0,0>"),
-    "signatures_tma":       (1500, 7, 97, 112, True, True, True, 0, "geom_kernel", "rsurf_wide_kernel<2,1,2,2,0>"),
-    "signatures_thread":    (1500, 7, 97, 0, True, True, False, 0, "geom_kernel", "rsurf_wide_kernel<2,1,2,0,0>"),
+    "lpt2_few_lines":       (4, 3000, 300, 0, False, False, True, 0, "geom_kernel", "rsurf_wide_kernel<2,0,0>"),
+    "lpt2_many_lines":      (3, 20000, 301, 0, False, False, True, 0, "geom_lines_kernel", "rsurf_wide_kernel<2,0,0>"),
+    "hyperspectral_tma":    (2000, 16, 211, 224, False, True, True, 0, "geom_kernel", "rsurf_wide_kernel<4,0,3>"),
+    "hyperspectral_thread": (5000, 16, 211, 0, False, True, True, 0, "geom_lines_kernel", "rsurf_wide_kernel<4,0,0>"),
+    "signatures_tma":       (1500, 7, 97, 112, True, True, True, 0, "geom_kernel", "rsurf_wide_kernel<2,1,2>"),
+    "signatures_thread":    (1500, 7, 97, 0, True, True, False, 0, "geom_kernel", "rsurf_wide_kernel<2,1,0>"),
     "bands_geom_lines":     (4000, 16, 7, 0, True, True, True, 0, "geom_lines_kernel", "rsurf_flat_kernel"),
-    "unaligned_rsurf":      (2, 1200, 2101, 2112, False, False, False, 1, "geom_kernel", "rsurf_wide_kernel<4,0,2,0,0>"),
+    "unaligned_rsurf":      (2, 1200, 2101, 2112, False, False, False, 1, "geom_kernel", "rsurf_wide_kernel<4,0,0>"),
     # rows that cannot take TMA with 65..96 (or 96 written) columns: LPT = 3 wastes the fewest columns
-    "lpt3_dense":           (300, 16, 95, 0, False, True, True, 0, "geom_kernel", "rsurf_wide_kernel<3,0,2,0,0>"),
-    "lpt3_padded_unaligned": (2, 1500, 90, 96, False, False, False, 1, "geom_kernel", "rsurf_wide_kernel<3,0,2,0,0>"),
+    "lpt3_dense":           (300, 16, 95, 0, False, True, True, 0, "geom_kernel", "rsurf_wide_kernel<3,0,0>"),
+    "lpt3_padded_unaligned": (2, 1500, 90, 96, False, False, False, 1, "geom_kernel", "rsurf_wide_kernel<3,0,0>"),
 }
 
 
@@ -277,7 +277,7 @@ def test_brdf_dispatch_matrix(gort, oracle, traced, case, opt):
     if case == "unaligned_rsurf":
         # the same rows into an aligned buffer take the bulk-store path: same bits, padding included
         al = run_brdf(gort, traced, x.st, x.lut, x.ang, x.spectra, pitch, want_scomp, 0, opt)
-        assert al["kernels"] == {geom, "rsurf_wide_kernel<4,0,2,3,0>"}, "aligned rows ran %r" % sorted(al["kernels"])
+        assert al["kernels"] == {geom, "rsurf_wide_kernel<4,0,3>"}, "aligned rows ran %r" % sorted(al["kernels"])
         assert np.array_equal(al["rsurf"], full["rsurf"], equal_nan=True)
         assert np.array_equal(al["kprop"], full["kprop"], equal_nan=True)
 

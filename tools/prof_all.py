@@ -33,6 +33,6 @@ G = w2["angles"].shape[1]
 d = [T(w2["structure"]), T(l1), T(w2["angles"]), T(r2[0]), T(t2[0]), T(s2[0])]
 out = torch.empty((1, G, 2112), dtype=torch.float64, device=dev)
 sc = torch.empty((1, G, 2112, 4), dtype=torch.float64, device=dev)
-g.brdf_dev(*d, out); g.synchronize()                 # geom_kernel, rsurf_wide_kernel (TMA rows, per-call table)
+g.brdf_dev(*d, out); g.synchronize()                 # geom_kernel, rsurf_wide_kernel (TMA rows)
 g.brdf_dev(*d, out, scomp=sc); g.synchronize()       # rsurf_wide_kernel with component signatures
 print("ok", np.isfinite(lut).mean(), np.isfinite(a).mean(), np.isfinite(b4).mean(), float(torch.isfinite(sc).double().mean()))

@@ -29,6 +29,7 @@ LUT_FULL, LUT_Q08 = 0, 1
 JAC_LAMBDA, JAC_R, JAC_B, JAC_H1, JAC_H2, JAC_FAVD, JAC_LAI = range(7)
 PROSPECT_NW = 2101
 SOIL_TABLE_NW = 2101
+MAX_BANDS = 64
 
 _LIB_PATH = Path(__file__).resolve().parent / "libgort_b200.so"
 _dp = C.POINTER(C.c_double)
@@ -61,6 +62,8 @@ ABI_SYMBOLS = [
     "gort_energy_batch_dev", "gort_gauleg", "gort_lut_write_text", "gort_lut_read_text",
     "gort_dfma_peak", "gort_profile_begin", "gort_profile_end", "gort_set_overlap", "gort_kernel_stamps_enable", "gort_kernel_stamps",
     "gort_forward_batch", "gort_jacobian_batch", "gort_lut_intermediates_batch", "gort_lut_intermediates_batch_dev", "gort_host_alloc_near", "gort_host_alloc_on_cpus", "gort_host_placement", "gort_soil_table_read", "gort_soil_from_table", "gort_soil_from_table_dev",
+    "gort_brdf_band_batch", "gort_brdf_band_batch_dev", "gort_energy_band_batch", "gort_energy_band_batch_dev",
+    "gort_forward_band_batch",
 ]
 
 
@@ -114,6 +117,11 @@ def load_library():
     lib.gort_energy_batch.argtypes = [vp, sp] + [vp] * 9
     lib.gort_energy_batch_dev.argtypes = [vp, vp, sp] + [vp] * 9
     lib.gort_forward_batch.argtypes = [vp, sp, C.c_int, vp, vp, vp, C.c_double, C.c_double, vp, vp, vp, vp]
+    lib.gort_brdf_band_batch.argtypes = [vp, sp, C.c_int] + [vp] * 8
+    lib.gort_brdf_band_batch_dev.argtypes = [vp, vp, sp, C.c_int] + [vp] * 8
+    lib.gort_energy_band_batch.argtypes = [vp, sp, C.c_int] + [vp] * 10
+    lib.gort_energy_band_batch_dev.argtypes = [vp, vp, sp, C.c_int] + [vp] * 10
+    lib.gort_forward_band_batch.argtypes = [vp, sp, C.c_int, vp, vp, vp, C.c_double, C.c_double, vp, C.c_int, vp, vp, vp, vp]
     lib.gort_jacobian_batch.argtypes = [vp, sp, C.c_int, C.c_int, C.c_double, vp, vp, vp, C.c_double, C.c_double, vp, vp, vp, vp]
     lib.gort_gauleg.argtypes = [vp, vp, vp]
     lib.gort_lut_write_text.argtypes = [vp, vp]
@@ -402,6 +410,48 @@ class Gort:
                                                 _ptr(tl), _ptr(rs), _ptr(alb), _ptr(fv), _ptr(fs)))
         return alb, fv, fs
 
+    # ---- sensor bands: weighted means over spectral response functions (definition: include/gort_b200.h) ----
+    def brdf_band(self, structure, lut, angles, rleaf, tleaf, rsoil, weights, beta=None, fd=None):
+        """brdf() averaged over bands: weights [B][W] (raw SRF values on the spectra's W columns, see band_weights)
+        -> rband [M][G][B]."""
+        st, lut, ang, rl, tl, rs, M, G, W, gps, sps = self._prep(structure, lut, angles, rleaf, tleaf, rsoil)
+        w, B = _band_weights_arg(weights, W)
+        sh = self._shape(M, G, W, gps, sps, beta, fd)
+        rband = np.empty((M, G, B))
+        self._check(self._lib.gort_brdf_band_batch(self._h, C.byref(sh), B, _ptr(w), _ptr(st), _ptr(lut), _ptr(ang),
+                                                   _ptr(rl), _ptr(tl), _ptr(rs), _ptr(rband)))
+        return rband
+
+    def energy_band(self, structure, lut, angles, rleaf, tleaf, rsoil, weights, beta=None, fd=None):
+        """energy() averaged over bands: -> albedo, favegt, fasoil each [M][G][B]."""
+        st, lut, ang, rl, tl, rs, M, G, W, gps, sps = self._prep(structure, lut, angles, rleaf, tleaf, rsoil)
+        w, B = _band_weights_arg(weights, W)
+        sh = self._shape(M, G, W, gps, sps, beta, fd)
+        out = [np.empty((M, G, B)) for _ in range(3)]
+        self._check(self._lib.gort_energy_band_batch(self._h, C.byref(sh), B, _ptr(w), _ptr(st), _ptr(lut), _ptr(ang),
+                                                     _ptr(rl), _ptr(tl), _ptr(rs), *[_ptr(o) for o in out]))
+        return tuple(out)
+
+    def forward_band(self, structure, leaf, soil, wavelength, weights, angles, method=LUT_FULL, user_leaf=-1.0,
+                     user_soil=-1.0, beta=None, fd=None, want_lut=False):
+        """forward() averaged over bands (gort_forward_band_batch): weights [B][W] on wavelength [W] -> rband [M][G][B]
+        (+ LUT records [M][184] with want_lut).  Spectra are computed on the union of the bands' supports only."""
+        st = _np(structure)
+        M = st.shape[1]
+        leaf = None if leaf is None else _np(leaf)
+        soil = None if soil is None else _np(soil)
+        wl = _np(wavelength).ravel()
+        ang = _np(angles)
+        G, W = ang.shape[-1], wl.shape[0]
+        w, B = _band_weights_arg(weights, W)
+        sh = self._shape(M, G, W, ang.ndim == 3, 1, beta, fd)
+        rband = np.empty((M, G, B))
+        lut = np.empty((M, LUT_STRIDE)) if want_lut else None
+        self._check(self._lib.gort_forward_band_batch(self._h, C.byref(sh), method, _ptr(st), _ptr(leaf), _ptr(soil),
+                                                      float(user_leaf), float(user_soil), _ptr(wl), B, _ptr(w),
+                                                      _ptr(ang), _ptr(rband), _ptr(lut)))
+        return (rband, lut) if want_lut else rband
+
     # ---- device API (torch CUDA tensors, float64, contiguous; enqueue only) ----
     def lut_dev(self, structure, out, method=LUT_FULL, stream=None):
         M = structure.shape[1]
@@ -463,6 +513,74 @@ class Gort:
         self._check(self._lib.gort_energy_batch_dev(self._h, stream, C.byref(sh), _ptr(structure), _ptr(lut),
                                                     _ptr(angles), _ptr(rleaf), _ptr(tleaf), _ptr(rsoil),
                                                     _ptr(albedo), _ptr(favegt), _ptr(fasoil)))
+
+    def brdf_band_dev(self, structure, lut, angles, rleaf, tleaf, rsoil, weights, rband, beta=None, fd=None, stream=None):
+        """brdf_band on device tensors: weights [B][W], rband [M][G][B].  A defective weight row gives NaN in its band."""
+        M = structure.shape[1]
+        G, W = angles.shape[-1], rleaf.shape[-1]
+        _check_band_dims(tuple(weights.shape), W)
+        assert tuple(rband.shape) == (M, G, weights.shape[0]), "rband must be [M][G][B]"
+        sh = self._shape(M, G, W, angles.dim() == 3, rleaf.dim() == 2, beta, fd)
+        self._check(self._lib.gort_brdf_band_batch_dev(self._h, stream, C.byref(sh), weights.shape[0], _ptr(weights),
+                                                       _ptr(structure), _ptr(lut), _ptr(angles), _ptr(rleaf),
+                                                       _ptr(tleaf), _ptr(rsoil), _ptr(rband)))
+
+    def energy_band_dev(self, structure, lut, angles, rleaf, tleaf, rsoil, weights, albedo, favegt, fasoil,
+                        beta=None, fd=None, stream=None):
+        M = structure.shape[1]
+        G, W = angles.shape[-1], rleaf.shape[-1]
+        _check_band_dims(tuple(weights.shape), W)
+        for o in (albedo, favegt, fasoil):
+            assert tuple(o.shape) == (M, G, weights.shape[0]), "outputs must be [M][G][B]"
+        sh = self._shape(M, G, W, angles.dim() == 3, rleaf.dim() == 2, beta, fd)
+        self._check(self._lib.gort_energy_band_batch_dev(self._h, stream, C.byref(sh), weights.shape[0], _ptr(weights),
+                                                         _ptr(structure), _ptr(lut), _ptr(angles), _ptr(rleaf),
+                                                         _ptr(tleaf), _ptr(rsoil), _ptr(albedo), _ptr(favegt),
+                                                         _ptr(fasoil)))
+
+
+def _check_band_dims(shape, W):
+    """weights must be [B][W] on the call's grid with 1 <= B <= MAX_BANDS: the library reads B * W doubles"""
+    if len(shape) != 2 or shape[1] != W or not 1 <= shape[0] <= MAX_BANDS:
+        raise ValueError("band weights must be [B][W] with W = %d columns of the call's grid and 1 <= B <= %d, got %s"
+                         % (W, MAX_BANDS, shape))
+
+
+def _band_weights_arg(weights, W):
+    w = _np(weights)
+    _check_band_dims(w.shape, W)
+    return w, w.shape[0]
+
+
+def band_weights(grid, srf_wavelength, srf_response):
+    """Band weights for a call's wavelength grid from tabulated spectral response functions: each SRF is linearly
+    interpolated onto `grid` [W], zero outside its table.  srf_wavelength [n] (ascending) and srf_response [n] give one
+    band; srf_response [B][n] with a shared srf_wavelength, or lists of per-band tables, give B bands.  Returns [B][W]
+    raw weights (the library normalises them).  Host only."""
+    grid = np.asarray(grid, dtype=np.float64).ravel()
+
+    def tables(a):
+        # one table [n], equal-length tables [B][n], or a list of tables of different lengths
+        try:
+            a = np.asarray(a, dtype=np.float64)
+        except ValueError:
+            return [np.asarray(t, dtype=np.float64).ravel() for t in a]
+        return [a] if a.ndim == 1 else list(a)
+
+    resp = tables(srf_response)
+    wls = tables(srf_wavelength)
+    if len(wls) == 1:
+        wls = wls * len(resp)
+    if len(wls) != len(resp):
+        raise ValueError("band_weights: %d wavelength tables for %d responses" % (len(wls), len(resp)))
+    rows = []
+    for x, y in zip(wls, resp):
+        x = np.asarray(x, dtype=np.float64).ravel()
+        y = np.asarray(y, dtype=np.float64).ravel()
+        if x.shape != y.shape or x.size < 1 or np.any(np.diff(x) <= 0):
+            raise ValueError("band_weights: an SRF table needs matching, strictly ascending wavelengths")
+        rows.append(np.interp(grid, x, y, left=0.0, right=0.0))
+    return np.stack(rows)
 
 
 # ---- LUT text files ("-W" / "-P", gortt.c:123-146) ------------------------------------------------

@@ -7,6 +7,7 @@
 #include <string.h>
 #include <math.h>
 #include <sched.h>
+#include <vector>
 #include "gort_internal.h"
 #include "../data/gort_tables.h"
 
@@ -785,6 +786,195 @@ int gort_energy_batch(gort_ctx *ctx, const gort_shape *shape, const double *stru
     TRY(d2h(ctx, favegt, d_v, n));
     TRY(d2h(ctx, fasoil, d_s, n));
     return check_cuda(ctx, cudaStreamSynchronize(ctx->stream), "gort_energy_batch");
+}
+
+// ---- sensor bands ---------------------------------------------------------------------------------
+// host_weights: the rows are on the host and are checked here (the _dev entry points cannot look at device weights)
+static int check_bands(gort_ctx *ctx, const gort_shape *sh, int n_bands, const double *weights, bool host_weights,
+                       const char *who)
+{
+    TRY(check_shape(ctx, sh, who));
+    if (n_bands < 1 || n_bands > GORT_MAX_BANDS)
+        return set_error(ctx, GORT_ERR_INVALID, "%s: n_bands %d outside 1..%d", who, n_bands, GORT_MAX_BANDS);
+    if (!weights) return set_error(ctx, GORT_ERR_INVALID, "%s: weights is NULL", who);
+    if (sh->out_pitch != 0) return set_error(ctx, GORT_ERR_INVALID, "%s: band outputs are dense (out_pitch must be 0)", who);
+    if (!host_weights) return GORT_OK;
+    const size_t W = sh->n_wl;
+    for (int b = 0; b < n_bands; b++) {
+        int positive = 0;
+        for (size_t i = 0; i < W; i++) {
+            const double w = weights[(size_t) b * W + i];
+            if (!isfinite(w) || w < 0.0) return set_error(ctx, GORT_ERR_INVALID, "%s: weight [%d][%zu] is not finite and >= 0", who, b, i);
+            positive |= w > 0.0;
+        }
+        if (!positive) return set_error(ctx, GORT_ERR_INVALID, "%s: band %d has no positive weight", who, b);
+    }
+    return GORT_OK;
+}
+
+int gort_brdf_band_batch_dev(gort_ctx *ctx, void *stream, const gort_shape *shape, int n_bands, const double *weights,
+                             const double *structure, const double *lut, const double *angles, const double *rleaf,
+                             const double *tleaf, const double *rsoil, double *rband)
+{
+    if (!ctx) return GORT_ERR_INVALID;
+    TRY(check_bands(ctx, shape, n_bands, weights, false, "gort_brdf_band_batch"));
+    if (!structure || !lut || !angles || !rleaf || !tleaf || !rsoil || !rband)
+        return set_error(ctx, GORT_ERR_INVALID, "gort_brdf_band_batch: NULL argument");
+    TRYCUDA(ctx, cudaSetDevice(ctx->device), "cudaSetDevice");
+    const cudaStream_t s = pick(ctx, stream);
+    TRY(order_after_previous(ctx, s));
+    return launch_brdf_band(ctx, s, *shape, n_bands, weights, structure, lut, angles, rleaf, tleaf, rsoil, rband);
+}
+
+int gort_brdf_band_batch(gort_ctx *ctx, const gort_shape *shape, int n_bands, const double *weights,
+                         const double *structure, const double *lut, const double *angles, const double *rleaf,
+                         const double *tleaf, const double *rsoil, double *rband)
+{
+    if (!ctx) return GORT_ERR_INVALID;
+    TRY(check_bands(ctx, shape, n_bands, weights, true, "gort_brdf_band_batch"));
+    if (!structure || !lut || !angles || !rleaf || !tleaf || !rsoil || !rband)
+        return set_error(ctx, GORT_ERR_INVALID, "gort_brdf_band_batch: NULL argument");
+    TRYCUDA(ctx, cudaSetDevice(ctx->device), "cudaSetDevice");
+    TRY(order_after_previous(ctx, ctx->stream));
+    Staged d;
+    TRY(stage_inputs(ctx, shape, structure, lut, angles, rleaf, tleaf, rsoil, &d));
+    const size_t n = (size_t) shape->n_sets * shape->n_geom * n_bands;
+    double *d_w, *d_out;
+    TRY(h2d(ctx, 6, weights, (size_t) n_bands * shape->n_wl, &d_w));
+    TRY(dout(ctx, 7, rband, n, &d_out));
+    TRY(launch_brdf_band(ctx, ctx->stream, *shape, n_bands, d_w, d.st, d.lut, d.ang, d.rl, d.tl, d.rs, d_out));
+    TRY(d2h(ctx, rband, d_out, n));
+    TRY(check_cuda(ctx, cudaStreamSynchronize(ctx->stream), "gort_brdf_band_batch"));
+    return check_pipeline_fault(ctx);
+}
+
+int gort_energy_band_batch_dev(gort_ctx *ctx, void *stream, const gort_shape *shape, int n_bands, const double *weights,
+                               const double *structure, const double *lut, const double *angles, const double *rleaf,
+                               const double *tleaf, const double *rsoil, double *albedo, double *favegt, double *fasoil)
+{
+    if (!ctx) return GORT_ERR_INVALID;
+    TRY(check_bands(ctx, shape, n_bands, weights, false, "gort_energy_band_batch"));
+    if (!structure || !lut || !angles || !rleaf || !tleaf || !rsoil || !albedo || !favegt || !fasoil)
+        return set_error(ctx, GORT_ERR_INVALID, "gort_energy_band_batch: NULL argument");
+    TRYCUDA(ctx, cudaSetDevice(ctx->device), "cudaSetDevice");
+    const cudaStream_t s = pick(ctx, stream);
+    TRY(order_after_previous(ctx, s));
+    return launch_energy_band(ctx, s, *shape, n_bands, weights, structure, lut, angles, rleaf, tleaf, rsoil, albedo, favegt, fasoil);
+}
+
+int gort_energy_band_batch(gort_ctx *ctx, const gort_shape *shape, int n_bands, const double *weights,
+                           const double *structure, const double *lut, const double *angles, const double *rleaf,
+                           const double *tleaf, const double *rsoil, double *albedo, double *favegt, double *fasoil)
+{
+    if (!ctx) return GORT_ERR_INVALID;
+    TRY(check_bands(ctx, shape, n_bands, weights, true, "gort_energy_band_batch"));
+    if (!structure || !lut || !angles || !rleaf || !tleaf || !rsoil || !albedo || !favegt || !fasoil)
+        return set_error(ctx, GORT_ERR_INVALID, "gort_energy_band_batch: NULL argument");
+    TRYCUDA(ctx, cudaSetDevice(ctx->device), "cudaSetDevice");
+    TRY(order_after_previous(ctx, ctx->stream));
+    Staged d;
+    TRY(stage_inputs(ctx, shape, structure, lut, angles, rleaf, tleaf, rsoil, &d));
+    const size_t n = (size_t) shape->n_sets * shape->n_geom * n_bands;
+    double *d_w, *d_a, *d_v, *d_s;
+    TRY(h2d(ctx, 6, weights, (size_t) n_bands * shape->n_wl, &d_w));
+    TRY(dout(ctx, 7, albedo, n, &d_a));
+    TRY(dout(ctx, 8, favegt, n, &d_v));
+    TRY(dout(ctx, 9, fasoil, n, &d_s));
+    TRY(launch_energy_band(ctx, ctx->stream, *shape, n_bands, d_w, d.st, d.lut, d.ang, d.rl, d.tl, d.rs, d_a, d_v, d_s));
+    TRY(d2h(ctx, albedo, d_a, n));
+    TRY(d2h(ctx, favegt, d_v, n));
+    TRY(d2h(ctx, fasoil, d_s, n));
+    return check_cuda(ctx, cudaStreamSynchronize(ctx->stream), "gort_energy_band_batch");
+}
+
+// gort_forward_batch with band outputs: the same chunked three-stream pipeline, with the spectra computed on the union U
+// of the bands' supports only (the host compacts wavelengths and weight columns to U before the loop)
+int gort_forward_band_batch(gort_ctx *ctx, const gort_shape *shape, int lut_method, const double *structure,
+                            const double *leaf, const double *soil, double user_leaf, double user_soil,
+                            const double *wavelength, int n_bands, const double *weights,
+                            const double *angles, double *rband, double *lut_out)
+{
+    if (!ctx) return GORT_ERR_INVALID;
+    TRY(check_bands(ctx, shape, n_bands, weights, true, "gort_forward_band_batch"));
+    if (!structure || !wavelength || !angles || !rband || (user_leaf < 0.0 && !leaf) || (user_soil < 0.0 && !soil))
+        return set_error(ctx, GORT_ERR_INVALID, "gort_forward_band_batch: NULL argument");
+    if (lut_method != GORT_LUT_FULL && lut_method != GORT_LUT_Q08)
+        return set_error(ctx, GORT_ERR_INVALID, "gort_forward_band_batch: unknown LUT method %d", lut_method);
+    const size_t M = shape->n_sets, G = shape->n_geom, W = shape->n_wl, B = n_bands;
+    for (size_t i = 0; i < W; i++)
+        if (wavelength[i] < GORT_WL_MIN || wavelength[i] > GORT_WL_MAX)
+            return set_error(ctx, GORT_ERR_RANGE, "wavlength out of range (400-2500)");
+    // union of the supports, in grid order
+    std::vector<size_t> cols;
+    for (size_t i = 0; i < W; i++) {
+        bool any = false;
+        for (size_t b = 0; b < B; b++) any |= weights[b * W + i] > 0.0;
+        if (any) cols.push_back(i);
+    }
+    const size_t U = cols.size();
+    std::vector<double> wl_u(U), w_u(B * U);
+    for (size_t k = 0; k < U; k++) {
+        wl_u[k] = wavelength[cols[k]];
+        for (size_t b = 0; b < B; b++) w_u[b * U + k] = weights[b * W + cols[k]];
+    }
+    TRYCUDA(ctx, cudaSetDevice(ctx->device), "cudaSetDevice");
+    if (!ctx->copy_stream) {
+        TRYCUDA(ctx, cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking), "cudaStreamCreate");
+        TRYCUDA(ctx, cudaStreamCreateWithFlags(&ctx->copy_stream_out, cudaStreamNonBlocking), "cudaStreamCreate");
+        for (int i = 0; i < 6; i++) TRYCUDA(ctx, cudaEventCreateWithFlags(&ctx->fwd_ev[i], cudaEventDisableTiming), "cudaEventCreate");
+    }
+    // streams, chunking and events as gort_forward_batch
+    cudaStream_t A = ctx->stream, Bs = ctx->copy_stream, D = ctx->copy_stream_out;
+    size_t C = (M + 7) / 8;
+    if (C > 16384) C = 16384;
+    if (C < 1024) C = 1024;
+    if (C > M) C = M;
+    const bool per_set_geom = shape->geom_per_set != 0;
+    TRY(order_after_previous(ctx, A));
+    // slots 0-8 and 9-17: the two chunk buffers; 18 the union's wavelengths, 19 shared angles, 20 the union's weights
+    double *d_wl, *d_ang_shared = NULL, *d_w;
+    TRY(h2d(ctx, 18, wl_u.data(), U, &d_wl));
+    if (!per_set_geom) TRY(h2d(ctx, 19, angles, 4 * G, &d_ang_shared));
+    TRY(h2d(ctx, 20, w_u.data(), B * U, &d_w));
+    double *buf[2][9];
+    const size_t sz[9] = {6 * C, 7 * C, 4 * C, per_set_geom ? 4 * C * G : 8, C * GORT_LUT_STRIDE, C * U, C * U, C * U, C * G * B};
+    for (int b = 0; b < 2; b++)
+        for (int k = 0; k < 9; k++) {
+            buf[b][k] = (double *) scratch(ctx, 9 * b + k, sz[k] * sizeof(double));
+            if (!buf[b][k]) return GORT_ERR_NOMEM;
+        }
+    gort_shape sh = *shape;
+    sh.n_wl = (int) U;
+    sh.spectra_per_set = 1;
+    int chunk_no = 0;
+    for (size_t m0 = 0; m0 < M; m0 += C, chunk_no++) {
+        const size_t c = M - m0 < C ? M - m0 : C;
+        const int b = chunk_no & 1;
+        if (chunk_no >= 2) TRYCUDA(ctx, cudaStreamWaitEvent(Bs, ctx->fwd_ev[2 + b], 0), "cudaStreamWaitEvent");
+        TRY(copy_rows(ctx, Bs, buf[b][0], c, structure + m0, M, c, 6, cudaMemcpyHostToDevice, "forward: structure"));
+        if (user_leaf < 0.0) TRY(copy_rows(ctx, Bs, buf[b][1], c, leaf + m0, M, c, 7, cudaMemcpyHostToDevice, "forward: leaf"));
+        if (user_soil < 0.0) TRY(copy_rows(ctx, Bs, buf[b][2], c, soil + m0, M, c, 4, cudaMemcpyHostToDevice, "forward: soil"));
+        if (per_set_geom) TRY(copy_rows(ctx, Bs, buf[b][3], c * G, angles + m0 * G, M * G, c * G, 4, cudaMemcpyHostToDevice, "forward: angles"));
+        TRYCUDA(ctx, cudaEventRecord(ctx->fwd_ev[b], Bs), "cudaEventRecord");
+        TRYCUDA(ctx, cudaStreamWaitEvent(A, ctx->fwd_ev[b], 0), "cudaStreamWaitEvent");
+        if (chunk_no >= 2) TRYCUDA(ctx, cudaStreamWaitEvent(A, ctx->fwd_ev[4 + b], 0), "cudaStreamWaitEvent");
+        sh.n_sets = (int) c;
+        TRY(launch_lut(ctx, A, (int) c, buf[b][0], lut_method, buf[b][4]));
+        TRY(launch_spectra(ctx, A, (int) c, user_leaf < 0.0 ? buf[b][1] : NULL, user_soil < 0.0 ? buf[b][2] : NULL, user_leaf, user_soil,
+                           (int) U, d_wl, buf[b][5], buf[b][6], buf[b][7]));
+        TRY(launch_brdf_band(ctx, A, sh, n_bands, d_w, buf[b][0], buf[b][4], per_set_geom ? buf[b][3] : d_ang_shared,
+                             buf[b][5], buf[b][6], buf[b][7], buf[b][8]));
+        TRYCUDA(ctx, cudaEventRecord(ctx->fwd_ev[2 + b], A), "cudaEventRecord");
+        TRYCUDA(ctx, cudaStreamWaitEvent(D, ctx->fwd_ev[2 + b], 0), "cudaStreamWaitEvent");
+        TRYCUDA(ctx, cudaMemcpyAsync(rband + m0 * G * B, buf[b][8], c * G * B * sizeof(double), cudaMemcpyDeviceToHost, D), "forward: rband");
+        if (lut_out) TRYCUDA(ctx, cudaMemcpyAsync(lut_out + m0 * GORT_LUT_STRIDE, buf[b][4], c * GORT_LUT_STRIDE * sizeof(double), cudaMemcpyDeviceToHost, D), "forward: lut");
+        TRYCUDA(ctx, cudaEventRecord(ctx->fwd_ev[4 + b], D), "cudaEventRecord");
+    }
+    TRYCUDA(ctx, cudaStreamSynchronize(D), "gort_forward_band_batch");
+    TRYCUDA(ctx, cudaStreamSynchronize(Bs), "gort_forward_band_batch");
+    TRYCUDA(ctx, cudaStreamSynchronize(A), "gort_forward_band_batch");
+    note_other_work(ctx);
+    return check_pipeline_fault(ctx);
 }
 
 int gort_gauleg(gort_ctx *ctx, double *abscissa, double *weights)

@@ -11,6 +11,8 @@
 //   rsurf_flat_kernel    W < 64 (band sets): one thread per (line, band).
 //   energy_zenith_kernel / energy_kernel   hemispherical quadrature for albedo / fAPAR (gortt_albedo.c): the
 //                        quadrature collapses onto five weighted sums of node coefficients.
+//   band_support_kernel / brdf_band_kernel / energy_band_kernel   sensor bands: the SRF-weighted mean over wavelengths
+//                        moved onto the (sun, lambda) terms, 5 FP64 instructions per (line, band).
 //   gauleg_kernel, dfma_kernel            Gauss-Legendre nodes; FP64 FMA microbenchmark.
 #include <stdio.h>
 #include <stdlib.h>
@@ -374,6 +376,62 @@ static int ensure_flags(gort_ctx *ctx, cudaStream_t s, int which, size_t n)
     return GORT_OK;
 }
 
+// the record buffer and flag array of a new call: double-buffered by call parity, so that this call's geometry kernel
+// may run while the previous call's per-wavelength kernel still reads its own
+static int next_records(gort_ctx *ctx, cudaStream_t s, long L, double **rec, unsigned long long **flags)
+{
+    ctx->call_no++;
+    ctx->rec_idx ^= 1;
+    const int bi = ctx->rec_idx;
+    int rc = ensure_flags(ctx, s, bi, (size_t) ((L + 31) / 32));
+    if (rc != GORT_OK) return rc;
+    *rec = (double *) rec_buffer(ctx, bi, sizeof(double) * GORT_REC_STRIDE * (size_t) L);
+    if (!*rec) return GORT_ERR_NOMEM;
+    *flags = ctx->d_flags[bi];
+    return GORT_OK;
+}
+
+// geometry records of every line of a call (and kprop when asked for), with their per-tile ready flags.  pdl: launch as a
+// programmatic dependent of the previous kernel on the stream (overlap mode); otherwise plain stream order.
+static int launch_geom(gort_ctx *ctx, cudaStream_t s, const gort_shape &sh, const double *structure, const double *lut,
+                       const double *angles, double *rec, double *kprop, unsigned long long *flags, bool pdl)
+{
+    const long L = (long) sh.n_sets * sh.n_geom;
+    // the per-wavelength kernel that follows needs a large shared-memory carve-out; an SM only changes its
+    // carve-out when idle, so ask for the same one here or the dependent kernel's CTAs could not join this
+    // kernel's CTAs on an SM (measured: without it they entered only as geom_kernel's CTAs left)
+    if (!ctx->geom_carveout_set) {            // per device, so per context
+        cudaError_t e = cudaFuncSetAttribute(geom_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(geom_lines_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+        if (e != cudaSuccess) return check_cuda(ctx, e, "geometry kernel carve-out");
+        ctx->geom_carveout_set = 1;
+    }
+    cudaLaunchConfig_t cfg = {};
+    cfg.stream = s;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = pdl ? 1 : 0;
+    // enough lines to fill the GPU several times over: one thread per line (see geom_lines_kernel)
+    const bool by_line = L >= 64L * 4 * ctx->sm_count;
+    cudaError_t e;
+    if (by_line) {
+        cfg.gridDim = dim3((unsigned) ((L + 127) / 128));
+        cfg.blockDim = dim3(128);
+        e = cudaLaunchKernelEx(&cfg, geom_lines_kernel, sh.n_sets, sh.n_geom, sh.geom_per_set, sh.opt,
+                               structure, lut, angles, rec, kprop, flags, ctx->call_no);
+    } else {
+        cfg.gridDim = dim3((unsigned) ((L + 31) / 32));
+        cfg.blockDim = dim3(32 * GEOM_ROLES);
+        e = cudaLaunchKernelEx(&cfg, geom_kernel, sh.n_sets, sh.n_geom, sh.geom_per_set, sh.opt,
+                               structure, lut, angles, rec, kprop, flags, ctx->call_no);
+    }
+    if (e != cudaSuccess) return check_cuda(ctx, e, "geom_kernel launch");
+    ctx->launches++;
+    return GORT_OK;
+}
+
 int launch_brdf(gort_ctx *ctx, cudaStream_t s, const gort_shape &sh, const double *structure,
                 const double *lut, const double *angles, const double *rleaf, const double *tleaf,
                 const double *rsoil, double *rsurf, double *scomp, double *kprop)
@@ -388,18 +446,12 @@ int launch_brdf(gort_ctx *ctx, cudaStream_t s, const gort_shape &sh, const doubl
     if (((size_t) scomp & 31) != 0) return set_error(ctx, GORT_ERR_INVALID, "gort_brdf: scomp must be 32-byte aligned");
     // a call on another stream than the previous one has been ordered after it by the entry point (order_after_previous),
     // which also ended the previous call's claim to overlap
-    ctx->call_no++;
-    // line records and their ready flags are double-buffered by call parity: this call's geometry kernel may run while
-    // the previous call's per-wavelength kernel still reads its own
-    ctx->rec_idx ^= 1;
-    const int bi = ctx->rec_idx;
-    const size_t geom_tiles = (size_t) ((L + 31) / 32);
+    double *rec;
+    unsigned long long *flags;
     {
-        int rc = ensure_flags(ctx, s, bi, geom_tiles);
+        int rc = next_records(ctx, s, L, &rec, &flags);
         if (rc != GORT_OK) return rc;
     }
-    double *rec = (double *) rec_buffer(ctx, bi, sizeof(double) * GORT_REC_STRIDE * (size_t) L);
-    if (!rec) return GORT_ERR_NOMEM;
     cudaEvent_t *ev = (ctx->prof_ev && ctx->prof_n < ctx->prof_cap) ? ctx->prof_ev + 3 * ctx->prof_n : NULL;
     if (ev) { cudaError_t e = cudaEventRecord(ev[0], s); if (e != cudaSuccess) return check_cuda(ctx, e, "cudaEventRecord"); }
     // Cross-call overlap (gort_set_overlap, off by default): if the previous operation this context put on the stream
@@ -422,45 +474,15 @@ int launch_brdf(gort_ctx *ctx, cudaStream_t s, const gort_shape &sh, const doubl
     for (int k = 0; k < 7; k++) ctx->last_sig[k] = sig[k];
     const bool early_geom = ctx->overlap && !ev && !ctx->stamps_on && same && !alias && sh.n_wl >= 64;
     {
-        // the per-wavelength kernel that follows needs a large shared-memory carve-out; an SM only changes its
-        // carve-out when idle, so ask for the same one here or the dependent kernel's CTAs could not join this
-        // kernel's CTAs on an SM (measured: without it they entered only as geom_kernel's CTAs left)
-        if (!ctx->geom_carveout_set) {            // per device, so per context
-            cudaError_t e = cudaFuncSetAttribute(geom_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-            if (e == cudaSuccess) e = cudaFuncSetAttribute(geom_lines_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-            if (e != cudaSuccess) return check_cuda(ctx, e, "geometry kernel carve-out");
-            ctx->geom_carveout_set = 1;
-        }
-        cudaLaunchConfig_t cfg = {};
-        cfg.stream = s;
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[0].val.programmaticStreamSerializationAllowed = 1;
-        cfg.attrs = attr;
-        cfg.numAttrs = early_geom ? 1 : 0;
-        // enough lines to fill the GPU several times over: one thread per line (see geom_lines_kernel)
-        const bool by_line = L >= 64L * 4 * ctx->sm_count;
-        cudaError_t e;
-        if (by_line) {
-            cfg.gridDim = dim3((unsigned) ((L + 127) / 128));
-            cfg.blockDim = dim3(128);
-            e = cudaLaunchKernelEx(&cfg, geom_lines_kernel, sh.n_sets, sh.n_geom, sh.geom_per_set, sh.opt,
-                                   structure, lut, angles, rec, kprop, ctx->d_flags[bi], ctx->call_no);
-        } else {
-            cfg.gridDim = dim3((unsigned) geom_tiles);
-            cfg.blockDim = dim3(32 * GEOM_ROLES);
-            e = cudaLaunchKernelEx(&cfg, geom_kernel, sh.n_sets, sh.n_geom, sh.geom_per_set, sh.opt,
-                                   structure, lut, angles, rec, kprop, ctx->d_flags[bi], ctx->call_no);
-        }
-        if (e != cudaSuccess) return check_cuda(ctx, e, "geom_kernel launch");
-        ctx->launches++;
+        int rc = launch_geom(ctx, s, sh, structure, lut, angles, rec, kprop, flags, early_geom);
+        if (rc != GORT_OK) return rc;
     }
     if (ev) { cudaError_t e = cudaEventRecord(ev[1], s); if (e != cudaSuccess) return check_cuda(ctx, e, "cudaEventRecord"); }
     if (sh.n_wl >= 64) {
         // programmatic dependent launch: the kernel's prologue overlaps geom_kernel.  Off while per-kernel events
         // are being recorded (an event between the two launches would time the overlap)
         BrdfPlan pl;
-        pl.L = L; pl.rec = rec; pl.flags = ctx->d_flags[bi];
+        pl.L = L; pl.rec = rec; pl.flags = flags;
         pl.pdl = !ev && !ctx->stamps_on;      // events or stamps: plain stream order, so that a launch is separable
         pl.gate = early_geom;
         // wavelengths per thread: the value in {4, 3, 2} whose chunking wastes the fewest columns (ties: fewer chunks,
@@ -582,6 +604,87 @@ energy_zenith_kernel(int n_sets, int n_geom, int geom_per_set, gort_options opt,
     z[ZR_LSZA] = -log(pe_s) / c.kfavd;                                           // gortt_brdf.c:659-660
     z[ZR_LVZA] = -log(pe_v) / c.kfavd;
     z[ZR_FD] = fd; z[ZR_X] = x;
+}
+
+// The coefficient-sum stage of energy_kernel, for energy_band_kernel: the CTA's (set, sun line) node pass, the weighted
+// coefficients and their fixed-order sums into coef[5], the sun values into sunv[6]; returns fd.  The same statements as
+// in energy_kernel, which keeps its own inline copy: calling this function there changed its register allocation and
+// cost it 1 % on C3 (1.021 -> 1.032 ms, B200).
+__device__ __forceinline__ double energy_node_sums(int n_geom, int geom_per_set, long L, long line, int m, const Canopy& c,
+                                                   const double* __restrict__ angles, const double* __restrict__ gl,
+                                                   const double* __restrict__ zrec, double (*part)[GORT_EN_THREADS / 32],
+                                                   double* coef, double* sunv)
+{
+    const long a = geom_per_set ? line : (line - (long) m * n_geom);
+    const long na = geom_per_set ? L : n_geom;
+    const int tid = threadIdx.x;
+    double fd;
+    {
+        const int i = tid & 31, jj = tid >> 5;
+        const double* z = zrec + ((size_t) line * GORT_EN_NZ + jj) * GORT_EN_ZREC;      // same record for the whole warp
+        const double xr = 0.5 * (1. + 1.);
+        const double ym = 0.5 * (2. * GORT_PI - 0.), yr = 0.5 * (2. * GORT_PI + 0.);  // gortt_albedo.c:84-85
+        // azimuth of this node: saa after the reference's normalisation (gortt.c:253-274 via line_from_degrees)
+        const Line g = line_from_degrees(angles[0 * na + a], angles[1 * na + a], angles[2 * na + a], angles[3 * na + a]);
+        double y = ym + yr * gl[i];                                              // :91
+        double vaa = y;
+        for (int it = 0; it < 8 && vaa > 2 * GORT_PI; it++) vaa -= 2 * GORT_PI;  // :96
+        const double raa = fold_raa(g.saa - vaa);                                // :97-98
+        double sr, cr;
+        sincos(raa, &sr, &cr);
+        Primed P;
+        P.vza_p = z[ZR_VZA_P]; P.sza_p = z[ZR_SZA_P];
+        P.t.ts = z[ZR_TS]; P.t.tv = z[ZR_TV]; P.t.secs = z[ZR_SECS]; P.t.secv = z[ZR_SECV];
+        P.t.cs = z[ZR_CS]; P.t.cv = z[ZR_CV]; P.t.ss = z[ZR_SS]; P.t.sv = z[ZR_SV];
+        CrownLite s;
+        s.Mv = z[ZR_MV]; s.theta_Mi = z[ZR_THETA_MI]; s.Gamma_v = z[ZR_GAMMA_V];
+        const double vza = z[ZR_VZA];
+        const bool vgs = fabs(vza) > fabs(g.sza);
+        const Pass pa = kc_pass(c, P, s, vgs, raa, cr, sr);
+        Tail tl;
+        tl.e_v = z[ZR_EV]; tl.e_s = z[ZR_ES]; tl.t0 = z[ZR_T0]; tl.beta = z[ZR_BETA];
+        // pair part of gortt_kuusk, gortt_brdf.c:650-702
+        Hot h;
+        h.pn0_s = z[ZR_PN0S]; h.pe_s = z[ZR_PES];
+        {
+            const double cos_xi = z[ZR_CSZ] * z[ZR_CVZ] + z[ZR_SSZ] * z[ZR_SVZ] * cr;
+            const double lsza = z[ZR_LSZA], lvza = z[ZR_LVZA];
+            const double arg = lsza * lsza + lvza * lvza - 2. * lsza * lvza * cos_xi;
+            double t1, t2;
+            if (arg > 0.0) {
+                double lsv = sqrt(arg);
+                t2 = (1.0 - exp(-lsv / c.r)) / (lsv / c.r);
+            } else {
+                t2 = 1.0;
+            }
+            if ((lsza * lvza) > 0.0) t1 = sqrt(lsza * lvza);
+            else t1 = 0.0;
+            const double H = exp(c.kfavd * t1 * t2);
+            h.kuusk = h.pe_s * z[ZR_PEV] * H;
+        }
+        fd = z[ZR_FD];
+        const GeomRec r = geom_combine(c, P, pa, z[ZR_F0F0], z[ZR_F180F180], tl, h, raa, fd);
+        const double x = z[ZR_X];
+        const double wn = (gl[GORT_NQUAD + GORT_NQUAD / 2 + jj] * fabs(x) * xr) * (gl[GORT_NQUAD + i] * yr);   // :128-129, :132-133
+        double v[5] = {wn * r.cA, wn * r.Kc, wn * r.cG, wn * r.cZ, wn * r.Kt};
+#pragma unroll
+        for (int k = 0; k < 5; k++) {
+#pragma unroll
+            for (int off = 16; off > 0; off >>= 1) v[k] += __shfl_xor_sync(0xffffffffu, v[k], off);
+            if ((tid & 31) == 0) part[k][tid >> 5] = v[k];
+        }
+        if (tid == 0) {
+            sunv[0] = r.fd; sunv[1] = r.mus; sunv[2] = r.t0; sunv[3] = r.tp0; sunv[4] = r.pe_s; sunv[5] = r.pn0_s;
+        }
+    }
+    __syncthreads();
+    if (tid < 5) {
+        double sum = 0.0;
+        for (int w = 0; w < GORT_EN_THREADS / 32; w++) sum += part[tid][w];
+        coef[tid] = sum;
+    }
+    __syncthreads();
+    return fd;
 }
 
 __global__ void __launch_bounds__(GORT_EN_THREADS, 2)
@@ -709,6 +812,325 @@ int launch_energy(gort_ctx *ctx, cudaStream_t s, const gort_shape &sh, const dou
                                                            ctx->d_gauleg, zrec, rleaf, tleaf, rsoil, albedo, favegt, fasoil);
     ctx->launches++;
     return check_cuda(ctx, cudaGetLastError(), "gort_energy launch");
+}
+
+// ------------------------------------------------------------------------------------------------
+// Sensor bands: values averaged over spectral response functions (gort_*_band_batch, include/gort_b200.h).
+//
+// A band value is the weighted mean  sum_{w_i > 0} w_i x_i / sum_{w_i > 0} w_i  of the per-wavelength results x_i.  Both
+// paths are linear in five (sun, lambda) terms -- rsurf = cA A + Kc PDF + cG G + cZ Z + Kt T (gort_rsurf_wide.cuh), the
+// energy balance the same with the quadrature sums and one more term Z/rs (gortt_albedo.c:49) -- so the mean moves onto
+// the terms: the weighted means <A>, <PDF>, <G>, <Z>, <T> (, <Z/rs>) are formed once per (set, sun, band), and a line
+// costs 5 FP64 instructions per band.  Zero-weight columns are skipped, never multiplied: a NaN there cannot leak in.
+// Every sum runs in a fixed order (no atomics): identical calls give identical bits.
+#define BAND_THREADS 128
+#define BAND_LINES 16             // lines per CTA of brdf_band_kernel (C4's 16 geometries per member: one CTA per member)
+#define BAND_TILE 32              // columns per tile of brdf_band_kernel
+#define BAND_NLEAF 11             // the LeafTerms fields
+
+// per band: first and last column of positive weight and 1 / (sum of the positive weights); per column: whether any band
+// needs it.  A defective row (a weight that is NaN, infinite or negative, or no positive weight) gets an empty range and
+// 1/sum = NaN: its band comes out NaN and no other band is affected.
+struct BandSup { double *inv; int *first, *last; unsigned char *need; };
+
+__global__ void __launch_bounds__(BAND_THREADS)
+band_support_kernel(int n_bands, int n_wl, const double* __restrict__ weights, double* __restrict__ inv,
+                    int* __restrict__ first, int* __restrict__ last, unsigned char* __restrict__ need)
+{
+    __shared__ double s_sum[BAND_THREADS / 32];
+    __shared__ int s_lo[BAND_THREADS / 32], s_hi[BAND_THREADS / 32], s_bad[BAND_THREADS / 32];
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    if ((int) blockIdx.x >= n_bands) {
+        const int j = (blockIdx.x - n_bands) * BAND_THREADS + tid;
+        if (j >= n_wl) return;
+        unsigned char n = 0;
+        for (int b = 0; b < n_bands; b++) n |= weights[(size_t) b * n_wl + j] > 0.0;
+        need[j] = n;
+        return;
+    }
+    const int b = blockIdx.x;
+    const double* row = weights + (size_t) b * n_wl;
+    double sum = 0.0;
+    int lo = n_wl, hi = -1, bad = 0;
+    for (int j = tid; j < n_wl; j += BAND_THREADS) {
+        const double v = row[j];
+        if (v > 0.0) { sum += v; lo = min(lo, j); hi = max(hi, j); }
+        if (!(v >= 0.0) || isinf(v)) bad = 1;
+    }
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) {
+        sum += __shfl_xor_sync(0xffffffffu, sum, off);
+        lo = min(lo, __shfl_xor_sync(0xffffffffu, lo, off));
+        hi = max(hi, __shfl_xor_sync(0xffffffffu, hi, off));
+        bad |= __shfl_xor_sync(0xffffffffu, bad, off);
+    }
+    if (lane == 0) { s_sum[warp] = sum; s_lo[warp] = lo; s_hi[warp] = hi; s_bad[warp] = bad; }
+    __syncthreads();
+    if (tid == 0) {
+        double t = 0.0;
+        for (int w = 0; w < BAND_THREADS / 32; w++) {
+            t += s_sum[w]; lo = min(lo, s_lo[w]); hi = max(hi, s_hi[w]); bad |= s_bad[w];
+        }
+        if (bad || hi < 0 || isinf(t)) { first[b] = 1; last[b] = 0; inv[b] = __longlong_as_double(0x7ff8000000000000LL); }
+        else { first[b] = lo; last[b] = hi; inv[b] = 1.0 / t; }
+    }
+}
+
+// brdf_band_kernel: one CTA per (set, BAND_LINES consecutive lines of that set).  Warp 0 cuts the lines into runs that
+// share a sun (record flags) and reads each run's sun values.  The CTA then walks the bands' column range in tiles of
+// BAND_TILE columns, skipping tiles no band needs; per tile
+//   1. the (set, lambda) terms of the needed columns and the tile's weights go to shared memory (once per set and
+//      column, not once per line or run);
+//   2. all threads share the R x BAND_TILE (run, column) sun terms -- the expensive part, balanced over the CTA and
+//      computed once however many bands overlap the column;
+//   3. thread t adds the tile's columns of its pairs (run p / B, band p % B), p = t, t + 128, ..., in column order, to
+//      their five running sums in shared memory (each pair's sums touched by one thread only: fixed order, no atomics).
+// Finally each (line, band) is 5 FP64 instructions on its record's coefficients and the run's means.  A CTA never spans
+// two sets, so with per-member geometry (every line its own run) the set's leaf terms serve all its lines.
+__global__ void __launch_bounds__(BAND_THREADS, 6)
+brdf_band_kernel(int n_sets, int n_geom, int n_wl, int spectra_per_set, int n_bands, int tiles_per_set,
+                 const double* __restrict__ structure, const double* __restrict__ lut, const double* __restrict__ rec,
+                 const double* __restrict__ rleaf, const double* __restrict__ tleaf, const double* __restrict__ rsoil,
+                 const double* __restrict__ weights, const double* __restrict__ inv, const int* __restrict__ first,
+                 const int* __restrict__ last, const unsigned char* __restrict__ need, double* __restrict__ rband)
+{
+    // dynamic: the pairs' running sums / means [BAND_LINES runs][n_bands][5], then the tile's weights [n_bands][BAND_TILE]
+    // (sized by the call's band count: the CTAs per SM depend on it)
+    extern __shared__ double means[];
+    double* wts = means + 5 * BAND_LINES * n_bands;
+    __shared__ double leaf[BAND_NLEAF][BAND_TILE];
+    __shared__ double terms[BAND_LINES][4][BAND_TILE];  // PDF G Z T of (run, column)
+    __shared__ double sun[BAND_LINES][5];               // fd mus t0 tp0 pe_s of each run
+    __shared__ int s_first[GORT_MAX_BANDS], s_last[GORT_MAX_BANDS];
+    __shared__ double s_inv[GORT_MAX_BANDS];
+    __shared__ int run_of[BAND_LINES];
+    __shared__ bool s_need[BAND_TILE];
+    __shared__ int s_runs, s_lo, s_hi;
+
+    const int m = blockIdx.x / tiles_per_set;
+    const int g0 = (blockIdx.x - m * tiles_per_set) * BAND_LINES;
+    const long l0 = (long) m * n_geom + g0;
+    const int nl = min(BAND_LINES, n_geom - g0);
+    const int tid = threadIdx.x;
+    const Canopy c = canopy_load(structure, n_sets, m, lut);
+    for (int b = tid; b < n_bands; b += BAND_THREADS) { s_first[b] = first[b]; s_last[b] = last[b]; s_inv[b] = inv[b]; }
+    if (tid < 32) {
+        // record layout: (cA,Kc) (cG,cZ) (Kt,flags) (q,fd) (mus,t0) (tp0,pe_s) ...; flags bit0 new sun, bit1 new set
+        const double2* rr = reinterpret_cast<const double2*>(rec + (size_t) (l0 + min(tid, nl - 1)) * GORT_REC_STRIDE);
+        const bool start = tid < nl && (tid == 0 || (__double_as_longlong(rr[2].y) & 3) != 0);
+        const unsigned mask = __ballot_sync(0xffffffffu, start);
+        const int r = __popc(mask & (0xffffffffu >> (31 - tid))) - 1;
+        if (tid < nl) run_of[tid] = r;
+        if (start) {
+            const double2 s0 = rr[4], s1 = rr[5];
+            sun[r][0] = rr[3].y; sun[r][1] = s0.x; sun[r][2] = s0.y; sun[r][3] = s1.x; sun[r][4] = s1.y;
+        }
+        if (tid == 0) s_runs = __popc(mask);
+    }
+    __syncthreads();
+    if (tid == 0) {
+        int lo = n_wl, hi = -1;
+        for (int b = 0; b < n_bands; b++) if (s_first[b] <= s_last[b]) { lo = min(lo, s_first[b]); hi = max(hi, s_last[b]); }
+        s_lo = lo; s_hi = hi;
+    }
+    __syncthreads();
+    const int R = s_runs, lo = s_lo, hi = s_hi;
+    const size_t sb = spectra_per_set ? (size_t) m * n_wl : 0;
+    const int P = R * n_bands;
+    for (int i = tid; i < 5 * P; i += BAND_THREADS) means[i] = 0.0;
+    for (int c0 = lo; c0 <= hi; c0 += BAND_TILE) {
+        bool nj = false;
+        if (tid < BAND_TILE) {
+            const int j = c0 + tid;
+            nj = j <= hi && need[j];
+            s_need[tid] = nj;
+            if (nj) {
+                const LeafTerms Lf = leaf_terms(c, rleaf[sb + j], tleaf[sb + j], rsoil[sb + j]);
+                leaf[0][tid] = Lf.omega; leaf[1][tid] = Lf.gam; leaf[2][tid] = Lf.Tff; leaf[3][tid] = Lf.Rff;
+                leaf[4][tid] = Lf.pff; leaf[5][tid] = Lf.tff; leaf[6][tid] = Lf.tpff; leaf[7][tid] = Lf.A;
+                leaf[8][tid] = Lf.rs; leaf[9][tid] = Lf.Xf; leaf[10][tid] = Lf.Zf;
+            }
+        }
+        if (!__syncthreads_or(nj)) continue;
+        for (int i = tid; i < n_bands * BAND_TILE; i += BAND_THREADS) {
+            const int bb = i / BAND_TILE, k = i - bb * BAND_TILE;
+            wts[i] = c0 + k <= hi ? weights[(size_t) bb * n_wl + c0 + k] : 0.0;
+        }
+        for (int i = tid; i < R * BAND_TILE; i += BAND_THREADS) {
+            const int rr = i / BAND_TILE, k = i - rr * BAND_TILE;
+            if (!s_need[k]) continue;
+            LeafTerms Lf;
+            Lf.omega = leaf[0][k]; Lf.gam = leaf[1][k]; Lf.Tff = leaf[2][k]; Lf.Rff = leaf[3][k];
+            Lf.pff = leaf[4][k]; Lf.tff = leaf[5][k]; Lf.tpff = leaf[6][k]; Lf.A = leaf[7][k];
+            Lf.rs = leaf[8][k]; Lf.Xf = leaf[9][k]; Lf.Zf = leaf[10][k];
+            const SunTerms S = sun_terms(c, Lf, sun[rr][0], sun[rr][1], sun[rr][2], sun[rr][3], sun[rr][4]);
+            terms[rr][0][k] = S.PDF; terms[rr][1][k] = S.G; terms[rr][2][k] = S.Z; terms[rr][3][k] = S.T;
+        }
+        __syncthreads();
+        // the running sums of pair p live in means[5p..5p+5) and only thread p % BAND_THREADS touches them: with more
+        // pairs than threads a thread takes several pairs here, and the tile's terms above still serve them all
+        for (int p = tid; p < P; p += BAND_THREADS) {
+            const int r = p / n_bands, b = p - r * n_bands;
+            const int k1 = min(c0 + BAND_TILE - 1, s_last[b]) - c0;
+            int k = max(c0, s_first[b]) - c0;
+            if (k > k1) continue;
+            double* acc = means + 5 * p;
+            double a0 = acc[0], a1 = acc[1], a2 = acc[2], a3 = acc[3], a4 = acc[4];
+            for (; k <= k1; k++) {
+                const double w = wts[b * BAND_TILE + k];
+                if (!(w > 0.0)) continue;
+                a0 = fma(w, leaf[7][k], a0); a1 = fma(w, terms[r][0][k], a1); a2 = fma(w, terms[r][1][k], a2);
+                a3 = fma(w, terms[r][2][k], a3); a4 = fma(w, terms[r][3][k], a4);
+            }
+            acc[0] = a0; acc[1] = a1; acc[2] = a2; acc[3] = a3; acc[4] = a4;
+        }
+        __syncthreads();              // the next tile overwrites the tables
+    }
+    for (int p = tid; p < P; p += BAND_THREADS) {
+        const double iv = s_inv[p % n_bands];
+#pragma unroll
+        for (int k = 0; k < 5; k++) means[5 * p + k] *= iv;
+    }
+    __syncthreads();
+    for (int i = tid; i < nl * n_bands; i += BAND_THREADS) {
+        const int l = i / n_bands, b = i - l * n_bands;
+        const double* mv = means + (run_of[l] * n_bands + b) * 5;
+        const double2* rr = reinterpret_cast<const double2*>(rec + (size_t) (l0 + l) * GORT_REC_STRIDE);
+        const double2 v0 = rr[0], v1 = rr[1];
+        const double Kt = rr[2].x;
+        rband[(size_t) (l0 + l) * n_bands + b] = fma(v0.x, mv[0], fma(v0.y, mv[1], fma(v1.x, mv[2], fma(v1.y, mv[3], Kt * mv[4]))));
+    }
+}
+
+// energy_band_kernel: energy_kernel with a band tail.  After the coefficient sums of the CTA's (set, sun line), warp w
+// owns bands w, w + 16, ...: its lanes stride over the band's columns, each lane sums its columns in order, and a fixed
+// shuffle tree joins the lanes.  The balance of gortt_albedo.c:37-52 is linear in the six means.  The sun values and
+// the coefficient sums are read from shared memory where they are used: that keeps the kernel within the 64 registers
+// of two CTAs per SM without spilling.
+__global__ void __launch_bounds__(GORT_EN_THREADS, 2)
+energy_band_kernel(int n_sets, int n_geom, int n_wl, int geom_per_set, int spectra_per_set, int n_bands,
+                   const double* __restrict__ structure, const double* __restrict__ lut,
+                   const double* __restrict__ angles, const double* __restrict__ gl, const double* __restrict__ zrec,
+                   const double* __restrict__ rleaf, const double* __restrict__ tleaf, const double* __restrict__ rsoil,
+                   const double* __restrict__ weights, const double* __restrict__ inv, const int* __restrict__ first,
+                   const int* __restrict__ last, double* __restrict__ albedo, double* __restrict__ favegt,
+                   double* __restrict__ fasoil)
+{
+    __shared__ double part[5][GORT_EN_THREADS / 32];
+    __shared__ double coef[5];
+    __shared__ double sunv[6];                          // fd mus t0 tp0 pe_s pn0_s
+
+    const long L = (long) n_sets * n_geom;
+    const long line = blockIdx.x;
+    const int m = (int) (line / n_geom);
+    const int tid = threadIdx.x, lane = tid & 31;
+    const Canopy c = canopy_load(structure, n_sets, m, lut);
+    energy_node_sums(n_geom, geom_per_set, L, line, m, c, angles, gl, zrec, part, coef, sunv);
+    const size_t sb = spectra_per_set ? (size_t) m * n_wl : 0;
+    for (int b = tid >> 5; b < n_bands; b += GORT_EN_THREADS / 32) {
+        double acc[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};     // A PDF G Z T Z/rs
+        const int bl = last[b];
+        for (int j = first[b] + lane; j <= bl; j += 32) {
+            const double w = weights[(size_t) b * n_wl + j];
+            if (!(w > 0.0)) continue;
+            const double rs = rsoil[sb + j];
+            const LeafTerms Lf = leaf_terms(c, rleaf[sb + j], tleaf[sb + j], rs);
+            const SunTerms S = sun_terms(c, Lf, sunv[0], sunv[1], sunv[2], sunv[3], sunv[4]);
+            acc[0] = fma(w, Lf.A, acc[0]); acc[1] = fma(w, S.PDF, acc[1]); acc[2] = fma(w, S.G, acc[2]);
+            acc[3] = fma(w, S.Z, acc[3]); acc[4] = fma(w, S.T, acc[4]); acc[5] = fma(w, S.Z / rs, acc[5]);
+        }
+#pragma unroll
+        for (int k = 0; k < 6; k++)
+#pragma unroll
+            for (int off = 16; off > 0; off >>= 1) acc[k] += __shfl_xor_sync(0xffffffffu, acc[k], off);
+        if (lane == 0) {
+            const double iv = inv[b];
+            const double mA = acc[0] * iv, mP = acc[1] * iv, mG = acc[2] * iv, mZ = acc[3] * iv, mT = acc[4] * iv, mZr = acc[5] * iv;
+            const double Pn0 = sunv[5];
+            const double alb = fma(coef[0], mA, fma(coef[1], mP, fma(coef[2], mG, fma(coef[3], mZ, coef[4] * mT)))) / GORT_PI;
+            const double Fu2 = mG * Pn0 + mZ * (1. - Pn0);
+            const double Fd2 = Pn0 + mZr * (1. - Pn0);
+            const size_t o = (size_t) line * n_bands + b;
+            albedo[o] = alb;
+            favegt[o] = 1. - alb - Fd2 + Fu2;
+            fasoil[o] = Fd2 - Fu2;
+        }
+    }
+}
+
+static int band_support(gort_ctx *ctx, cudaStream_t s, int n_bands, int n_wl, const double *weights, BandSup *sp)
+{
+    const size_t B = (size_t) n_bands;
+    char *p = (char *) scratch(ctx, GORT_BAND_SLOT, (sizeof(double) + 2 * sizeof(int)) * B + (size_t) n_wl);
+    if (!p) return GORT_ERR_NOMEM;
+    sp->inv = (double *) p;
+    sp->first = (int *) (p + sizeof(double) * B);
+    sp->last = sp->first + B;
+    sp->need = (unsigned char *) (sp->last + B);
+    band_support_kernel<<<(unsigned) (n_bands + (n_wl + BAND_THREADS - 1) / BAND_THREADS), BAND_THREADS, 0, s>>>(
+        n_bands, n_wl, weights, sp->inv, sp->first, sp->last, sp->need);
+    ctx->launches++;
+    return check_cuda(ctx, cudaGetLastError(), "band_support_kernel launch");
+}
+
+int launch_brdf_band(gort_ctx *ctx, cudaStream_t s, const gort_shape &sh, int n_bands, const double *weights,
+                     const double *structure, const double *lut, const double *angles, const double *rleaf,
+                     const double *tleaf, const double *rsoil, double *rband)
+{
+    if (sh.n_sets <= 0 || sh.n_geom <= 0 || sh.n_wl <= 0 || n_bands < 1 || n_bands > GORT_MAX_BANDS)
+        return set_error(ctx, GORT_ERR_INVALID, "gort_brdf_band: n_sets, n_geom, n_wl and n_bands out of range");
+    const long L = (long) sh.n_sets * sh.n_geom;
+    // plain stream order throughout: a band call ends any overlap window of the BRDF path
+    note_other_work(ctx);
+    BandSup sp;
+    int rc = band_support(ctx, s, n_bands, sh.n_wl, weights, &sp);
+    if (rc != GORT_OK) return rc;
+    double *rec;
+    unsigned long long *flags;
+    rc = next_records(ctx, s, L, &rec, &flags);
+    if (rc != GORT_OK) return rc;
+    rc = launch_geom(ctx, s, sh, structure, lut, angles, rec, NULL, flags, false);
+    if (rc != GORT_OK) return rc;
+    if (!ctx->band_attr_set) {
+        cudaError_t e = cudaFuncSetAttribute(brdf_band_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                             (int) (sizeof(double) * (5 * BAND_LINES + BAND_TILE) * GORT_MAX_BANDS));
+        if (e != cudaSuccess) return check_cuda(ctx, e, "brdf_band_kernel shared memory");
+        ctx->band_attr_set = 1;
+    }
+    const int tiles = (sh.n_geom + BAND_LINES - 1) / BAND_LINES;
+    const size_t smem = sizeof(double) * (5 * BAND_LINES + BAND_TILE) * (size_t) n_bands;
+    brdf_band_kernel<<<(unsigned) ((long) tiles * sh.n_sets), BAND_THREADS, smem, s>>>(
+        sh.n_sets, sh.n_geom, sh.n_wl, sh.spectra_per_set, n_bands, tiles, structure, lut, rec, rleaf, tleaf, rsoil,
+        weights, sp.inv, sp.first, sp.last, sp.need, rband);
+    ctx->launches++;
+    return check_cuda(ctx, cudaGetLastError(), "brdf_band_kernel launch");
+}
+
+int launch_energy_band(gort_ctx *ctx, cudaStream_t s, const gort_shape &sh, int n_bands, const double *weights,
+                       const double *structure, const double *lut, const double *angles, const double *rleaf,
+                       const double *tleaf, const double *rsoil, double *albedo, double *favegt, double *fasoil)
+{
+    if (sh.n_sets <= 0 || sh.n_geom <= 0 || sh.n_wl <= 0 || n_bands < 1 || n_bands > GORT_MAX_BANDS)
+        return set_error(ctx, GORT_ERR_INVALID, "gort_energy_band: n_sets, n_geom, n_wl and n_bands out of range");
+    const long L = (long) sh.n_sets * sh.n_geom;
+    note_other_work(ctx);
+    BandSup sp;
+    int rc = band_support(ctx, s, n_bands, sh.n_wl, weights, &sp);
+    if (rc != GORT_OK) return rc;
+    double *zrec = (double *) workspace(ctx, sizeof(double) * GORT_EN_ZREC * GORT_EN_NZ * (size_t) L);
+    if (!zrec) return GORT_ERR_NOMEM;
+    {
+        const long items = L * GORT_EN_NZ;
+        energy_zenith_kernel<<<(unsigned) ((items + 127) / 128), 128, 0, s>>>(sh.n_sets, sh.n_geom, sh.geom_per_set, sh.opt, structure,
+                                                                             lut, angles, ctx->d_gauleg, zrec);
+        ctx->launches++;
+    }
+    energy_band_kernel<<<(unsigned) L, GORT_EN_THREADS, 0, s>>>(sh.n_sets, sh.n_geom, sh.n_wl, sh.geom_per_set,
+                                                                sh.spectra_per_set, n_bands, structure, lut, angles,
+                                                                ctx->d_gauleg, zrec, rleaf, tleaf, rsoil, weights,
+                                                                sp.inv, sp.first, sp.last, albedo, favegt, fasoil);
+    ctx->launches++;
+    return check_cuda(ctx, cudaGetLastError(), "gort_energy_band launch");
 }
 
 // ------------------------------------------------------------------------------------------------

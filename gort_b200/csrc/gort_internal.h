@@ -7,6 +7,7 @@
 
 #define GORT_NSCRATCH 32
 #define GORT_MAX_WIDE_CTAS 8192
+#define GORT_BAND_SLOT (GORT_NSCRATCH - 1)   // scratch slot of the band supports (gort_*_band_batch[_dev])
 
 struct gort_ctx {
     int device;
@@ -45,7 +46,7 @@ struct gort_ctx {
     cudaEvent_t xstream_ev;            // orders calls issued on different streams (order_after_previous)
     struct { int key_lpt, key_scomp, key_tmab, key_threads; int occ; } wide_plan[8];
     int n_wide_plan;
-    int geom_carveout_set, lut_attr_set;
+    int geom_carveout_set, lut_attr_set, band_attr_set;
     // development switch, read once from the environment by gort_create: GORT_TIMELINE=<call number>
     int dbg_timeline;
     unsigned long long *d_timeline;
@@ -82,6 +83,13 @@ int launch_brdf(gort_ctx *ctx, cudaStream_t s, const gort_shape &sh, const doubl
 int launch_energy(gort_ctx *ctx, cudaStream_t s, const gort_shape &sh, const double *structure,
                   const double *lut, const double *angles, const double *rleaf, const double *tleaf,
                   const double *rsoil, double *albedo, double *favegt, double *fasoil);
+// sensor bands: weights [n_bands][sh.n_wl] (device), outputs [M][G][n_bands]
+int launch_brdf_band(gort_ctx *ctx, cudaStream_t s, const gort_shape &sh, int n_bands, const double *weights,
+                     const double *structure, const double *lut, const double *angles, const double *rleaf,
+                     const double *tleaf, const double *rsoil, double *rband);
+int launch_energy_band(gort_ctx *ctx, cudaStream_t s, const gort_shape &sh, int n_bands, const double *weights,
+                       const double *structure, const double *lut, const double *angles, const double *rleaf,
+                       const double *tleaf, const double *rsoil, double *albedo, double *favegt, double *fasoil);
 int launch_lut(gort_ctx *ctx, cudaStream_t s, int n_sets, const double *structure, int method, double *lut);
 int launch_lut_out(gort_ctx *ctx, cudaStream_t s, int n_sets, const double *structure, int method, double *lut,
                    int n_dst, double *const *dst, int multicast);

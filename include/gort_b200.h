@@ -249,6 +249,46 @@ int gort_energy_batch_dev(gort_ctx *ctx, void *stream, const gort_shape *shape,
 /* the 32-point Gauss-Legendre rule the energy path uses (gauleg, gortt_albedo.c:142-198) */
 int gort_gauleg(gort_ctx *ctx, double *abscissa, double *weights);
 
+/* ---- sensor bands: BRDF, albedo and fAPAR averaged over spectral response functions (SRFs).  No reference
+ *      counterpart (the reference evaluates single wavelengths); a satellite measures bands.
+ *      A call has a grid of W = shape->n_wl wavelength columns: the columns of rleaf/tleaf/rsoil, or wavelength[W] for
+ *      gort_forward_band_batch.  weights [B][W] holds one row per band, raw SRF values (the library normalises).  For
+ *      band b with S_b = { i : weights[b][i] > 0 }
+ *          value[b] = sum_{i in S_b} weights[b][i] * x_i / sum_{i in S_b} weights[b][i]
+ *      where x_i is exactly what the per-wavelength entry point returns for column i with the same inputs: rsurf for
+ *      the BRDF (gort_brdf_batch), albedo / favegt / fasoil for the energy balance (gort_energy_batch).  Columns outside
+ *      S_b are never read for band b (a NaN there does not propagate); a NaN inside S_b makes the band NaN (grazing
+ *      angles give NaN bands, as they give NaN wavelengths).  Outputs are [M][G][B], dense.
+ *      The host-pointer entry points return GORT_ERR_INVALID and enqueue nothing unless 1 <= n_bands <= GORT_MAX_BANDS,
+ *      every weight is finite and >= 0, every row has a positive weight and shape->out_pitch == 0.  The _dev entry
+ *      points check n_bands, the shape and the pointers only: they cannot inspect device weights without synchronising,
+ *      so a defective row (a NaN, infinite or negative weight, or no positive weight) gives NaN in its own band and
+ *      every other band stays correct.  Band calls run in plain stream order and end any overlap window
+ *      (gort_set_overlap).  Identical calls give identical bits (every sum runs in a fixed order). */
+#define GORT_MAX_BANDS 64
+int gort_brdf_band_batch(gort_ctx *ctx, const gort_shape *shape, int n_bands, const double *weights,
+                         const double *structure, const double *lut, const double *angles,
+                         const double *rleaf, const double *tleaf, const double *rsoil, double *rband);
+int gort_brdf_band_batch_dev(gort_ctx *ctx, void *stream, const gort_shape *shape, int n_bands, const double *weights,
+                             const double *structure, const double *lut, const double *angles,
+                             const double *rleaf, const double *tleaf, const double *rsoil, double *rband);
+int gort_energy_band_batch(gort_ctx *ctx, const gort_shape *shape, int n_bands, const double *weights,
+                           const double *structure, const double *lut, const double *angles,
+                           const double *rleaf, const double *tleaf, const double *rsoil,
+                           double *albedo, double *favegt, double *fasoil);
+int gort_energy_band_batch_dev(gort_ctx *ctx, void *stream, const gort_shape *shape, int n_bands, const double *weights,
+                               const double *structure, const double *lut, const double *angles,
+                               const double *rleaf, const double *tleaf, const double *rsoil,
+                               double *albedo, double *favegt, double *fasoil);
+/* The ensemble forward operator of gort_forward_batch with band outputs: rband [M][G][B] = the definition above applied to
+ * the rsurf gort_forward_batch returns for the same arguments.  The spectra are computed only on the union of the bands'
+ * supports (a full 2101-column grid with a few narrow bands costs the bands' columns), yet every wavelength[] is
+ * range-checked (GORT_ERR_RANGE) as in gort_forward_batch.  lut_out as there. */
+int gort_forward_band_batch(gort_ctx *ctx, const gort_shape *shape, int lut_method, const double *structure,
+                            const double *leaf, const double *soil, double user_leaf, double user_soil,
+                            const double *wavelength, int n_bands, const double *weights,
+                            const double *angles, double *rband, double *lut_out);
+
 /* ---- LUT text layout ("-W" / "-P", gortt.c:123-146) -- host-side formatting only --------- */
 /* writes 90 rows "%d %0.40f %0.40f\n" and the "-1" row for one LUT record; returns bytes
  * written or a negative GORT_ERR_*.  fp is a FILE*. */

@@ -64,6 +64,7 @@ ABI_SYMBOLS = [
     "gort_forward_batch", "gort_jacobian_batch", "gort_lut_intermediates_batch", "gort_lut_intermediates_batch_dev", "gort_host_alloc_near", "gort_host_alloc_on_cpus", "gort_host_placement", "gort_soil_table_read", "gort_soil_from_table", "gort_soil_from_table_dev",
     "gort_brdf_band_batch", "gort_brdf_band_batch_dev", "gort_energy_band_batch", "gort_energy_band_batch_dev",
     "gort_forward_band_batch",
+    "gort_lut_tangent_batch_dev", "gort_brdf_tangent_batch_dev", "gort_lai_tangent_batch",
 ]
 
 
@@ -123,6 +124,9 @@ def load_library():
     lib.gort_energy_band_batch_dev.argtypes = [vp, vp, sp, C.c_int] + [vp] * 10
     lib.gort_forward_band_batch.argtypes = [vp, sp, C.c_int, vp, vp, vp, C.c_double, C.c_double, vp, C.c_int, vp, vp, vp, vp]
     lib.gort_jacobian_batch.argtypes = [vp, sp, C.c_int, C.c_int, C.c_double, vp, vp, vp, C.c_double, C.c_double, vp, vp, vp, vp]
+    lib.gort_lut_tangent_batch_dev.argtypes = [vp, vp, C.c_int, vp, C.c_int, vp, vp]
+    lib.gort_brdf_tangent_batch_dev.argtypes = [vp, vp, sp] + [vp] * 8
+    lib.gort_lai_tangent_batch.argtypes = [vp, sp, C.c_int, C.c_int, vp, vp, vp, C.c_double, C.c_double, vp, vp, vp, vp]
     lib.gort_gauleg.argtypes = [vp, vp, vp]
     lib.gort_lut_write_text.argtypes = [vp, vp]
     lib.gort_lut_write_text.restype = C.c_long
@@ -402,6 +406,25 @@ class Gort:
                                                   _ptr(jac), _ptr(rsurf)))
         return (jac, rsurf) if want_rsurf else jac
 
+    def lai_tangent(self, structure, leaf, soil, wavelength, angles, param=JAC_LAI, method=LUT_FULL,
+                    user_leaf=-1.0, user_soil=-1.0, beta=None, fd=None, want_rsurf=False):
+        """d rsurf / d LAI (JAC_LAI, default) or d / d favd (JAC_FAVD) [M][G][W], exact, by forward-mode tangents
+        through the whole chain on the GPU (gort_lai_tangent_batch); optionally rsurf as well (the bits of forward())."""
+        st = _np(structure)
+        M = st.shape[1]
+        leaf = None if leaf is None else _np(leaf)
+        soil = None if soil is None else _np(soil)
+        wl = _np(wavelength).ravel()
+        ang = _np(angles)
+        G, W = ang.shape[-1], wl.shape[0]
+        sh = self._shape(M, G, W, ang.ndim == 3, 1, beta, fd)
+        jac = np.empty((M, G, W))
+        rsurf = np.empty((M, G, W)) if want_rsurf else None
+        self._check(self._lib.gort_lai_tangent_batch(self._h, C.byref(sh), method, int(param), _ptr(st), _ptr(leaf),
+                                                     _ptr(soil), float(user_leaf), float(user_soil), _ptr(wl), _ptr(ang),
+                                                     _ptr(jac), _ptr(rsurf)))
+        return (jac, rsurf) if want_rsurf else jac
+
     def energy(self, structure, lut, angles, rleaf, tleaf, rsoil, beta=None, fd=None):
         st, lut, ang, rl, tl, rs, M, G, W, gps, sps = self._prep(structure, lut, angles, rleaf, tleaf, rsoil)
         sh = self._shape(M, G, W, gps, sps, beta, fd)
@@ -464,6 +487,21 @@ class Gort:
         arr = (C.c_void_p * max(1, len(dst_ptrs)))(*[int(a) for a in dst_ptrs])
         self._check(self._lib.gort_lut_batch_scatter_dev(self._h, stream, M, _ptr(structure), method, _ptr(out),
                                                          len(dst_ptrs), arr, 1 if multicast else 0))
+
+    def lut_tangent_dev(self, structure, lut, dlut, method=LUT_FULL, stream=None):
+        """LUT records into lut (the bits of lut_dev) and their favd tangent into dlut, both [M][184]."""
+        M = structure.shape[1]
+        self._check(self._lib.gort_lut_tangent_batch_dev(self._h, stream, M, _ptr(structure), method, _ptr(lut), _ptr(dlut)))
+
+    def brdf_tangent_dev(self, structure, lut, dlut, angles, rleaf, tleaf, rsoil, drsurf, beta=None, fd=None, stream=None):
+        """d rsurf / d favd [M][G][W] (dense) of brdf_dev's rsurf, from lut and its tangent dlut (lut_tangent_dev)."""
+        M = structure.shape[1]
+        G, W = angles.shape[-1], rleaf.shape[-1]
+        assert tuple(drsurf.shape) == (M, G, W), "drsurf must be [M][G][W]"
+        sh = self._shape(M, G, W, angles.dim() == 3, rleaf.dim() == 2, beta, fd)
+        self._check(self._lib.gort_brdf_tangent_batch_dev(self._h, stream, C.byref(sh), _ptr(structure), _ptr(lut),
+                                                          _ptr(dlut), _ptr(angles), _ptr(rleaf), _ptr(tleaf),
+                                                          _ptr(rsoil), _ptr(drsurf)))
 
     def spectra_dev(self, leaf, soil, wavelength, rleaf, tleaf, rsoil, user_leaf=-1.0, user_soil=-1.0,
                     stream=None):

@@ -602,6 +602,90 @@ static int copy_rows(gort_ctx *ctx, cudaStream_t s, double *dst, size_t dst_pitc
                                              width * sizeof(double), (size_t) rows, kind, s), what);
 }
 
+}  // extern "C"
+
+// The chunked ensemble pipeline of gort_forward_batch, gort_forward_band_batch and gort_lai_tangent_batch: members in
+// chunks on three streams -- the inputs of chunk i+1 go up (stream B) and the results of chunk i-1 come down (stream D)
+// while chunk i's kernels run (stream A); two chunk buffers alternate.  kernels(A, c, bufs) enqueues one chunk's kernels
+// on A.  out_pm[k] sizes the chunk buffer out[k] (doubles per member; 0: none).  After the kernels every copy with a
+// host pointer takes its per_member doubles per member from out[src] (src < 0: the LUT records) to the host.  The caller
+// has uploaded the grid's wavelengths and shared angles (slots 22 and up); the chunk buffers use scratch slots 0-21.
+struct EnsBufs { double *st, *leaf, *soil, *ang, *lut, *rl, *tl, *rs, *out[3]; };
+struct EnsCopy { double *host; int src; size_t per_member; };
+
+template <class Kernels>
+static int ensemble_chunks(gort_ctx *ctx, const gort_shape *shape, const double *structure, const double *leaf,
+                           const double *soil, double user_leaf, double user_soil, const double *angles, size_t n_col,
+                           const size_t out_pm[3], int n_copies, const EnsCopy *copies, const char *who, Kernels kernels)
+{
+    if (!ctx->copy_stream) {
+        TRYCUDA(ctx, cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking), "cudaStreamCreate");
+        TRYCUDA(ctx, cudaStreamCreateWithFlags(&ctx->copy_stream_out, cudaStreamNonBlocking), "cudaStreamCreate");
+        for (int i = 0; i < 6; i++) TRYCUDA(ctx, cudaEventCreateWithFlags(&ctx->fwd_ev[i], cudaEventDisableTiming), "cudaEventCreate");
+    }
+    // three streams: the two copy directions have their own engines, and on ONE copy stream the inputs of chunk i+1 would
+    // queue behind the results of chunk i, which wait for chunk i's kernels -- no copy would run under a kernel
+    cudaStream_t A = ctx->stream, B = ctx->copy_stream, D = ctx->copy_stream_out;
+    const size_t M = shape->n_sets, G = shape->n_geom;
+    // chunk: at least 8 per batch when the batch is large, never above 16384 members, at least 1024
+    size_t C = (M + 7) / 8;
+    if (C > 16384) C = 16384;
+    if (C < 1024) C = 1024;
+    if (C > M) C = M;
+    const bool per_set_geom = shape->geom_per_set != 0;
+    EnsBufs buf[2];
+    const size_t sz[11] = {6 * C, 7 * C, 4 * C, per_set_geom ? 4 * C * G : 8, C * GORT_LUT_STRIDE, C * n_col, C * n_col,
+                           C * n_col, C * out_pm[0], C * out_pm[1], C * out_pm[2]};
+    for (int b = 0; b < 2; b++) {
+        double **p[11] = {&buf[b].st, &buf[b].leaf, &buf[b].soil, &buf[b].ang, &buf[b].lut, &buf[b].rl, &buf[b].tl,
+                          &buf[b].rs, &buf[b].out[0], &buf[b].out[1], &buf[b].out[2]};
+        for (int k = 0; k < 11; k++) {
+            *p[k] = NULL;
+            if (sz[k] == 0) continue;
+            *p[k] = (double *) scratch(ctx, 11 * b + k, sz[k] * sizeof(double));
+            if (!*p[k]) return GORT_ERR_NOMEM;
+        }
+    }
+    // the kernels wait for the previous call; the input copies on B need not: they only fill this call's scratch slots,
+    // which no other call reads while this one runs (every host-pointer call returns synchronised)
+    TRY(order_after_previous(ctx, A));
+    // events per buffer: [b] inputs ready (B), [2+b] kernels done (A), [4+b] outputs copied (D)
+    int chunk_no = 0;
+    for (size_t m0 = 0; m0 < M; m0 += C, chunk_no++) {
+        const size_t c = M - m0 < C ? M - m0 : C;
+        const int b = chunk_no & 1;
+        const EnsBufs &d = buf[b];
+        // -- stream B: inputs of this chunk (after the kernels that last read this buffer's inputs) --
+        if (chunk_no >= 2) TRYCUDA(ctx, cudaStreamWaitEvent(B, ctx->fwd_ev[2 + b], 0), "cudaStreamWaitEvent");
+        TRY(copy_rows(ctx, B, d.st, c, structure + m0, M, c, 6, cudaMemcpyHostToDevice, "forward: structure"));
+        if (user_leaf < 0.0) TRY(copy_rows(ctx, B, d.leaf, c, leaf + m0, M, c, 7, cudaMemcpyHostToDevice, "forward: leaf"));
+        if (user_soil < 0.0) TRY(copy_rows(ctx, B, d.soil, c, soil + m0, M, c, 4, cudaMemcpyHostToDevice, "forward: soil"));
+        if (per_set_geom) TRY(copy_rows(ctx, B, d.ang, c * G, angles + m0 * G, M * G, c * G, 4, cudaMemcpyHostToDevice, "forward: angles"));
+        TRYCUDA(ctx, cudaEventRecord(ctx->fwd_ev[b], B), "cudaEventRecord");
+        // -- stream A: kernels (after the inputs are in, and after the previous outputs of this buffer have left) --
+        TRYCUDA(ctx, cudaStreamWaitEvent(A, ctx->fwd_ev[b], 0), "cudaStreamWaitEvent");
+        if (chunk_no >= 2) TRYCUDA(ctx, cudaStreamWaitEvent(A, ctx->fwd_ev[4 + b], 0), "cudaStreamWaitEvent");
+        TRY(kernels(A, c, d));
+        TRYCUDA(ctx, cudaEventRecord(ctx->fwd_ev[2 + b], A), "cudaEventRecord");
+        // -- stream D: results of this chunk --
+        TRYCUDA(ctx, cudaStreamWaitEvent(D, ctx->fwd_ev[2 + b], 0), "cudaStreamWaitEvent");
+        for (int k = 0; k < n_copies; k++) {
+            const EnsCopy &q = copies[k];
+            if (!q.host) continue;
+            TRYCUDA(ctx, cudaMemcpyAsync(q.host + m0 * q.per_member, q.src < 0 ? d.lut : d.out[q.src],
+                                         c * q.per_member * sizeof(double), cudaMemcpyDeviceToHost, D), "forward: results");
+        }
+        TRYCUDA(ctx, cudaEventRecord(ctx->fwd_ev[4 + b], D), "cudaEventRecord");
+    }
+    TRYCUDA(ctx, cudaStreamSynchronize(D), who);
+    TRYCUDA(ctx, cudaStreamSynchronize(B), who);
+    TRYCUDA(ctx, cudaStreamSynchronize(A), who);
+    note_other_work(ctx);
+    return check_pipeline_fault(ctx);
+}
+
+extern "C" {
+
 int gort_forward_batch(gort_ctx *ctx, const gort_shape *shape, int lut_method, const double *structure,
                        const double *leaf, const double *soil, double user_leaf, double user_soil,
                        const double *wavelength, const double *angles, double *rsurf, double *lut_out)
@@ -612,75 +696,28 @@ int gort_forward_batch(gort_ctx *ctx, const gort_shape *shape, int lut_method, c
         return set_error(ctx, GORT_ERR_INVALID, "gort_forward_batch: NULL argument");
     if (lut_method != GORT_LUT_FULL && lut_method != GORT_LUT_Q08)
         return set_error(ctx, GORT_ERR_INVALID, "gort_forward_batch: unknown LUT method %d", lut_method);
-    const size_t M = shape->n_sets, G = shape->n_geom, W = shape->n_wl;
+    const size_t G = shape->n_geom, W = shape->n_wl;
     for (size_t i = 0; i < W; i++)
         if (wavelength[i] < GORT_WL_MIN || wavelength[i] > GORT_WL_MAX)
             return set_error(ctx, GORT_ERR_RANGE, "wavlength out of range (400-2500)");
     TRYCUDA(ctx, cudaSetDevice(ctx->device), "cudaSetDevice");
-    if (!ctx->copy_stream) {
-        TRYCUDA(ctx, cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking), "cudaStreamCreate");
-        TRYCUDA(ctx, cudaStreamCreateWithFlags(&ctx->copy_stream_out, cudaStreamNonBlocking), "cudaStreamCreate");
-        for (int i = 0; i < 6; i++) TRYCUDA(ctx, cudaEventCreateWithFlags(&ctx->fwd_ev[i], cudaEventDisableTiming), "cudaEventCreate");
-    }
-    // three streams: the two copy directions have their own engines, and on ONE copy stream the inputs of chunk i+1 would
-    // queue behind the results of chunk i, which wait for chunk i's kernels -- no copy would run under a kernel
-    cudaStream_t A = ctx->stream, B = ctx->copy_stream, D = ctx->copy_stream_out;
-    // chunk: at least 8 per batch when the batch is large, never above 16384 members, at least 1024
-    size_t C = (M + 7) / 8;
-    if (C > 16384) C = 16384;
-    if (C < 1024) C = 1024;
-    if (C > M) C = M;
-    const bool per_set_geom = shape->geom_per_set != 0;
-    // device buffers: slots 0-8 and 9-17 are the two chunk buffers, 18 the wavelengths, 19 shared angles
+    // slot 22 the wavelengths, 23 shared angles
     double *d_wl, *d_ang_shared = NULL;
-    TRY(h2d(ctx, 18, wavelength, W, &d_wl));
-    if (!per_set_geom) TRY(h2d(ctx, 19, angles, 4 * G, &d_ang_shared));
-    double *buf[2][9];
-    const size_t sz[9] = {6 * C, 7 * C, 4 * C, per_set_geom ? 4 * C * G : 8, C * GORT_LUT_STRIDE, C * W, C * W, C * W, C * G * W};
-    for (int b = 0; b < 2; b++)
-        for (int k = 0; k < 9; k++) {
-            buf[b][k] = (double *) scratch(ctx, 9 * b + k, sz[k] * sizeof(double));
-            if (!buf[b][k]) return GORT_ERR_NOMEM;
-        }
-    // events per buffer: [b] inputs ready (B), [2+b] kernels done (A), [4+b] outputs copied (D)
+    TRY(h2d(ctx, 22, wavelength, W, &d_wl));
+    if (!shape->geom_per_set) TRY(h2d(ctx, 23, angles, 4 * G, &d_ang_shared));
     gort_shape sh = *shape;
     sh.spectra_per_set = 1;
     sh.out_pitch = 0;
-    // the kernels wait for the previous call; the input copies on B need not: they only fill this call's scratch slots,
-    // which no other call reads while this one runs (every host-pointer call returns synchronised)
-    TRY(order_after_previous(ctx, A));
-    int chunk_no = 0;
-    for (size_t m0 = 0; m0 < M; m0 += C, chunk_no++) {
-        const size_t c = M - m0 < C ? M - m0 : C;
-        const int b = chunk_no & 1;
-        // -- stream B: inputs of this chunk (after the kernels that last read this buffer's inputs) --
-        if (chunk_no >= 2) TRYCUDA(ctx, cudaStreamWaitEvent(B, ctx->fwd_ev[2 + b], 0), "cudaStreamWaitEvent");
-        TRY(copy_rows(ctx, B, buf[b][0], c, structure + m0, M, c, 6, cudaMemcpyHostToDevice, "forward: structure"));
-        if (user_leaf < 0.0) TRY(copy_rows(ctx, B, buf[b][1], c, leaf + m0, M, c, 7, cudaMemcpyHostToDevice, "forward: leaf"));
-        if (user_soil < 0.0) TRY(copy_rows(ctx, B, buf[b][2], c, soil + m0, M, c, 4, cudaMemcpyHostToDevice, "forward: soil"));
-        if (per_set_geom) TRY(copy_rows(ctx, B, buf[b][3], c * G, angles + m0 * G, M * G, c * G, 4, cudaMemcpyHostToDevice, "forward: angles"));
-        TRYCUDA(ctx, cudaEventRecord(ctx->fwd_ev[b], B), "cudaEventRecord");
-        // -- stream A: kernels (after the inputs are in, and after the previous outputs of this buffer have left) --
-        TRYCUDA(ctx, cudaStreamWaitEvent(A, ctx->fwd_ev[b], 0), "cudaStreamWaitEvent");
-        if (chunk_no >= 2) TRYCUDA(ctx, cudaStreamWaitEvent(A, ctx->fwd_ev[4 + b], 0), "cudaStreamWaitEvent");
+    const size_t out_pm[3] = {G * W, 0, 0};
+    const EnsCopy copies[2] = {{rsurf, 0, G * W}, {lut_out, -1, GORT_LUT_STRIDE}};
+    return ensemble_chunks(ctx, shape, structure, leaf, soil, user_leaf, user_soil, angles, W, out_pm, 2, copies, "gort_forward_batch",
+                           [&](cudaStream_t A, size_t c, const EnsBufs &d) {
         sh.n_sets = (int) c;
-        TRY(launch_lut(ctx, A, (int) c, buf[b][0], lut_method, buf[b][4]));
-        TRY(launch_spectra(ctx, A, (int) c, user_leaf < 0.0 ? buf[b][1] : NULL, user_soil < 0.0 ? buf[b][2] : NULL, user_leaf, user_soil,
-                           (int) W, d_wl, buf[b][5], buf[b][6], buf[b][7]));
-        TRY(launch_brdf(ctx, A, sh, buf[b][0], buf[b][4], per_set_geom ? buf[b][3] : d_ang_shared, buf[b][5], buf[b][6], buf[b][7],
-                        buf[b][8], NULL, NULL));
-        TRYCUDA(ctx, cudaEventRecord(ctx->fwd_ev[2 + b], A), "cudaEventRecord");
-        // -- stream D: results of this chunk --
-        TRYCUDA(ctx, cudaStreamWaitEvent(D, ctx->fwd_ev[2 + b], 0), "cudaStreamWaitEvent");
-        TRYCUDA(ctx, cudaMemcpyAsync(rsurf + m0 * G * W, buf[b][8], c * G * W * sizeof(double), cudaMemcpyDeviceToHost, D), "forward: rsurf");
-        if (lut_out) TRYCUDA(ctx, cudaMemcpyAsync(lut_out + m0 * GORT_LUT_STRIDE, buf[b][4], c * GORT_LUT_STRIDE * sizeof(double), cudaMemcpyDeviceToHost, D), "forward: lut");
-        TRYCUDA(ctx, cudaEventRecord(ctx->fwd_ev[4 + b], D), "cudaEventRecord");
-    }
-    TRYCUDA(ctx, cudaStreamSynchronize(D), "gort_forward_batch");
-    TRYCUDA(ctx, cudaStreamSynchronize(B), "gort_forward_batch");
-    TRYCUDA(ctx, cudaStreamSynchronize(A), "gort_forward_batch");
-    note_other_work(ctx);
-    return check_pipeline_fault(ctx);
+        TRY(launch_lut(ctx, A, (int) c, d.st, lut_method, d.lut));
+        TRY(launch_spectra(ctx, A, (int) c, user_leaf < 0.0 ? d.leaf : NULL, user_soil < 0.0 ? d.soil : NULL, user_leaf, user_soil,
+                           (int) W, d_wl, d.rl, d.tl, d.rs));
+        return launch_brdf(ctx, A, sh, d.st, d.lut, sh.geom_per_set ? d.ang : d_ang_shared, d.rl, d.tl, d.rs, d.out[0], NULL, NULL);
+    });
 }
 
 // ---- finite-difference Jacobian through the whole chain (SURVEY.md 8f row 4) -----------------------------
@@ -748,6 +785,73 @@ int gort_jacobian_batch(gort_ctx *ctx, const gort_shape *shape, int lut_method, 
     }
     TRYCUDA(ctx, cudaStreamSynchronize(A), "gort_jacobian_batch");
     return check_pipeline_fault(ctx);
+}
+
+// ---- exact favd / LAI tangent (forward mode) -----------------------------------------------------------------------
+int gort_lut_tangent_batch_dev(gort_ctx *ctx, void *stream, int n_sets, const double *structure, int method, double *lut,
+                               double *dlut)
+{
+    if (!ctx) return GORT_ERR_INVALID;
+    if (!structure || !lut || !dlut || n_sets <= 0) return set_error(ctx, GORT_ERR_INVALID, "gort_lut_tangent_batch: bad arguments");
+    if (method != GORT_LUT_FULL && method != GORT_LUT_Q08) return set_error(ctx, GORT_ERR_INVALID, "gort_lut_tangent_batch: unknown method %d", method);
+    TRYCUDA(ctx, cudaSetDevice(ctx->device), "cudaSetDevice");
+    const cudaStream_t s = pick(ctx, stream);
+    TRY(order_after_previous(ctx, s));
+    return launch_lut_tangent(ctx, s, n_sets, structure, method, lut, dlut);
+}
+
+int gort_brdf_tangent_batch_dev(gort_ctx *ctx, void *stream, const gort_shape *shape, const double *structure,
+                                const double *lut, const double *dlut, const double *angles, const double *rleaf,
+                                const double *tleaf, const double *rsoil, double *drsurf)
+{
+    if (!ctx) return GORT_ERR_INVALID;
+    TRY(check_shape(ctx, shape, "gort_brdf_tangent_batch"));
+    if (!structure || !lut || !dlut || !angles || !rleaf || !tleaf || !rsoil || !drsurf)
+        return set_error(ctx, GORT_ERR_INVALID, "gort_brdf_tangent_batch: NULL argument");
+    if (shape->out_pitch != 0) return set_error(ctx, GORT_ERR_INVALID, "gort_brdf_tangent_batch: drsurf is dense (out_pitch must be 0)");
+    TRYCUDA(ctx, cudaSetDevice(ctx->device), "cudaSetDevice");
+    const cudaStream_t s = pick(ctx, stream);
+    TRY(order_after_previous(ctx, s));
+    return launch_brdf_tangent(ctx, s, *shape, structure, lut, dlut, angles, rleaf, tleaf, rsoil, drsurf, 0);
+}
+
+int gort_lai_tangent_batch(gort_ctx *ctx, const gort_shape *shape, int lut_method, int param, const double *structure,
+                           const double *leaf, const double *soil, double user_leaf, double user_soil,
+                           const double *wavelength, const double *angles, double *jac, double *rsurf)
+{
+    if (!ctx) return GORT_ERR_INVALID;
+    TRY(check_shape(ctx, shape, "gort_lai_tangent_batch"));
+    if (!structure || !wavelength || !angles || !jac || (user_leaf < 0.0 && !leaf) || (user_soil < 0.0 && !soil))
+        return set_error(ctx, GORT_ERR_INVALID, "gort_lai_tangent_batch: NULL argument");
+    if (param != GORT_JAC_FAVD && param != GORT_JAC_LAI)
+        return set_error(ctx, GORT_ERR_INVALID, "gort_lai_tangent_batch: parameter %d is not GORT_JAC_FAVD or GORT_JAC_LAI", param);
+    if (lut_method != GORT_LUT_FULL && lut_method != GORT_LUT_Q08)
+        return set_error(ctx, GORT_ERR_INVALID, "gort_lai_tangent_batch: unknown LUT method %d", lut_method);
+    const size_t G = shape->n_geom, W = shape->n_wl;
+    for (size_t i = 0; i < W; i++)
+        if (wavelength[i] < GORT_WL_MIN || wavelength[i] > GORT_WL_MAX)
+            return set_error(ctx, GORT_ERR_RANGE, "wavlength out of range (400-2500)");
+    TRYCUDA(ctx, cudaSetDevice(ctx->device), "cudaSetDevice");
+    double *d_wl, *d_ang_shared = NULL;
+    TRY(h2d(ctx, 22, wavelength, W, &d_wl));
+    if (!shape->geom_per_set) TRY(h2d(ctx, 23, angles, 4 * G, &d_ang_shared));
+    gort_shape sh = *shape;
+    sh.spectra_per_set = 1;
+    sh.out_pitch = 0;
+    // chunk buffers: out[0] jac, out[1] rsurf, out[2] the LUT tangent
+    const size_t out_pm[3] = {G * W, rsurf ? G * W : 0, GORT_LUT_STRIDE};
+    const EnsCopy copies[2] = {{jac, 0, G * W}, {rsurf, 1, G * W}};
+    return ensemble_chunks(ctx, shape, structure, leaf, soil, user_leaf, user_soil, angles, W, out_pm, 2, copies, "gort_lai_tangent_batch",
+                           [&](cudaStream_t A, size_t c, const EnsBufs &d) {
+        sh.n_sets = (int) c;
+        const double *ang = sh.geom_per_set ? d.ang : d_ang_shared;
+        TRY(launch_lut_tangent(ctx, A, (int) c, d.st, lut_method, d.lut, d.out[2]));
+        TRY(launch_spectra(ctx, A, (int) c, user_leaf < 0.0 ? d.leaf : NULL, user_soil < 0.0 ? d.soil : NULL, user_leaf, user_soil,
+                           (int) W, d_wl, d.rl, d.tl, d.rs));
+        // rsurf from the existing BRDF kernels on this LUT: the bits of gort_forward_batch
+        if (rsurf) TRY(launch_brdf(ctx, A, sh, d.st, d.lut, ang, d.rl, d.tl, d.rs, d.out[1], NULL, NULL));
+        return launch_brdf_tangent(ctx, A, sh, d.st, d.lut, d.out[2], ang, d.rl, d.tl, d.rs, d.out[0], param == GORT_JAC_LAI);
+    });
 }
 
 int gort_energy_batch_dev(gort_ctx *ctx, void *stream, const gort_shape *shape, const double *structure,
@@ -900,7 +1004,7 @@ int gort_forward_band_batch(gort_ctx *ctx, const gort_shape *shape, int lut_meth
         return set_error(ctx, GORT_ERR_INVALID, "gort_forward_band_batch: NULL argument");
     if (lut_method != GORT_LUT_FULL && lut_method != GORT_LUT_Q08)
         return set_error(ctx, GORT_ERR_INVALID, "gort_forward_band_batch: unknown LUT method %d", lut_method);
-    const size_t M = shape->n_sets, G = shape->n_geom, W = shape->n_wl, B = n_bands;
+    const size_t G = shape->n_geom, W = shape->n_wl, B = n_bands;
     for (size_t i = 0; i < W; i++)
         if (wavelength[i] < GORT_WL_MIN || wavelength[i] > GORT_WL_MAX)
             return set_error(ctx, GORT_ERR_RANGE, "wavlength out of range (400-2500)");
@@ -918,63 +1022,26 @@ int gort_forward_band_batch(gort_ctx *ctx, const gort_shape *shape, int lut_meth
         for (size_t b = 0; b < B; b++) w_u[b * U + k] = weights[b * W + cols[k]];
     }
     TRYCUDA(ctx, cudaSetDevice(ctx->device), "cudaSetDevice");
-    if (!ctx->copy_stream) {
-        TRYCUDA(ctx, cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking), "cudaStreamCreate");
-        TRYCUDA(ctx, cudaStreamCreateWithFlags(&ctx->copy_stream_out, cudaStreamNonBlocking), "cudaStreamCreate");
-        for (int i = 0; i < 6; i++) TRYCUDA(ctx, cudaEventCreateWithFlags(&ctx->fwd_ev[i], cudaEventDisableTiming), "cudaEventCreate");
-    }
-    // streams, chunking and events as gort_forward_batch
-    cudaStream_t A = ctx->stream, Bs = ctx->copy_stream, D = ctx->copy_stream_out;
-    size_t C = (M + 7) / 8;
-    if (C > 16384) C = 16384;
-    if (C < 1024) C = 1024;
-    if (C > M) C = M;
-    const bool per_set_geom = shape->geom_per_set != 0;
-    TRY(order_after_previous(ctx, A));
-    // slots 0-8 and 9-17: the two chunk buffers; 18 the union's wavelengths, 19 shared angles, 20 the union's weights
+    // slot 22 the union's wavelengths, 23 shared angles, 24 the union's weights
     double *d_wl, *d_ang_shared = NULL, *d_w;
-    TRY(h2d(ctx, 18, wl_u.data(), U, &d_wl));
-    if (!per_set_geom) TRY(h2d(ctx, 19, angles, 4 * G, &d_ang_shared));
-    TRY(h2d(ctx, 20, w_u.data(), B * U, &d_w));
-    double *buf[2][9];
-    const size_t sz[9] = {6 * C, 7 * C, 4 * C, per_set_geom ? 4 * C * G : 8, C * GORT_LUT_STRIDE, C * U, C * U, C * U, C * G * B};
-    for (int b = 0; b < 2; b++)
-        for (int k = 0; k < 9; k++) {
-            buf[b][k] = (double *) scratch(ctx, 9 * b + k, sz[k] * sizeof(double));
-            if (!buf[b][k]) return GORT_ERR_NOMEM;
-        }
+    TRY(h2d(ctx, 22, wl_u.data(), U, &d_wl));
+    if (!shape->geom_per_set) TRY(h2d(ctx, 23, angles, 4 * G, &d_ang_shared));
+    TRY(h2d(ctx, 24, w_u.data(), B * U, &d_w));
     gort_shape sh = *shape;
     sh.n_wl = (int) U;
     sh.spectra_per_set = 1;
-    int chunk_no = 0;
-    for (size_t m0 = 0; m0 < M; m0 += C, chunk_no++) {
-        const size_t c = M - m0 < C ? M - m0 : C;
-        const int b = chunk_no & 1;
-        if (chunk_no >= 2) TRYCUDA(ctx, cudaStreamWaitEvent(Bs, ctx->fwd_ev[2 + b], 0), "cudaStreamWaitEvent");
-        TRY(copy_rows(ctx, Bs, buf[b][0], c, structure + m0, M, c, 6, cudaMemcpyHostToDevice, "forward: structure"));
-        if (user_leaf < 0.0) TRY(copy_rows(ctx, Bs, buf[b][1], c, leaf + m0, M, c, 7, cudaMemcpyHostToDevice, "forward: leaf"));
-        if (user_soil < 0.0) TRY(copy_rows(ctx, Bs, buf[b][2], c, soil + m0, M, c, 4, cudaMemcpyHostToDevice, "forward: soil"));
-        if (per_set_geom) TRY(copy_rows(ctx, Bs, buf[b][3], c * G, angles + m0 * G, M * G, c * G, 4, cudaMemcpyHostToDevice, "forward: angles"));
-        TRYCUDA(ctx, cudaEventRecord(ctx->fwd_ev[b], Bs), "cudaEventRecord");
-        TRYCUDA(ctx, cudaStreamWaitEvent(A, ctx->fwd_ev[b], 0), "cudaStreamWaitEvent");
-        if (chunk_no >= 2) TRYCUDA(ctx, cudaStreamWaitEvent(A, ctx->fwd_ev[4 + b], 0), "cudaStreamWaitEvent");
+    const size_t out_pm[3] = {G * B, 0, 0};
+    const EnsCopy copies[2] = {{rband, 0, G * B}, {lut_out, -1, GORT_LUT_STRIDE}};
+    // streams, chunking and events as gort_forward_batch
+    return ensemble_chunks(ctx, shape, structure, leaf, soil, user_leaf, user_soil, angles, U, out_pm, 2, copies, "gort_forward_band_batch",
+                           [&](cudaStream_t A, size_t c, const EnsBufs &d) {
         sh.n_sets = (int) c;
-        TRY(launch_lut(ctx, A, (int) c, buf[b][0], lut_method, buf[b][4]));
-        TRY(launch_spectra(ctx, A, (int) c, user_leaf < 0.0 ? buf[b][1] : NULL, user_soil < 0.0 ? buf[b][2] : NULL, user_leaf, user_soil,
-                           (int) U, d_wl, buf[b][5], buf[b][6], buf[b][7]));
-        TRY(launch_brdf_band(ctx, A, sh, n_bands, d_w, buf[b][0], buf[b][4], per_set_geom ? buf[b][3] : d_ang_shared,
-                             buf[b][5], buf[b][6], buf[b][7], buf[b][8]));
-        TRYCUDA(ctx, cudaEventRecord(ctx->fwd_ev[2 + b], A), "cudaEventRecord");
-        TRYCUDA(ctx, cudaStreamWaitEvent(D, ctx->fwd_ev[2 + b], 0), "cudaStreamWaitEvent");
-        TRYCUDA(ctx, cudaMemcpyAsync(rband + m0 * G * B, buf[b][8], c * G * B * sizeof(double), cudaMemcpyDeviceToHost, D), "forward: rband");
-        if (lut_out) TRYCUDA(ctx, cudaMemcpyAsync(lut_out + m0 * GORT_LUT_STRIDE, buf[b][4], c * GORT_LUT_STRIDE * sizeof(double), cudaMemcpyDeviceToHost, D), "forward: lut");
-        TRYCUDA(ctx, cudaEventRecord(ctx->fwd_ev[4 + b], D), "cudaEventRecord");
-    }
-    TRYCUDA(ctx, cudaStreamSynchronize(D), "gort_forward_band_batch");
-    TRYCUDA(ctx, cudaStreamSynchronize(Bs), "gort_forward_band_batch");
-    TRYCUDA(ctx, cudaStreamSynchronize(A), "gort_forward_band_batch");
-    note_other_work(ctx);
-    return check_pipeline_fault(ctx);
+        TRY(launch_lut(ctx, A, (int) c, d.st, lut_method, d.lut));
+        TRY(launch_spectra(ctx, A, (int) c, user_leaf < 0.0 ? d.leaf : NULL, user_soil < 0.0 ? d.soil : NULL, user_leaf, user_soil,
+                           (int) U, d_wl, d.rl, d.tl, d.rs));
+        return launch_brdf_band(ctx, A, sh, n_bands, d_w, d.st, d.lut, sh.geom_per_set ? d.ang : d_ang_shared,
+                                d.rl, d.tl, d.rs, d.out[0]);
+    });
 }
 
 int gort_gauleg(gort_ctx *ctx, double *abscissa, double *weights)

@@ -378,7 +378,7 @@ static int ensure_flags(gort_ctx *ctx, cudaStream_t s, int which, size_t n)
 
 // the record buffer and flag array of a new call: double-buffered by call parity, so that this call's geometry kernel
 // may run while the previous call's per-wavelength kernel still reads its own
-static int next_records(gort_ctx *ctx, cudaStream_t s, long L, double **rec, unsigned long long **flags)
+int next_records(gort_ctx *ctx, cudaStream_t s, long L, double **rec, unsigned long long **flags)
 {
     ctx->call_no++;
     ctx->rec_idx ^= 1;
@@ -393,8 +393,8 @@ static int next_records(gort_ctx *ctx, cudaStream_t s, long L, double **rec, uns
 
 // geometry records of every line of a call (and kprop when asked for), with their per-tile ready flags.  pdl: launch as a
 // programmatic dependent of the previous kernel on the stream (overlap mode); otherwise plain stream order.
-static int launch_geom(gort_ctx *ctx, cudaStream_t s, const gort_shape &sh, const double *structure, const double *lut,
-                       const double *angles, double *rec, double *kprop, unsigned long long *flags, bool pdl)
+int launch_geom(gort_ctx *ctx, cudaStream_t s, const gort_shape &sh, const double *structure, const double *lut,
+                const double *angles, double *rec, double *kprop, unsigned long long *flags, bool pdl)
 {
     const long L = (long) sh.n_sets * sh.n_geom;
     // the per-wavelength kernel that follows needs a large shared-memory carve-out; an SM only changes its

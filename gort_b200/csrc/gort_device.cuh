@@ -433,4 +433,106 @@ __device__ __forceinline__ double view_rsurf(const Canopy& c, const LeafTerms& L
     return fma(Kz, S.Z, fma(Kt, S.T, fma(Kg, S.G, Kc * C))); // gortt.c:557
 }
 
+// ---- forward-mode tangent with respect to favd (gort_brdf_tangent_batch_dev) --------------------------------------
+// favd enters the BRDF through elai, kfavd and the LUT record (epgap rows, k_openep); dlut is the record's tangent.
+// Everything else of the record (Kc, Kg, Kt, Kz, K'g, K'z, fd, mus) does not depend on it.  At the few kinks the
+// derivative is that of the branch the forward computation takes.
+
+// d elai / d favd: elai without its favd factor (gortt.c:657)
+__device__ __forceinline__ double elai_tangent(const Canopy& c)
+{
+    return (1.333333) * c.lambda * GORT_PI * c.ellip * (c.rr * c.r);
+}
+
+// tangents of the Kuusk hotspot (gortt_brdf.c:638-702) and of the sun-side LUT interpolation; the forward values are
+// formed again exactly as hotspot() forms them, so every branch is the forward's
+struct HotTan { double dkuusk, dpn0_s, dpe_s; };
+__device__ __forceinline__ HotTan hotspot_tangent(const Canopy& c, const double* __restrict__ lut_m,
+                                                  const double* __restrict__ dlut_m, double vza, double sza, double cr)
+{
+    HotTan o;
+    double pn0_s, pe_s, pn0_v, pe_v, dpn0_v, dpe_v;
+    zenith_lerp(lut_m, sza, pn0_s, pe_s);
+    zenith_lerp(lut_m, vza, pn0_v, pe_v);
+    zenith_lerp(dlut_m, sza, o.dpn0_s, o.dpe_s);          // zenith_lerp is linear in the rows
+    zenith_lerp(dlut_m, vza, dpn0_v, dpe_v);
+    double ssz, csz, svz, cvz;
+    sincos(sza, &ssz, &csz);
+    sincos(vza, &svz, &cvz);
+    const double cos_xi = csz * cvz + ssz * svz * cr;
+    const double dk = 0.5;                                 // d kfavd / d favd
+    const double lsza = -log(pe_s) / c.kfavd;
+    const double lvza = -log(pe_v) / c.kfavd;
+    const double dlsza = (-(o.dpe_s / pe_s) - lsza * dk) / c.kfavd;
+    const double dlvza = (-(dpe_v / pe_v) - lvza * dk) / c.kfavd;
+    const double arg = lsza * lsza + lvza * lvza - 2. * lsza * lvza * cos_xi;
+    double t1, t2, dt1 = 0.0, dt2 = 0.0;
+    if (arg > 0.0) {
+        const double lsv = sqrt(arg);
+        const double darg = 2.0 * (lsza * dlsza + lvza * dlvza - cos_xi * (dlsza * lvza + lsza * dlvza));
+        const double x = lsv / c.r, ex = exp(-x);
+        t2 = (1.0 - ex) / x;
+        dt2 = (ex - t2) / x * (darg / (2.0 * lsv) / c.r);   // d/dx (1 - e^-x)/x = (e^-x - t2)/x
+    } else {
+        t2 = 1.0;
+    }
+    if ((lsza * lvza) > 0.0) {
+        t1 = sqrt(lsza * lvza);
+        dt1 = (dlsza * lvza + lsza * dlvza) / (2.0 * t1);
+    } else {
+        t1 = 0.0;
+    }
+    const double H = exp(c.kfavd * t1 * t2);
+    const double dH = H * (dk * t1 * t2 + c.kfavd * (dt1 * t2 + t1 * dt2));
+    o.dkuusk = (o.dpe_s * pe_v + pe_s * dpe_v) * H + pe_s * pe_v * dH;
+    return o;
+}
+
+// tangents of the (set, lambda) terms; dkoe = d k_openep / d favd (k_open has none)
+struct LeafTan { double dTff, dpff, dtff, dtpff, dXf, dZf; };
+__device__ __forceinline__ LeafTan leaf_tangent(const Canopy& c, const LeafTerms& L, double delai, double dkoe)
+{
+    LeafTan D;
+    D.dTff = -(L.gam * delai) * L.Tff;
+    const double tr = L.Tff * L.Rff;
+    const double den = 1. - tr * tr;
+    const double dden = -2.0 * tr * L.Rff * D.dTff;
+    D.dpff = fdiv(-2.0 * L.Rff * L.Tff * D.dTff - L.pff * dden, den);
+    D.dtff = fdiv(D.dTff * (1. - L.Rff * L.Rff) - L.tff * dden, den);
+    const double K = c.k_open + c.k_openep;
+    D.dtpff = D.dtff * (1.0 - K) + (1.0 - L.tff) * dkoe;
+    const double u = fdiv(L.rs, 1.0 - L.rs * L.pff);
+    D.dXf = (u * u * D.dpff) * (L.tpff - c.k_open) + u * D.dtpff;
+    D.dZf = (D.dtpff - dkoe) * L.rs;
+    return D;
+}
+
+// the (sun, lambda) terms the tangent evaluation needs: G and Z, and the tangents of Z, PDF and T (sun_terms' chain)
+struct SunTan { double G, Z, dZ, dPDF, dT; };
+__device__ __forceinline__ SunTan sun_tangent(const Canopy& c, const LeafTerms& L, const LeafTan& D, double dkoe,
+                                              double fd, double mus, double t0, double tp0, double pe_s,
+                                              double dt0, double dtp0, double dpe_s)
+{
+    SunTan O;
+    const double two_mu_g = 2.0 * mus * L.gam;
+    const double Rdf = fdiv(1.0 - L.gam, 1.0 + two_mu_g);
+    const double cT = (L.omega / 2.0) * fdiv(1. + 2. * mus, 1. - two_mu_g * two_mu_g);
+    const double Tdf = cT * (L.Tff - t0), dTdf = cT * (D.dTff - dt0);
+    const double SS = t0 * Rdf + Tdf * L.Rff, dSS = dt0 * Rdf + dTdf * L.Rff;
+    const double tdf = Tdf - L.pff * SS, dtdf = dTdf - D.dpff * SS - L.pff * dSS;
+    const double dpdf = -(D.dtff * SS + L.tff * dSS);
+    const double tpdf = tdf * (1 - tp0), dtpdf = dtdf * (1 - tp0) - tdf * dtp0;
+    const double omf = 1 - fd;
+    O.G = fd * L.rs + omf * L.rs;
+    O.Z = fd * ((tpdf + pe_s) * L.rs) + omf * L.Zf;
+    O.dZ = fd * ((dtpdf + dpe_s) * L.rs) + omf * D.dZf;
+    const double K = c.k_open + c.k_openep;
+    const double dCfG = (dkoe * (O.G - O.Z) + (1 - K) * O.dZ) * c.k_openep + (K * O.G + (1 - K) * O.Z) * dkoe;
+    const double dCdCG = (dtpdf + dtp0) * L.Xf + (tpdf + tp0) * D.dXf;
+    const double dCfCG = D.dtpff * L.Xf + L.tpff * D.dXf;
+    O.dT = fd * dCdCG + omf * dCfCG;
+    O.dPDF = fd * (dpdf + dCdCG) + omf * (D.dpff + dCfG + dCfCG);
+    return O;
+}
+
 }  // namespace gort

@@ -46,7 +46,7 @@ struct gort_ctx {
     cudaEvent_t xstream_ev;            // orders calls issued on different streams (order_after_previous)
     struct { int key_lpt, key_scomp, key_tmab, key_threads; int occ; } wide_plan[8];
     int n_wide_plan;
-    int geom_carveout_set, lut_attr_set, band_attr_set;
+    int geom_carveout_set, lut_attr_set, lut_tan_attr_set, band_attr_set;
     // development switch, read once from the environment by gort_create: GORT_TIMELINE=<call number>
     int dbg_timeline;
     unsigned long long *d_timeline;
@@ -80,6 +80,14 @@ int order_after_previous(gort_ctx *ctx, cudaStream_t s);
 int launch_brdf(gort_ctx *ctx, cudaStream_t s, const gort_shape &sh, const double *structure,
                 const double *lut, const double *angles, const double *rleaf, const double *tleaf,
                 const double *rsoil, double *rsurf, double *scomp, double *kprop);
+// the BRDF pipeline's record buffer and flags for a new call, and the geometry kernel that fills them (gort_brdf.cu)
+int next_records(gort_ctx *ctx, cudaStream_t s, long L, double **rec, unsigned long long **flags);
+int launch_geom(gort_ctx *ctx, cudaStream_t s, const gort_shape &sh, const double *structure, const double *lut,
+                const double *angles, double *rec, double *kprop, unsigned long long *flags, bool pdl);
+// favd tangent of rsurf, drsurf [M][G][W] dense; lai != 0 scales it by d favd / d LAI (gort_tangent.cu)
+int launch_brdf_tangent(gort_ctx *ctx, cudaStream_t s, const gort_shape &sh, const double *structure, const double *lut,
+                        const double *dlut, const double *angles, const double *rleaf, const double *tleaf,
+                        const double *rsoil, double *drsurf, int lai);
 int launch_energy(gort_ctx *ctx, cudaStream_t s, const gort_shape &sh, const double *structure,
                   const double *lut, const double *angles, const double *rleaf, const double *tleaf,
                   const double *rsoil, double *albedo, double *favegt, double *fasoil);
@@ -93,6 +101,9 @@ int launch_energy_band(gort_ctx *ctx, cudaStream_t s, const gort_shape &sh, int 
 int launch_lut(gort_ctx *ctx, cudaStream_t s, int n_sets, const double *structure, int method, double *lut);
 int launch_lut_out(gort_ctx *ctx, cudaStream_t s, int n_sets, const double *structure, int method, double *lut,
                    int n_dst, double *const *dst, int multicast);
+// the same records and dlut [n_sets][GORT_LUT_STRIDE] = their favd tangent (gort_lut_tangent_batch_dev)
+int launch_lut_tangent(gort_ctx *ctx, cudaStream_t s, int n_sets, const double *structure, int method, double *lut,
+                       double *dlut);
 int launch_lut_dead(gort_ctx *ctx, cudaStream_t s, int n_sets, const double *structure, double *vb, double *fb,
                     double *t_open, double *dt_open, double *dk_open, double *k_open);
 int launch_spectra(gort_ctx *ctx, cudaStream_t s, int n_sets, const double *leaf, const double *soil,

@@ -652,16 +652,30 @@ struct CrownSmem {
                                              // read with four 16-byte loads instead of eight 8-byte ones
     double part[LUT_NSP][SUB][32];           // partial within-crown gap sums per entry height
 };
-#define LUT_CROWN_OCC(SUB) ((SUB) == 1 ? 3 : 2)
-
+// the tangent kernels add the partial sums of the favd tangent
 template <int SUB>
-__global__ void __launch_bounds__(32 * LUT_NSP, LUT_CROWN_OCC(SUB))
-lut_crown_kernel(int m0, const double* __restrict__ structure, size_t N, LutWork w, const LutOut out)
+struct CrownSmemTan {
+    CrownSmem<SUB> p;
+    double dpart[LUT_NSP][SUB][32];
+};
+#define LUT_CROWN_OCC(SUB) ((SUB) == 1 ? 3 : 2)
+#define LUT_CROWN_TAN_OCC(SUB) ((SUB) == 1 ? 3 : 1)
+
+// TAN = true: the same records and dlut, their favd tangent (p_n0 rows 0, epgap rows).  favd enters the record only
+// through the bin attenuation exp(-s_bin tau'), s_bin = row ds, tau' = 0.5 favd b/r, whose favd derivative is
+// -0.5 (b/r) ds row exp(-s_bin tau').  The factor -0.5 (b/r) ds is common to the sub-group (one shape), so the tangent
+// accumulates sum row wgt exp(-s_bin tau') next to the primal sum -- one more FMA per member and crown count -- and is
+// scaled once when the row is stored.  The bins, the weights and the primal arithmetic are those of the primal kernel.
+template <int SUB, bool TAN>
+__global__ void __launch_bounds__(32 * LUT_NSP, TAN ? LUT_CROWN_TAN_OCC(SUB) : LUT_CROWN_OCC(SUB))
+lut_crown_kernel(int m0, const double* __restrict__ structure, size_t N, LutWork w, const LutOut out,
+                 double* __restrict__ dlut)
 {
     extern __shared__ __align__(16) unsigned char crown_smem_raw[];
     CrownSmem<SUB>& sm = *reinterpret_cast<CrownSmem<SUB>*>(crown_smem_raw);
     double (*s_tab)[SUB] = sm.tab;
     double (*s_part)[SUB][32] = sm.part;
+    double (*s_dpart)[SUB][32] = TAN ? reinterpret_cast<CrownSmemTan<SUB>*>(crown_smem_raw)->dpart : nullptr;
     const int lane = threadIdx.x & 31, k = threadIdx.x >> 5;
     const int* __restrict__ list = SUB == 1 ? w.s1 : w.s8;
     const int n_items = 3 * w.cnt[SUB == 1 ? 1 : 2];
@@ -694,9 +708,13 @@ lut_crown_kernel(int m0, const double* __restrict__ structure, size_t N, LutWork
         s_tab[bin][j] = exp(-sbin * (0.5 * favd_p));
     }
     const bool live = t < GORT_NTH, path = t < GORT_NTH - 1;
-    double e_t[SUB];
+    double e_t[SUB], de_t[SUB];
 #pragma unroll
     for (int j = 0; j < SUB; j++) e_t[j] = 0.0;
+    if (TAN) {
+#pragma unroll
+        for (int j = 0; j < SUB; j++) de_t[j] = 0.0;
+    }
     const double* vg = w.vg + (size_t) hd * GORT_NLAYERS * LUT_ZW + t;
     double pn0_0 = 0.0;
     if (live && k == 0) pn0_0 = exp(-1.0 * lv_p * vg[0]);                        // gortt_pn_kopen.c:30: the p_n0 row of the LUT
@@ -746,9 +764,11 @@ lut_crown_kernel(int m0, const double* __restrict__ structure, size_t N, LutWork
             redo |= (frac - 2u) > (0x3fffffffu - 4u);
             ub_last = ubd;
             const int row = min(idx, n_tab - 1);
+            const double rw = TAN ? (double) row * wgt : 0.0;
             // gortt_calc_epgap + gortt_calc_pgap, :1110-1114, :1138
             if (SUB == 1) {
                 e_t[0] = fma(s_tab[row][0], wgt, e_t[0]);
+                if (TAN) de_t[0] = fma(s_tab[row][0], rw, de_t[0]);
             } else {
                 const double2* __restrict__ tp = reinterpret_cast<const double2*>(&s_tab[row][0]);
 #pragma unroll
@@ -756,6 +776,10 @@ lut_crown_kernel(int m0, const double* __restrict__ structure, size_t N, LutWork
                     const double2 v = tp[j2];
                     e_t[2 * j2] = fma(v.x, wgt, e_t[2 * j2]);
                     e_t[2 * j2 + 1] = fma(v.y, wgt, e_t[2 * j2 + 1]);
+                    if (TAN) {
+                        de_t[2 * j2] = fma(v.x, rw, de_t[2 * j2]);
+                        de_t[2 * j2 + 1] = fma(v.y, rw, de_t[2 * j2 + 1]);
+                    }
                 }
             }
         }
@@ -764,6 +788,10 @@ lut_crown_kernel(int m0, const double* __restrict__ structure, size_t N, LutWork
         if (redo) {
 #pragma unroll
             for (int j = 0; j < SUB; j++) e_t[j] = 0.0;
+            if (TAN) {
+#pragma unroll
+                for (int j = 0; j < SUB; j++) de_t[j] = 0.0;
+            }
             pw = c0; qn = 1.0;
 #pragma unroll 1
             for (int nn = 1; nn <= LUT_MAXCROWNS; nn++) {
@@ -774,15 +802,26 @@ lut_crown_kernel(int m0, const double* __restrict__ structure, size_t N, LutWork
                 if (fabs(u - rint(u)) < 1e-9)
                     u = sp * (1.0 - exp(-1.0 * (double) nn * es / sp)) / S.c.ds + 0.5;   // the literal formula, :508, :134-139
                 const int idx = (int) u;
+                const double rw = TAN ? (double) idx * wgt : 0.0;
                 if (idx >= 0 && idx < n_tab) {
 #pragma unroll
                     for (int j = 0; j < SUB; j++) e_t[j] = fma(s_tab[idx][j], wgt, e_t[j]);
+                    if (TAN) {
+#pragma unroll
+                        for (int j = 0; j < SUB; j++) de_t[j] = fma(s_tab[idx][j], rw, de_t[j]);
+                    }
                 } else {
                     const double sbin = (double) idx * S.c.ds;
 #pragma unroll
                     for (int j = 0; j < SUB; j++) {                              // beyond the table: the formula itself
                         const double tau_j = 0.5 * (structure[5 * N + m + (j < nj ? j : 0)] * S.ellip);
-                        e_t[j] = fma(exp(-sbin * tau_j), wgt, e_t[j]);
+                        if (TAN) {
+                            const double x = exp(-sbin * tau_j);
+                            e_t[j] = fma(x, wgt, e_t[j]);
+                            de_t[j] = fma(x, rw, de_t[j]);
+                        } else {
+                            e_t[j] = fma(exp(-sbin * tau_j), wgt, e_t[j]);
+                        }
                     }
                 }
             }
@@ -790,16 +829,27 @@ lut_crown_kernel(int m0, const double* __restrict__ structure, size_t N, LutWork
     }
 #pragma unroll
     for (int j = 0; j < SUB; j++) s_part[k][j][lane] = e_t[j];
+    if (TAN) {
+#pragma unroll
+        for (int j = 0; j < SUB; j++) s_dpart[k][j][lane] = de_t[j];
+    }
     __syncthreads();
     // rows of the LUT record: p_n0[0][t] and epgap[0][t] (the 13 entry heights added in the reference's order, :457);
     // the openness factors are formed by kopen_kernel afterwards
     if (live) {
         if (k == 0) for (int j = 0; j < nj; j++) lut_store(out, (size_t) (m + j) * GORT_LUT_STRIDE + t, pn0_0);
+        if (TAN && k == 0) for (int j = 0; j < nj; j++) dlut[(size_t) (m + j) * GORT_LUT_STRIDE + t] = 0.0;   // p_n0 has no favd
         for (int j = k; j < nj; j += LUT_NSP) {
             double e = s_part[0][j][lane];
 #pragma unroll
             for (int q2 = 1; q2 < LUT_NSP; q2++) e += s_part[q2][j][lane];
             lut_store(out, (size_t) (m + j) * GORT_LUT_STRIDE + GORT_NTH + t, e);
+            if (TAN) {
+                double de = s_dpart[0][j][lane];
+#pragma unroll
+                for (int q2 = 1; q2 < LUT_NSP; q2++) de += s_dpart[q2][j][lane];
+                dlut[(size_t) (m + j) * GORT_LUT_STRIDE + GORT_NTH + t] = de * (-(0.5 * S.ellip) * S.c.ds);
+            }
         }
     }
   }
@@ -941,13 +991,18 @@ lut_dead_kernel(int n, int m0, const double* __restrict__ structure, size_t N, L
     }
 }
 
-// gortt_pn_kopen.c:1144-1200
-__global__ void __launch_bounds__(LUT_THREADS)
-lut_q08_kernel(int n_sets, const double* __restrict__ structure, double* __restrict__ lut)
+// gortt_pn_kopen.c:1144-1200; with TAN also dlut, the favd tangent of the closed form: l is linear in favd
+// (dl = b 4/3 cc), a = cc (exp(k1 cc^2) - exp(-k2 l)) gives da = cc k2 exp(-k2 l) dl, and
+// epg = exp(-a / cos theta') - pn0 gives depg = -(da / cos theta') exp(-a / cos theta'); the same trapezoid on the
+// tangent rows gives dk_openep.  p_n0 and k_open have no favd.
+template <bool TAN>
+__device__ __forceinline__ void q08_record(int n_sets, const double* __restrict__ structure, double* __restrict__ lut,
+                                           double* __restrict__ dlut)
 {
     __shared__ double s_pn0[GORT_NTH];
     __shared__ double s_epg[GORT_NTH];
     __shared__ double s_sin2[GORT_NTH];
+    __shared__ double s_depg[TAN ? GORT_NTH : 1];
     const int m = blockIdx.x;
     const int t = threadIdx.x;
     const double lambda = structure[0 * (size_t) n_sets + m];
@@ -973,6 +1028,16 @@ lut_q08_kernel(int n_sets, const double* __restrict__ structure, double* __restr
         double* o = lut + (size_t) m * GORT_LUT_STRIDE;
         o[t] = pn0;
         o[GORT_NTH + t] = epg;
+        if (TAN) {
+            const double dl = b * 4. / 3. * cc;
+            const double da = cc * (k2 * exp(-k2 * l)) * dl;
+            const double ct = cos(theta_p);
+            const double depg = -(da / ct) * exp(-a / ct);
+            s_depg[t] = depg;
+            double* d = dlut + (size_t) m * GORT_LUT_STRIDE;
+            d[t] = 0.0;
+            d[GORT_NTH + t] = depg;
+        }
     }
     __syncthreads();
     if (t == 0) {
@@ -990,7 +1055,30 @@ lut_q08_kernel(int n_sets, const double* __restrict__ structure, double* __restr
         double* o = lut + (size_t) m * GORT_LUT_STRIDE;
         o[2 * GORT_NTH] = ko;
         o[2 * GORT_NTH + 1] = ke;
+        if (TAN) {
+            double dke = 0.0, last = 0.0 * s_sin2[0];
+            for (int i = 1; i < GORT_NTH; i++) {
+                const double tmp = s_depg[i] * s_sin2[i];
+                dke += (tmp + last) / 2.0 * dth;
+                last = tmp;
+            }
+            double* d = dlut + (size_t) m * GORT_LUT_STRIDE;
+            d[2 * GORT_NTH] = 0.0;
+            d[2 * GORT_NTH + 1] = dke;
+        }
     }
+}
+
+__global__ void __launch_bounds__(LUT_THREADS)
+lut_q08_kernel(int n_sets, const double* __restrict__ structure, double* __restrict__ lut)
+{
+    q08_record<false>(n_sets, structure, lut, nullptr);
+}
+
+__global__ void __launch_bounds__(LUT_THREADS)
+lut_q08_tangent_kernel(int n_sets, const double* __restrict__ structure, double* __restrict__ lut, double* __restrict__ dlut)
+{
+    q08_record<true>(n_sets, structure, lut, dlut);
 }
 
 // gortt_calc_kopen, gortt_pn_kopen.c:351-375 for h = 0: k_open = trapezoid rule of p_n0 sin(2 theta) over the 91
@@ -1071,6 +1159,9 @@ int launch_lut_dead(gort_ctx *ctx, cudaStream_t s, int n_sets, const double *str
     return check_cuda(ctx, cudaGetLastError(), "gort_lut_intermediates launch");
 }
 
+static int launch_lut_impl(gort_ctx *ctx, cudaStream_t s, int n_sets, const double *structure, int method, double *lut,
+                           int n_dst, double *const *dst, int multicast, double *dlut);
+
 int launch_lut(gort_ctx *ctx, cudaStream_t s, int n_sets, const double *structure, int method, double *lut)
 {
     return launch_lut_out(ctx, s, n_sets, structure, method, lut, 0, NULL, 0);
@@ -1079,6 +1170,19 @@ int launch_lut(gort_ctx *ctx, cudaStream_t s, int n_sets, const double *structur
 int launch_lut_out(gort_ctx *ctx, cudaStream_t s, int n_sets, const double *structure, int method, double *lut,
                    int n_dst, double *const *dst, int multicast)
 {
+    return launch_lut_impl(ctx, s, n_sets, structure, method, lut, n_dst, dst, multicast, NULL);
+}
+
+int launch_lut_tangent(gort_ctx *ctx, cudaStream_t s, int n_sets, const double *structure, int method, double *lut,
+                       double *dlut)
+{
+    return launch_lut_impl(ctx, s, n_sets, structure, method, lut, 0, NULL, 0, dlut);
+}
+
+// dlut != NULL: the tangent kernels, which also write dlut (no further destinations then)
+static int launch_lut_impl(gort_ctx *ctx, cudaStream_t s, int n_sets, const double *structure, int method, double *lut,
+                           int n_dst, double *const *dst, int multicast, double *dlut)
+{
     note_other_work(ctx);
     LutOut out;
     out.local = lut;
@@ -1086,7 +1190,8 @@ int launch_lut_out(gort_ctx *ctx, cudaStream_t s, int n_sets, const double *stru
     out.mc = multicast;
     for (int q = 0; q < GORT_LUT_MAX_DST; q++) out.dst[q] = q < n_dst ? dst[q] : NULL;
     if (method == GORT_LUT_Q08) {
-        lut_q08_kernel<<<n_sets, LUT_THREADS, 0, s>>>(n_sets, structure, lut);
+        if (dlut) lut_q08_tangent_kernel<<<n_sets, LUT_THREADS, 0, s>>>(n_sets, structure, lut, dlut);
+        else lut_q08_kernel<<<n_sets, LUT_THREADS, 0, s>>>(n_sets, structure, lut);
         ctx->launches++;
         if (n_dst > 0) {
             lut_rows_out_kernel<<<ctx->sm_count * 4, 256, 0, s>>>((size_t) n_sets * GORT_LUT_STRIDE, out);
@@ -1099,9 +1204,15 @@ int launch_lut_out(gort_ctx *ctx, cudaStream_t s, int n_sets, const double *stru
     // batches, which made a 16 384-set shard of the C5 grid do 7x the geometry work).  Results do not depend on it.
     const int cap = LUT_GROUP_CAP;
     if (!ctx->lut_attr_set) {
-        cudaError_t e = cudaFuncSetAttribute(lut_crown_kernel<LUT_SUB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) sizeof(CrownSmem<LUT_SUB>));
+        cudaError_t e = cudaFuncSetAttribute(lut_crown_kernel<LUT_SUB, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) sizeof(CrownSmem<LUT_SUB>));
         if (e != cudaSuccess) return check_cuda(ctx, e, "lut_crown_kernel shared memory");
         ctx->lut_attr_set = 1;
+    }
+    if (dlut && !ctx->lut_tan_attr_set) {
+        cudaError_t e = cudaFuncSetAttribute(lut_crown_kernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) sizeof(CrownSmemTan<1>));
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(lut_crown_kernel<LUT_SUB, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) sizeof(CrownSmemTan<LUT_SUB>));
+        if (e != cudaSuccess) return check_cuda(ctx, e, "lut_crown_kernel<.., true> shared memory");
+        ctx->lut_tan_attr_set = 1;
     }
     const int chunk = n_sets < LUT_CHUNK ? n_sets : LUT_CHUNK;
     const int n_pass = (n_sets + chunk - 1) / chunk;
@@ -1139,12 +1250,26 @@ int launch_lut_out(gort_ctx *ctx, cudaStream_t s, int n_sets, const double *stru
         lut_tube_kernel<<<(unsigned) (tube_ctas < tube_max ? tube_ctas : tube_max), 32 * LUT_TUBE_WARPS, 0, s>>>(wc);
         const long items = (long) n * 3;
         const long c1 = (long) ctx->sm_count * LUT_CROWN_OCC(1), c8 = (long) ctx->sm_count * LUT_CROWN_OCC(LUT_SUB);
-        lut_crown_kernel<1><<<(unsigned) (items < c1 ? items : c1), 32 * LUT_NSP, sizeof(CrownSmem<1>), s>>>(m0, structure, N, wc, oc);
-        lut_crown_kernel<LUT_SUB><<<(unsigned) (items < c8 ? items : c8), 32 * LUT_NSP, sizeof(CrownSmem<LUT_SUB>), s>>>(m0, structure, N, wc, oc);
+        if (dlut) {
+            const long t1 = (long) ctx->sm_count * LUT_CROWN_TAN_OCC(1), t8 = (long) ctx->sm_count * LUT_CROWN_TAN_OCC(LUT_SUB);
+            lut_crown_kernel<1, true><<<(unsigned) (items < t1 ? items : t1), 32 * LUT_NSP, sizeof(CrownSmemTan<1>), s>>>(m0, structure, N, wc, oc, dlut);
+            lut_crown_kernel<LUT_SUB, true><<<(unsigned) (items < t8 ? items : t8), 32 * LUT_NSP, sizeof(CrownSmemTan<LUT_SUB>), s>>>(m0, structure, N, wc, oc, dlut);
+        } else {
+            lut_crown_kernel<1, false><<<(unsigned) (items < c1 ? items : c1), 32 * LUT_NSP, sizeof(CrownSmem<1>), s>>>(m0, structure, N, wc, oc, NULL);
+            lut_crown_kernel<LUT_SUB, false><<<(unsigned) (items < c8 ? items : c8), 32 * LUT_NSP, sizeof(CrownSmem<LUT_SUB>), s>>>(m0, structure, N, wc, oc, NULL);
+        }
         ctx->launches += 5;
     }
     kopen_kernel<<<(unsigned) (((long) n_sets * 32 + 127) / 128), 128, 0, s>>>(n_sets, out);
     ctx->launches++;
+    if (dlut) {
+        // k_open / k_openep are linear in the rows: the same trapezoid on the tangent rows
+        LutOut dout;
+        dout.local = dlut; dout.n = 0; dout.mc = 0;
+        for (int q = 0; q < GORT_LUT_MAX_DST; q++) dout.dst[q] = NULL;
+        kopen_kernel<<<(unsigned) (((long) n_sets * 32 + 127) / 128), 128, 0, s>>>(n_sets, dout);
+        ctx->launches++;
+    }
     return check_cuda(ctx, cudaGetLastError(), "gort_lut launch");
 }
 

@@ -235,6 +235,32 @@ int gort_jacobian_batch(gort_ctx *ctx, const gort_shape *shape, int lut_method, 
                         const double *structure, const double *leaf, const double *soil, double user_leaf,
                         double user_soil, const double *wavelength, const double *angles, double *jac, double *rsurf);
 
+/* ---- exact tangent of the BRDF with respect to favd (or LAI) in forward mode, for variational and Gauss-Newton
+ *      retrievals that want the gradient of gort_forward_batch to full precision.  No reference counterpart: the reference
+ *      has no derivative code (its only hook is the LAI -> favd map of gortt.c:1127-1131).  favd does not move a
+ *      histogram bin of the gap-probability LUT, so the chain is smooth in it; at the few kinks of the BRDF (the clamps
+ *      and branches of the hotspot and of the openness terms) the derivative is that of the branch the forward
+ *      computation takes.  Where the forward result is not finite (grazing angles) the tangent is not finite either.
+ *      gort_lut_tangent_batch_dev: lut as gort_lut_batch_dev writes it, bit for bit, and dlut [M][GORT_LUT_STRIDE] =
+ *        d record / d favd: the p_n0 rows and k_open are exactly 0, the epgap rows and k_openep hold the derivatives.
+ *      gort_brdf_tangent_batch_dev: drsurf [M][G][W] dense = d rsurf / d favd for the rsurf gort_brdf_batch_dev computes
+ *        from the same arguments (lut, and dlut from gort_lut_tangent_batch_dev); geom_per_set, spectra_per_set and
+ *        the options as there.  out_pitch != 0 is GORT_ERR_INVALID and nothing is enqueued.  Runs in plain stream
+ *        order and ends any overlap window (gort_set_overlap).
+ *      gort_lai_tangent_batch: the ensemble call, host pointers, arguments as gort_jacobian_batch without rel_step.
+ *        param is GORT_JAC_FAVD or GORT_JAC_LAI (anything else is GORT_ERR_INVALID); for LAI the favd tangent is
+ *        multiplied by d favd / d LAI = 3 / (4 lambda pi r^2 b).  jac [M][G][W]; rsurf (optional, may be NULL)
+ *        [M][G][W] comes from the BRDF kernels of gort_forward_batch on the same LUT, so it is bit-identical to
+ *        gort_forward_batch's.  One LUT pass per member (the central difference runs three). */
+int gort_lut_tangent_batch_dev(gort_ctx *ctx, void *stream, int n_sets, const double *structure, int method,
+                               double *lut, double *dlut);
+int gort_brdf_tangent_batch_dev(gort_ctx *ctx, void *stream, const gort_shape *shape, const double *structure,
+                                const double *lut, const double *dlut, const double *angles, const double *rleaf,
+                                const double *tleaf, const double *rsoil, double *drsurf);
+int gort_lai_tangent_batch(gort_ctx *ctx, const gort_shape *shape, int lut_method, int param, const double *structure,
+                           const double *leaf, const double *soil, double user_leaf, double user_soil,
+                           const double *wavelength, const double *angles, double *jac, double *rsurf);
+
 /* ---- energy balance: replaces gortt_energy / gortt_albedo / gauleg (include/gortt.h:273-275;
  *      gortt.c:208-209, :322).  One result per input line (only sza/saa of the line matter):
  *      albedo, favegt, fasoil are [M][G][W]. ---------------------------------------------- */
